@@ -19,6 +19,9 @@ in HBM (62.9 GB per pass per GPU).  Weak scaling: every rank runs its own 65,536
               broadcast each (mg_kdtree_broadcast), 1M reversible-jump chains shared out over the ranks.
   --impl reference   the CPU restatement of the OCaml reference (oracle/; no OCaml toolchain exists in this image)
               on all host threads, on a bounded sample of the headline workload.
+  --dump-outputs DIR  what the last timed step of the headline workload computed (final states, accept counters, a
+              seeded sample of the sample block) as .npy files, so that two builds can be compared output for output.
+              Only rank 0's chains are written, and nothing of the evidence or rjmcmc legs.
 Every multi-GPU step goes through the C ABI's communicator (mg_comm_*, NCCL); torch.distributed only launches the
 ranks, carries the 128-byte NCCL id and takes the max of the timings.
 """
@@ -45,6 +48,9 @@ NSTEPS = 10000          # steps per chain per pass; n = NSTEPS + 1 samples, nski
 SEED = 0x5EED0001
 BYTES_PER_STEP = 8 * (D + 2)   # SURVEY.md 8d: one recorded sample per chain-step at nskip = 1
 EV_N, EV_D = 10_000_000, 20    # config 3
+DUMP_BYTES = 60_000_000        # --dump-outputs: data bytes of all files together (64 MB less room for the .npy headers)
+DUMP_CHAINS = 65536            # --dump-outputs: chains whose final state and counter are written
+DUMP_SEED = 20240601           # --dump-outputs: the chains and slots sampled from larger outputs
 
 
 def model():
@@ -133,6 +139,32 @@ def traffic_of(kernel_name):
     except Exception:
         pass
     return None, None
+
+
+def dump_outputs(path, state, samples, accept):
+    """Writes what the timed call (mg_mcmc_array_dev) hands its caller after the last timed step, as float64 .npy
+    files, so that two builds run with the same arguments can be compared value for value:
+      final_state [D+2][k]  coordinates, log-likelihood and log-prior of k chains (all of them up to DUMP_CHAINS,
+                            else a seeded sample), chain ids in final_state_chain [k]
+      accept      [k]       accepted steps of the same chains over the warm-up and timed calls
+      samples     [m][D+2]  a seeded sample of m (step, chain) slots of the [n][D+2][C] sample block, filling what is
+                            left of DUMP_BYTES; step and chain of each row in samples_slot [m][2]."""
+    import torch
+    n, F, Cn = samples.shape
+    rng = np.random.default_rng(DUMP_SEED)
+    chains = np.arange(Cn) if Cn <= DUMP_CHAINS else np.sort(rng.choice(Cn, DUMP_CHAINS, replace=False))
+    ci = torch.from_numpy(chains).to(state.device)
+    out = {"final_state": state[:, ci], "final_state_chain": chains, "accept": accept[ci]}
+    left = DUMP_BYTES - 8 * len(chains) * (F + 2)
+    m = min(n * Cn, max(0, left // (8 * (F + 2))))
+    slots = np.sort(rng.choice(n * Cn, m, replace=False))
+    step, chain = slots // Cn, slots % Cn
+    out["samples"] = samples[torch.from_numpy(step).to(state.device), :, torch.from_numpy(chain).to(state.device)]
+    out["samples_slot"] = np.stack([step, chain], axis=1)
+    os.makedirs(path, exist_ok=True)
+    for name, a in out.items():
+        a = a.cpu().numpy() if isinstance(a, torch.Tensor) else a
+        np.save(os.path.join(path, name + ".npy"), np.ascontiguousarray(a, dtype=np.float64))
 
 
 def cpu_reference(nthreads, target_seconds=12.0):
@@ -432,7 +464,13 @@ def main():
     ap.add_argument("--ev-n", type=int, default=EV_N)
     ap.add_argument("--rj-chains", type=int, default=1_000_000)
     ap.add_argument("--rj-ntree", type=int, default=10_000_000)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed to DIR/<name>.npy (rank 0; see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
 
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -509,6 +547,8 @@ def main():
     clocks = sampler.stop() if rank == 0 else None
     ms_per_step = total_ms / args.steps
     value = Cn * T * world / (ms_per_step * 1e-3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, state, samples, accept)   # before the e2e calls below overwrite the block
 
     # ---- e2e: C-ABI call with host buffers -------------------------------
     x0 = torch.empty((Cn, D), dtype=torch.float64).pin_memory()

@@ -1,8 +1,11 @@
-"""Regenerates tests/golden/gc_data.py from the reference (run in the build
-container, where /root/reference exists; the GPU box only reads the output)."""
+"""Regenerates tests/golden/gc_data.py from a checkout of the OCaml reference (farr/mcmc-ocaml):
+    python tests/golden/make_gc_data.py <reference checkout>
+The tests only read the output."""
+import os
 import re
+import sys
 
-src = open("/root/reference/bin/gaussian_cauchy_efficiency.ml").read()
+src = open(os.path.join(sys.argv[1], "bin", "gaussian_cauchy_efficiency.ml")).read()
 m = re.search(r"let data = \[\|(.*?)\|\]", src, re.S)
 vals = [float(v) for v in m.group(1).replace("\n", " ").split(";") if v.strip()]
 assert len(vals) == 100
