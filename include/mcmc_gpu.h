@@ -506,6 +506,53 @@ int mg_stats_autocorrelation(mg_ctx *ctx, const double *x, int64_t n,
                              int32_t nslides, double *out_r,
                              double *out_length);
 
+/* Ensemble convergence diagnostics of a sample block (an addition beyond the
+ * reference, like the integrated length above; DESIGN.md 4b).  Block
+ * x[s][f][c], s < n, f < F = D+2, c < C.
+ * Sequences: split = 1 -> N = n/2 (floor), M = 2C, sequence c = rows [0, N) of
+ * chain c, sequence C+c = rows [n-N, n) (an odd n drops its middle row);
+ * split = 0 -> N = n, M = C.  Per sequence m and field f:
+ *   xbar_m = (1/N) sum_s x_s,  s2_m = N/(N-1) gamma_m(0),
+ *   gamma_m(t) = (1/N) sum_{s=0}^{N-1-t} (x_s - xbar_m)(x_{s+t} - xbar_m).
+ * Pooled: W = mean_m s2_m, B = N/(M-1) sum_m (xbar_m - xbar)^2 (0 if M = 1),
+ *   var+ = (N-1)/N W + B/N, Rhat = sqrt(var+/W) (NaN if M = 1, +inf if W = 0
+ *   and the means differ), rho_0 = 1, rho_t = 1 - (W - mean_m gamma_m(t))/var+.
+ * Geyer's initial monotone sequence: P_k = rho_2k + rho_2k+1 (k < L/2),
+ *   K = first k with P_k <= 0 (none: K = L/2, window_closed = 0), P'_0 = P_0,
+ *   P'_k = min(P_k, P'_k-1), tau = -1 + 2 sum_{k<K} P'_k, ESS = M N / tau.
+ * Per sequence: the same rule on gamma_m(t)/gamma_m(0) gives seq_tau (NaN for a
+ * constant sequence or one with a non-finite value).  A field that is constant
+ * over the block or holds a non-finite value has NaN Rhat, ESS, tau and rho.
+ * MG_EINVAL: null or inconsistent arguments, L < 2, L >= N, L > MG_DIAG_MAXLAG,
+ * split with n < 4.  The definition holds for any 2 <= L <= N-1; the kernel
+ * keeps a sequence's lag sums in registers and so stops at MG_DIAG_MAXLAG = 256
+ * (a known gap: a chain with tau above ~50-100 may need a longer window, which
+ * then shows as window_closed = 0 and tau as a lower bound). */
+#define MG_DIAG_MAXLAG 256
+typedef struct {
+  int64_t n;        /* rows of the block (samples per chain) */
+  int64_t nchains;  /* C */
+  int32_t dim;      /* D: fields 0..D+1 are diagnosed */
+  int32_t maxlag;   /* L: lags 0..L-1, 2 <= L <= min(N-1, MG_DIAG_MAXLAG) */
+  int32_t split;    /* 1: each chain is two sequences (split-R-hat) */
+  int32_t reserved;
+} mg_diag_cfg;
+/* d_samples: device [n][D+2][C] (the layout of mg_mcmc_array_dev /
+ * _resident), not modified.  out_rhat, out_ess, out_tau: host [D+2];
+ * out_window_closed: host int32 [D+2]; out_rho: host [D+2][L] or NULL;
+ * d_seq_tau: device [D+2][M] or NULL. */
+int mg_stats_chain_diagnostics_dev(mg_ctx *ctx, const double *d_samples,
+                                   const mg_diag_cfg *cfg, double *out_rhat,
+                                   double *out_ess, double *out_tau,
+                                   int32_t *out_window_closed, double *out_rho,
+                                   double *d_seq_tau);
+/* the same on a host block; seq_tau: host [D+2][M] or NULL */
+int mg_stats_chain_diagnostics(mg_ctx *ctx, const double *samples,
+                               const mg_diag_cfg *cfg, double *out_rhat,
+                               double *out_ess, double *out_tau,
+                               int32_t *out_window_closed, double *out_rho,
+                               double *seq_tau);
+
 /* Stats.draw_uniform a b / draw_gaussian mu sigma / draw_cauchy x0 gamma
  * (stats.ml:126-128, 113-124 [Leva's ratio of uniforms], 89-91), n draws at
  * once.  Draw i comes from the call's Philox stream; the reference's global
@@ -640,6 +687,20 @@ int mg_rjmcmc_array_sharded(mg_comm *comm, const mg_rj_model *A,
 int mg_comm_pool_moments(mg_comm *comm, int64_t n_local, const double *mean_local,
                          const double *std_local, int32_t F, int64_t *n_total,
                          double *out_mean, double *out_std);
+/* mg_stats_chain_diagnostics_dev over chains sharded across the ranks: each
+ * rank passes its own [n][D+2][C_r] block (same n, dim, maxlag and split on
+ * every rank).  The pooled outputs are identical on every rank (one rank: the
+ * bits of the single-GPU call); d_seq_tau covers the local sequences [D+2][M_r].
+ * dim and maxlag size the exchanged record, so they MUST agree on every rank: a
+ * rank whose dim or maxlag is out of range returns before the collective, and
+ * ranks that disagree enter it with different sizes; in both cases the other
+ * ranks wait for ever (as in mg_comm_pool_moments).  A differing n or split,
+ * or a failure of the local pass, is reported as an error on every rank. */
+int mg_comm_chain_diagnostics(mg_comm *comm, const double *d_samples_local,
+                              const mg_diag_cfg *cfg_local, double *out_rhat,
+                              double *out_ess, double *out_tau,
+                              int32_t *out_window_closed, double *out_rho,
+                              double *d_seq_tau);
 
 /* ------------------------------------------------------------------ */
 /* Read_write: the text format of the reference's tools (host only)    */

@@ -66,6 +66,14 @@ class mg_nested_cfg(C.Structure):
                 ("epsrel", C.c_double), ("mode_hopping_frac", C.c_double), ("max_points", C.c_int64)]
 
 
+class mg_diag_cfg(C.Structure):
+    _fields_ = [("n", C.c_int64), ("nchains", C.c_int64), ("dim", C.c_int32), ("maxlag", C.c_int32),
+                ("split", C.c_int32), ("reserved", C.c_int32)]
+
+
+DIAG_MAXLAG = 256   # MG_DIAG_MAXLAG
+
+
 def as_f64(a, shape=None) -> np.ndarray:
     a = np.ascontiguousarray(a, dtype=np.float64)
     if shape is not None:

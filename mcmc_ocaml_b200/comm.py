@@ -169,3 +169,14 @@ class Comm:
         self.ctx.check(self.ctx.lib.mg_comm_pool_moments(self.h, C.c_int64(n_local), _abi.ptr(m), _abi.ptr(s), C.c_int32(m.size),
                                                          C.byref(nt), _abi.ptr(om), _abi.ptr(os_)))
         return int(nt.value), om, os_
+
+    def chain_diagnostics(self, samples_ptr: int, n: int, D: int, nchains_local: int, maxlag: int, *, split: bool = True,
+                          seq_tau_ptr: int | None = None):
+        """``stats.chain_diagnostics_dev`` over chains sharded across the ranks (this rank's device block
+        [n][D+2][C_r]); the pooled outputs are identical on every rank, ``seq_tau_ptr`` gets the local sequences."""
+        from . import stats
+        cfg = stats._diag_cfg(n, D, nchains_local, maxlag, split)
+        outs = stats._diag_outputs(D, maxlag)
+        self.ctx.check(stats._diag_call(self.ctx.lib.mg_comm_chain_diagnostics, self.h, C.c_void_p(samples_ptr), cfg,
+                                        outs, C.c_void_p(seq_tau_ptr) if seq_tau_ptr else None))
+        return stats.ChainDiagnostics(*outs)

@@ -643,3 +643,52 @@ extern "C" int mg_kdtree_build_distributed(mg_comm *c, const double *d_pts, int6
   *out = tr;
   return MG_OK;
 }
+
+// Ensemble diagnostics (diagnostics.cu) of chains sharded over the ranks: every rank runs the local pass on its own
+// [n][D+2][C_r] block and pools it into one record per field, (count, mean and M2 of the sequence means, sum s_m^2,
+// sum_m gamma_m(t)) = F (L + 4) doubles, plus its status; the records are all-gathered and folded in rank order by the
+// same host step as the single-GPU call, so every rank gets the same bytes and one rank gives the single-GPU bits.
+namespace mg {
+int diag_check_cfg(mg_ctx *ctx, const mg_diag_cfg *cfg);
+int diag_local_record(mg_ctx *ctx, const double *d_x, const mg_diag_cfg *cfg, double *d_seq_tau, std::vector<double> &rec);
+void diag_finish(const double *recs, int R, int F, int L, int64_t N, double *rhat, double *ess, double *tau,
+                 int32_t *closed, double *rho);
+}  // namespace mg
+
+extern "C" int mg_comm_chain_diagnostics(mg_comm *c, const double *d_samples_local, const mg_diag_cfg *cfg_local,
+                                         double *out_rhat, double *out_ess, double *out_tau, int32_t *out_window_closed,
+                                         double *out_rho, double *d_seq_tau) {
+  if (!c) return MG_EINVAL;
+  mg_ctx *ctx = c->ctx;
+  // dim and maxlag size the exchanged record: every rank must pass the same values (include/mcmc_gpu.h).  A rank that
+  // fails this check returns before the collective and the others wait for it, as in mg_comm_pool_moments; every
+  // later failure (other checks, the local pass) still takes part in the all-gather and is reported on every rank.
+  MG_REQUIRE(ctx, cfg_local && cfg_local->dim >= 1 && cfg_local->maxlag >= 2 && cfg_local->maxlag <= MG_DIAG_MAXLAG,
+             "chain_diagnostics (comm): bad configuration");
+  MG_CUDA(ctx, cudaSetDevice(ctx->device));
+  const int F = cfg_local->dim + 2, L = cfg_local->maxlag, W = L + 4;
+  int rc = diag_check_cfg(ctx, cfg_local);
+  if (rc == MG_OK && !(d_samples_local && out_rhat && out_ess && out_tau && out_window_closed))
+    rc = set_err(ctx, MG_EINVAL, "chain_diagnostics (comm): null argument");
+  std::vector<double> rec;
+  if (rc == MG_OK) rc = diag_local_record(ctx, d_samples_local, cfg_local, d_seq_tau, rec);
+  std::vector<double> mine((size_t)F * W + 3, 0.0), all(mine.size() * c->nranks);
+  if (rc == MG_OK) std::copy(rec.begin(), rec.end(), mine.begin());
+  const int64_t N = cfg_local->split ? cfg_local->n / 2 : cfg_local->n;
+  mine[(size_t)F * W] = (double)rc;
+  mine[(size_t)F * W + 1] = (double)N;
+  mine[(size_t)F * W + 2] = (double)cfg_local->split;
+  const int rc2 = mg_comm_allgather(c, mine.data(), all.data(), (int64_t)(sizeof(double) * mine.size()));
+  if (rc) return rc;
+  if (rc2) return rc2;
+  std::vector<double> recs((size_t)F * W * c->nranks);
+  for (int r = 0; r < c->nranks; ++r) {
+    const double *q = all.data() + mine.size() * r;
+    if (q[(size_t)F * W] != 0.0) return set_err(ctx, (int)q[(size_t)F * W], "chain_diagnostics (comm): rank %d failed", r);
+    if (q[(size_t)F * W + 1] != (double)N || q[(size_t)F * W + 2] != (double)cfg_local->split)
+      return set_err(ctx, MG_EINVAL, "chain_diagnostics (comm): rank %d has another n or split", r);
+    std::copy(q, q + (size_t)F * W, recs.begin() + (size_t)F * W * r);
+  }
+  diag_finish(recs.data(), c->nranks, F, L, N, out_rhat, out_ess, out_tau, out_window_closed, out_rho);
+  return MG_OK;
+}

@@ -2,6 +2,7 @@
 from __future__ import annotations
 
 import ctypes as C
+from dataclasses import dataclass
 
 import numpy as np
 
@@ -73,6 +74,70 @@ def sample_block_stats(samples_ptr: int, n: int, D: int, nchains: int, *, ctx: C
     ctx.check(ctx.lib.mg_stats_sample_block_dev(ctx.h, C.c_void_p(samples_ptr), C.c_int64(n), C.c_int32(D),
                                                 C.c_int64(nchains), _abi.ptr(m), _abi.ptr(s)))
     return m, s
+
+
+# --- ensemble convergence diagnostics (an addition beyond the reference, DESIGN.md 4b) ---------------------------
+
+@dataclass
+class ChainDiagnostics:
+    """Per field (0..D-1 values, D log_likelihood, D+1 log_prior): split-Rhat, effective sample size, integrated
+    autocorrelation time (Geyer's initial monotone sequence), whether a non-positive pair closed the lag window, the
+    ensemble autocorrelation rho[F][L]; ``seq_tau[F][M]`` (per sequence) when asked for."""
+    rhat: np.ndarray
+    ess: np.ndarray
+    tau: np.ndarray
+    window_closed: np.ndarray
+    rho: np.ndarray
+    seq_tau: np.ndarray | None = None
+
+
+def _diag_cfg(n: int, D: int, nchains: int, maxlag: int, split: bool):
+    return _abi.mg_diag_cfg(n=int(n), nchains=int(nchains), dim=int(D), maxlag=int(maxlag), split=1 if split else 0,
+                            reserved=0)
+
+
+def _diag_outputs(D: int, maxlag: int):
+    F = D + 2
+    return (np.empty(F), np.empty(F), np.empty(F), np.empty(F, dtype=np.int32), np.empty((F, int(maxlag))))
+
+
+def _diag_call(fn, handle, ptr_arg, cfg, outs, seq_tau_arg):
+    rh, es, ta, wc, rho = outs
+    return fn(handle, ptr_arg, C.byref(cfg), _abi.ptr(rh), _abi.ptr(es), _abi.ptr(ta), _abi.ptr(wc, _abi.c_int32_p),
+              _abi.ptr(rho), seq_tau_arg)
+
+
+def chain_diagnostics(samples, maxlag: int, *, split: bool = True, per_sequence: bool = False,
+                      ctx: Context | None = None) -> ChainDiagnostics:
+    """Diagnostics of a host sample block: an ``McmcSamples`` (a chain-major block is transposed here) or an array
+    [n][D+2][C].  ``per_sequence`` adds tau of every sequence ([F][M], M = 2C with ``split``)."""
+    ctx = ctx or default_context()
+    if hasattr(samples, "layout"):
+        blk = samples.block if samples.layout == "step" else np.transpose(samples.block, (1, 2, 0))
+    else:
+        blk = samples
+    blk = _abi.as_f64(blk)
+    if blk.ndim != 3 or blk.shape[1] < 3:
+        raise _abi.InvalidArgument("chain_diagnostics: the block must be [n][D+2][C] with D >= 1")
+    n, F, nc = blk.shape
+    D = F - 2
+    cfg = _diag_cfg(n, D, nc, maxlag, split)
+    outs = _diag_outputs(D, maxlag)
+    seq = np.empty((F, (2 if split else 1) * nc)) if per_sequence else None
+    ctx.check(_diag_call(ctx.lib.mg_stats_chain_diagnostics, ctx.h, _abi.ptr(blk), cfg, outs, _abi.ptr(seq)))
+    return ChainDiagnostics(*outs, seq)
+
+
+def chain_diagnostics_dev(samples_ptr: int, n: int, D: int, nchains: int, maxlag: int, *, split: bool = True,
+                          seq_tau_ptr: int | None = None, ctx: Context | None = None) -> ChainDiagnostics:
+    """The same over a device sample block [n][D+2][C] (``mg_mcmc_array_dev`` / ``_resident``), which is not
+    modified; per-sequence tau goes to the device array ``seq_tau_ptr`` ([D+2][M] float64) when given."""
+    ctx = ctx or default_context()
+    cfg = _diag_cfg(n, D, nchains, maxlag, split)
+    outs = _diag_outputs(D, maxlag)
+    ctx.check(_diag_call(ctx.lib.mg_stats_chain_diagnostics_dev, ctx.h, C.c_void_p(samples_ptr), cfg, outs,
+                         C.c_void_p(seq_tau_ptr) if seq_tau_ptr else None))
+    return ChainDiagnostics(*outs)
 
 
 # --- draws and densities (stats.ml:89-128, 240-248) ------------------------------------------------------------

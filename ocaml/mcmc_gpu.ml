@@ -41,6 +41,14 @@ external multi_mean_raw :
 external multi_std_raw :
   ctx -> (float, float64_elt, c_layout) Array2.t -> (float, float64_elt, c_layout) Array1.t ->
   (float, float64_elt, c_layout) Array1.t -> unit = "mcmcgpu_stats_multi_std"
+external chain_diagnostics_raw :
+  ctx -> int -> int -> (float, float64_elt, c_layout) Array3.t -> (float, float64_elt, c_layout) Array2.t ->
+  (float, float64_elt, c_layout) Array2.t -> (float, float64_elt, c_layout) Array2.t -> unit
+  = "mcmcgpu_chain_diagnostics_bytecode" "mcmcgpu_chain_diagnostics_native"
+external chain_diagnostics_dev_raw :
+  ctx -> int64 -> int -> int -> int -> int -> int -> (float, float64_elt, c_layout) Array2.t ->
+  (float, float64_elt, c_layout) Array2.t -> int64 -> unit
+  = "mcmcgpu_chain_diagnostics_dev_bytecode" "mcmcgpu_chain_diagnostics_dev_native"
 (* the record the stub reads field by field (rj_of_value in mcmc_gpu_stubs.c) *)
 type rj_model_raw = {
   r_like : logfn; r_prior : logfn; r_prop : proposal; r_into : tree option;
@@ -179,6 +187,29 @@ let multi_std ctx ?mean (xs : float array array) =
   let out = Array1.create float64 c_layout (Array.length xs.(0)) in
   multi_std_raw ctx (ba2 xs) (match mean with None -> ba1 [||] | Some mu -> ba1 mu) out;
   Array.init (Array1.dim out) (fun i -> out.{i})
+
+(* Ensemble convergence diagnostics of a sample block (an addition beyond the reference, include/mcmc_gpu.h) *)
+type chain_diagnostics = {
+  rhat : float array; ess : float array; tau : float array; window_closed : bool array;
+  rho : float array array; seq_tau : float array array option }
+let diag_result f maxlag out rho seq_tau =
+  { rhat = Array.init f (fun i -> out.{0, i}); ess = Array.init f (fun i -> out.{1, i});
+    tau = Array.init f (fun i -> out.{2, i}); window_closed = Array.init f (fun i -> out.{3, i} <> 0.);
+    rho = Array.init f (fun i -> Array.init maxlag (fun t -> rho.{i, t}));
+    seq_tau = Option.map (fun s -> Array.init f (fun i -> Array.init (Array2.dim2 s) (fun m -> s.{i, m}))) seq_tau }
+let chain_diagnostics ctx ?(split = true) ?(per_sequence = false) ~maxlag
+    (block : (float, float64_elt, c_layout) Array3.t) =
+  let f = Array3.dim2 block and c = Array3.dim3 block in
+  let m = if split then 2 * c else c in
+  let out = Array2.create float64 c_layout 4 f and rho = Array2.create float64 c_layout f maxlag in
+  let st = if per_sequence then Array2.create float64 c_layout f m else Array2.create float64 c_layout 0 0 in
+  chain_diagnostics_raw ctx maxlag (if split then 1 else 0) block out rho st;
+  diag_result f maxlag out rho (if per_sequence then Some st else None)
+let chain_diagnostics_dev ctx ?(split = true) ?(seq_tau = 0L) ~maxlag ~n ~dim ~nchains (block : int64) =
+  let f = dim + 2 in
+  let out = Array2.create float64 c_layout 4 f and rho = Array2.create float64 c_layout f maxlag in
+  chain_diagnostics_dev_raw ctx block n dim nchains maxlag (if split then 1 else 0) out rho seq_tau;
+  diag_result f maxlag out rho None
 
 (* Nested.nested_evidence ?epsrel ?nmcmc ?nlive ?mode_hopping_frac (nested.ml:122-146; nested.mli:50-61) with draw_prior
    uniform on [prior_low, prior_high]; ?batch live points are replaced per iteration (1 = the reference's schedule).

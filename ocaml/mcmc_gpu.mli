@@ -95,6 +95,21 @@ val enclosing_ellipse : ctx -> float -> float array array -> ellipse
 val multi_mean : ctx -> float array array -> float array
 val multi_std : ctx -> ?mean:float array -> float array array -> float array
 
+type chain_diagnostics = {
+  rhat : float array; ess : float array; tau : float array; window_closed : bool array;
+  rho : float array array; seq_tau : float array array option }
+val chain_diagnostics :
+  ctx -> ?split:bool -> ?per_sequence:bool -> maxlag:int -> (float, Bigarray.float64_elt, Bigarray.c_layout) Bigarray.Array3.t ->
+  chain_diagnostics
+(** Ensemble convergence diagnostics of a sample block [n][D+2][C] (an addition beyond the reference): per field
+    split-Rhat, ESS, Geyer's integrated autocorrelation time, whether the lag window closed and the ensemble
+    autocorrelation at lags [0, maxlag); [?per_sequence] adds tau of every sequence.  Definitions in mcmc_gpu.h.
+    [Invalid_argument] for maxlag < 2, maxlag >= N or above 256, split with n < 4. *)
+val chain_diagnostics_dev :
+  ctx -> ?split:bool -> ?seq_tau:int64 -> maxlag:int -> n:int -> dim:int -> nchains:int -> int64 ->
+  chain_diagnostics
+(** The same on a device block (its address); [?seq_tau] is the device address of a [D+2][M] float64 array. *)
+
 (** {2 Nested (nested.mli:50-69)} *)
 val nested_evidence :
   ctx -> ?epsrel:float -> ?nmcmc:int -> ?nlive:int -> ?mode_hopping_frac:float -> ?batch:int -> ?max_points:int ->

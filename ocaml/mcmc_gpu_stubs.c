@@ -270,6 +270,65 @@ CAMLprim value mcmcgpu_stats_multi_std(value ctx, value xs, value mean_opt, valu
   CAMLreturn(Val_unit);
 }
 
+/* ---- ensemble convergence diagnostics (mg_stats_chain_diagnostics*, an addition beyond the reference) ------------
+ * out: [4][F] = rhat, ess, tau, window_closed (0. / 1.); rho: [F][L]; seq_tau: [F][M], or [0][0] for none.
+ * external chain_diagnostics : ctx -> int (* maxlag *) -> int (* split *) -> (float, float64_elt, c_layout) Array3.t
+ *   (* block [n][D+2][C] *) -> Array2.t (* out *) -> Array2.t (* rho *) -> Array2.t (* seq_tau *) -> unit
+ * More than 5 arguments: bytecode / native pair. */
+static void diag_run(mg_ctx *c, const double *blk_host, const double *blk_dev, mg_diag_cfg *cfg, value out, value rho,
+                     double *seq_tau) {
+  const int F = cfg->dim + 2;
+  int32_t *closed = (int32_t *)malloc(sizeof(int32_t) * (size_t)F);
+  double *o = (double *)Caml_ba_data_val(out);
+  double *prho = (double *)Caml_ba_data_val(rho);
+  if (!closed) caml_failwith("chain_diagnostics: out of memory");
+  caml_release_runtime_system();
+  int rc = blk_host ? mg_stats_chain_diagnostics(c, blk_host, cfg, o, o + F, o + 2 * F, closed, prho, seq_tau)
+                    : mg_stats_chain_diagnostics_dev(c, blk_dev, cfg, o, o + F, o + 2 * F, closed, prho, seq_tau);
+  caml_acquire_runtime_system();
+  if (rc == MG_OK)
+    for (int f = 0; f < F; ++f) o[3 * F + f] = (double)closed[f];
+  free(closed);
+  check(c, rc);
+}
+CAMLprim value mcmcgpu_chain_diagnostics_native(value ctx, value maxlag, value split, value blk, value out, value rho,
+                                                value seq_tau) {
+  CAMLparam5(ctx, maxlag, split, blk, out);
+  CAMLxparam2(rho, seq_tau);
+  struct caml_ba_array *b = Caml_ba_array_val(blk);
+  mg_diag_cfg cfg;
+  memset(&cfg, 0, sizeof cfg);
+  cfg.n = b->dim[0]; cfg.dim = (int32_t)b->dim[1] - 2; cfg.nchains = b->dim[2];
+  cfg.maxlag = Int_val(maxlag); cfg.split = Int_val(split);
+  double *st = Caml_ba_array_val(seq_tau)->dim[0] > 0 ? (double *)Caml_ba_data_val(seq_tau) : NULL;
+  diag_run(Ctx_val(ctx), (const double *)Caml_ba_data_val(blk), NULL, &cfg, out, rho, st);
+  CAMLreturn(Val_unit);
+}
+CAMLprim value mcmcgpu_chain_diagnostics_bytecode(value *a, int argn) {
+  (void)argn;
+  return mcmcgpu_chain_diagnostics_native(a[0], a[1], a[2], a[3], a[4], a[5], a[6]);
+}
+/* the same on a device block (its device address as int64, e.g. from another CUDA library); seq_tau: device
+ * address of [F][M] doubles or 0L.
+ * external chain_diagnostics_dev : ctx -> int64 -> int (* n *) -> int (* dim *) -> int (* nchains *) ->
+ *   int (* maxlag *) -> int (* split *) -> Array2.t (* out *) -> Array2.t (* rho *) -> int64 -> unit */
+CAMLprim value mcmcgpu_chain_diagnostics_dev_native(value ctx, value ptr, value n, value dim, value nchains, value maxlag,
+                                                    value split, value out, value rho, value seq_tau) {
+  CAMLparam5(ctx, ptr, n, dim, nchains);
+  CAMLxparam3(maxlag, split, out);
+  CAMLxparam2(rho, seq_tau);
+  mg_diag_cfg cfg;
+  memset(&cfg, 0, sizeof cfg);
+  cfg.n = Long_val(n); cfg.dim = Int_val(dim); cfg.nchains = Long_val(nchains);
+  cfg.maxlag = Int_val(maxlag); cfg.split = Int_val(split);
+  diag_run(Ctx_val(ctx), NULL, (const double *)(intptr_t)Int64_val(ptr), &cfg, out, rho, (double *)(intptr_t)Int64_val(seq_tau));
+  CAMLreturn(Val_unit);
+}
+CAMLprim value mcmcgpu_chain_diagnostics_dev_bytecode(value *a, int argn) {
+  (void)argn;
+  return mcmcgpu_chain_diagnostics_dev_native(a[0], a[1], a[2], a[3], a[4], a[5], a[6], a[7], a[8], a[9]);
+}
+
 /* ---- Stats.draw_uniform / draw_gaussian / draw_cauchy (stats.ml:89-91,113-128), n draws per call ----------
  * external stats_draw : ctx -> int -> float -> float -> (float, float64_elt, c_layout) Array1.t -> unit
  * kind: 0 uniform a b | 1 gaussian mu sigma | 2 cauchy x0 gamma (MG_DRAW_*) */

@@ -11,6 +11,8 @@ NCCL id and allocates the test data):
   5. RJMCMC sharded (mg_rjmcmc_array_sharded): model counts equal to the one-rank run of all chains.
   6. kd-tree built by all ranks together (mg_kdtree_build_distributed): every array equal to the single-GPU tree's on
      every rank; both builds timed.
+  7. ensemble diagnostics of the chains of step 4, sharded as there (mg_comm_chain_diagnostics): the same bytes on
+     every rank, within 1e-12 of the one-GPU call on all chains.  It runs right after step 4, whose chains it uses.
 Prints one JSON line on rank 0."""
 from __future__ import annotations
 
@@ -138,6 +140,21 @@ def main():
         out["ensemble_std_err"] = float(np.max(np.abs(ps - rp.std(0, ddof=1))))
         out["accept_equal"] = bool(int(acc) == int(ref.accept.sum()) and ntot == rp.shape[0])
         out["shard_chains_bit_exact"] = bool(np.array_equal(ref.block[:, :, cb:ce], s.block))
+    # ---- 7. ensemble diagnostics of the sharded chains (mg_comm_chain_diagnostics) ----------------
+    # every rank diagnoses its own chains; the pooled outputs must be the same bytes on every rank and within 1e-12 of
+    # the one-GPU call on all chains
+    from mcmc_ocaml_b200 import stats
+    dblk = torch.as_tensor(np.ascontiguousarray(s.block), device=dev); torch.cuda.synchronize()
+    dgr = comm.chain_diagnostics(dblk.data_ptr(), n, Dd, ce - cb, 32)
+    vec = np.concatenate([dgr.rhat, dgr.ess, dgr.tau, dgr.window_closed.astype(np.float64), dgr.rho.ravel()])
+    allv = np.asarray(comm.allgather(vec)).reshape(world, -1)
+    del dblk
+    if rank == 0:
+        one = stats.chain_diagnostics(ref.block, 32, ctx=ctx)
+        ov = np.concatenate([one.rhat, one.ess, one.tau, one.window_closed.astype(np.float64), one.rho.ravel()])
+        out["diagnostics_identical_on_all_ranks"] = bool(all(np.array_equal(allv[r_], allv[0], equal_nan=True)
+                                                             for r_ in range(world)))
+        out["diagnostics_within_1e12_of_single_gpu"] = bool(np.allclose(vec, ov, rtol=1e-12, atol=1e-12, equal_nan=True))
     # ---- 5. sharded RJMCMC over the broadcast tree(s) ----------------------------
     d2 = Dm
     likeA = P.gauss_diag(np.full(d2, 0.5), np.full(d2, 0.08)); priorA = P.box(np.zeros(d2), np.ones(d2), 0.0)
@@ -188,6 +205,7 @@ def main():
                          and out["ensemble_mean_err"] < 1e-12 and out["ensemble_std_err"] < 1e-12
                          and out["harmonic_sharded_rel_err"] < 1e-14 and out["evidence_identical_on_all_ranks"]
                          and out["evidence_bit_identical_to_single_gpu"] and out["rj_counts_equal"]
+                         and out["diagnostics_identical_on_all_ranks"] and out["diagnostics_within_1e12_of_single_gpu"]
                          and all(out[f"dist_build_ms{ms}"]["identical_to_single_gpu_on_every_rank"] for ms in (2, 64)))
         s_ = json.dumps(out)
         print(s_)
