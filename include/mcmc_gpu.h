@@ -319,8 +319,9 @@ int mg_kdtree_from_blob_dev(mg_ctx *ctx, const void *d_blob, int64_t nbytes,
  * locates it once for every stored point (N x (2 D + 2) doubles next to the
  * tree, not inside the blob); leaf-level draws then gather one record instead
  * of ~log2 N dependent node loads, with bit-identical results.
- * mg_rjmcmc_array* enable it by themselves for trees of at most 8 dimensions
- * (MCMC_GPU_DRAW_CACHE=0 turns that off). */
+ * mg_rjmcmc_array* enable it by themselves for leaf-level draws (nstop = 0)
+ * from trees of at most 8 dimensions, when the run takes at least as many
+ * chain-steps as the tree has points. */
 int mg_kdtree_enable_draw_cache(mg_kdtree *t);
 /* Kd_tree.bounds_volume (kd_tree.ml:177-182) */
 double mg_bounds_volume(const double *low, const double *high, int32_t D);

@@ -367,31 +367,6 @@ int build_tree(mg_ctx *ctx, const double *d_pts, int64_t N, int D, const double 
 constexpr int KDD_MAXL = 96;         // levels of a subtree
 constexpr int KDD_MAXR = 64;         // ranks
 
-// level table of a breadth-first tree with adjacent children: lb[l] = first node of level l, lb[nl] = nnodes
-__global__ void __launch_bounds__(1024) kdd_levels_kernel(const KdNode *__restrict__ nodes, int32_t nnodes, int32_t *__restrict__ lb,
-                                                          int32_t *__restrict__ nl) {
-  __shared__ int s_max;
-  int b = 0, e = 1, l = 0;
-  if (threadIdx.x == 0) lb[0] = 0;
-  while (b < e && l < KDD_MAXL) {
-    if (threadIdx.x == 0) s_max = -1;
-    __syncthreads();
-    int m = -1;
-    for (int i = b + threadIdx.x; i < e; i += blockDim.x) { const int lf = nodes[i].left; m = lf > m ? lf : m; }
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) { const int x = __shfl_xor_sync(0xffffffffu, m, o); m = x > m ? x : m; }
-    if ((threadIdx.x & 31) == 0 && m >= 0) atomicMax(&s_max, m);
-    __syncthreads();
-    const int last = s_max;
-    ++l;
-    b = e; e = last >= 0 ? last + 2 : e;          // the last internal node's children end the next level
-    if (threadIdx.x == 0) lb[l] = b;
-    __syncthreads();
-  }
-  if (threadIdx.x == 0) *nl = l;
-  (void)nnodes;
-}
-
 __global__ void kdd_gather_rows_kernel(const double *__restrict__ pts, const int32_t *__restrict__ perm, int64_t n, int D,
                                        double *__restrict__ out) {
   const int64_t k = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -545,24 +520,11 @@ extern "C" int mg_kdtree_build_distributed(mg_comm *c, const double *d_pts, int6
   const char *sb = rc_sub == MG_OK ? (const char *)sub.t->d_blob : nullptr;
   struct Rec { int32_t nl, nn, npts, pbegin; int32_t lb[KDD_MAXL + 1]; int32_t bad; };
   Rec mine{};
-  static const std::vector<int32_t> no_levels;
-  const std::vector<int32_t> &lvb = rc_sub == MG_OK ? sub.t->level_begin : no_levels;
-  static const bool force_kernel = getenv("MCMC_GPU_KDD_LEVELS_KERNEL") != nullptr;   // tests: take the first builder's path
-  if (rc_sub != MG_OK) {
-    mine.nl = 0;
-  } else if (!force_kernel && lvb.size() >= 2 && lvb.size() <= (size_t)KDD_MAXL + 1) {     // the builder kept its level table
-    mine.nl = (int32_t)lvb.size() - 1;
-    for (size_t l = 0; l < lvb.size(); ++l) mine.lb[l] = lvb[l];
-  } else {                                                           // first builder: read the levels off the nodes
-    DevBuf<int32_t> d_lb, d_nl;
-    MG_CUDA(ctx, d_lb.alloc(KDD_MAXL + 1, s)); MG_CUDA(ctx, d_nl.alloc(1, s));
-    kdd_levels_kernel<<<1, 1024, 0, s>>>((const KdNode *)(sb + sh.off_nodes), (int32_t)sh.nnodes, d_lb.get(), d_nl.get());
-    MG_CHECK_LAUNCH(ctx);
-    MG_CUDA(ctx, cudaMemcpyAsync(mine.lb, d_lb.get(), sizeof mine.lb, cudaMemcpyDeviceToHost, s));
-    MG_CUDA(ctx, cudaMemcpyAsync(&mine.nl, d_nl.get(), sizeof(int32_t), cudaMemcpyDeviceToHost, s));
-    MG_CUDA(ctx, cudaStreamSynchronize(s));
+  if (rc_sub == MG_OK) {                         // the builder's level table, cut at KDD_MAXL levels (then flagged below)
+    const std::vector<int32_t> &lvb = sub.t->level_begin;
+    mine.nl = (int32_t)std::min<size_t>(lvb.size() - 1, KDD_MAXL);
+    for (int l = 0; l <= mine.nl; ++l) mine.lb[l] = lvb[l];
   }
-  phase("levels");
   mine.nn = (int32_t)sh.nnodes; mine.npts = my_n; mine.pbegin = my_b;
   mine.bad = rc_sub != MG_OK ? 2 : ((mine.nl >= KDD_MAXL || mine.lb[mine.nl] != mine.nn) ? 1 : 0);
   std::vector<Rec> recs((size_t)R);

@@ -335,14 +335,11 @@ int build_tree(mg_ctx *ctx, const double *d_pts, int64_t N, int D, const double 
   MG_REQUIRE(ctx, D >= 1 && D <= 64, "kd-tree: dim must be in 1..64");
   MG_REQUIRE(ctx, N < (1LL << 30), "kd-tree: too many points for int32 indices");
   if (min_split < 2) min_split = 2;
-  // MCMC_GPU_KD_BUILD=1 keeps the first builder (presorted index lists); the default is the second one (key columns
-  // moved level by level, subtrees finished in shared memory), which hands inputs it is not made for back to the first
-  static const int which = [] { const char *e = getenv("MCMC_GPU_KD_BUILD"); return e ? atoi(e) : 2; }();
-  if (which != 1) {
-    const int rc = build_tree_v2(ctx, d_pts, N, D, low, high, min_split, out);
-    if (rc != MG_V2_FALLBACK) return rc;
-    if (getenv("MCMC_GPU_DEBUG")) fprintf(stderr, "kd-tree: second builder handed the input back (ties / depth), first builder runs\n");
-  }
+  // The second builder (key columns moved level by level, subtrees finished in shared memory) hands inputs it is not
+  // made for back to the first one (presorted index lists)
+  const int rc = build_tree_v2(ctx, d_pts, N, D, low, high, min_split, out);
+  if (rc != MG_V2_FALLBACK) return rc;
+  if (getenv("MCMC_GPU_DEBUG")) fprintf(stderr, "kd-tree: second builder handed the input back (ties / depth), first builder runs\n");
   // NaN coordinates are rejected (Pervasives.compare orders them, IEEE does not)
   DevBuf<int> d_flag;
   MG_CUDA(ctx, d_flag.alloc(1, s));
@@ -377,8 +374,7 @@ static int build_tree_v1(mg_ctx *ctx, const double *d_pts, int64_t N, int D, con
     MG_CHECK_LAUNCH(ctx);
     int rc;
     bool sorted = false;
-    static const bool use32 = [] { const char *e = getenv("MCMC_GPU_SORT32"); return e ? atoi(e) != 0 : true; }();
-    if (use32 && N >= 65536) {
+    if (N >= 65536) {
       // 32-bit window under the highest varying byte of each dimension (see make_key32_kernel)
       std::vector<unsigned char> cb;
       std::vector<double> veff;
@@ -448,8 +444,10 @@ static int build_tree_v1(mg_ctx *ctx, const double *d_pts, int64_t N, int D, con
   int nlevels = 0;
   int64_t flags_cap = 0;
   DevBuf<int32_t> scan_tmp;
+  std::vector<int32_t> level_begin;
   for (;;) {
     ++nlevels;
+    level_begin.push_back((int32_t)lb);
     if (nlevels > 100000) return set_err(ctx, MG_EFAIL, "kd-tree: too many levels");
     const int64_t nlvl = le - lb;
     if (2 * nlvl > flags_cap) {
@@ -488,6 +486,7 @@ static int build_tree_v1(mg_ctx *ctx, const double *d_pts, int64_t N, int D, con
     std::swap(lin, lout); std::swap(sin, sout);
     lb = le; le = nnodes + 2 * nsplit; nnodes = le;
   }
+  level_begin.push_back((int32_t)nnodes);
   // ---- assemble the blob ----------------------------------------------------
   KdHeader h{};
   h.magic = KD_MAGIC; h.N = N; h.nnodes = nnodes; h.D = D; h.nlevels = nlevels; h.min_split = min_split;
@@ -502,7 +501,7 @@ static int build_tree_v1(mg_ctx *ctx, const double *d_pts, int64_t N, int D, con
   h.off_pts = off; off = align256(off + (with_pts ? 8 * N * D : 0));
   h.nbytes = off;
   mg_kdtree *t = new mg_kdtree;
-  t->ctx = ctx; t->h = h;
+  t->ctx = ctx; t->h = h; t->level_begin = std::move(level_begin);
   // from the stream-ordered pool (kept cached between builds: a synchronous cudaMalloc / cudaFree of a 2 GB blob
   // costs 0.1-0.4 s now and then and synchronises the device)
   cudaError_t e = cudaMallocAsync(&t->d_blob, (size_t)h.nbytes, s);

@@ -171,7 +171,7 @@ struct mg_kdtree {
   bool owns_blob = true;
   double *d_draw_cache = nullptr;   // [N][2 D + 2], see KdView::dcache (not part of the blob: rebuilt per rank)
   mg::KdHeader h{};
-  std::vector<int32_t> level_begin;  // first node of every level and nnodes at the end, when the builder knows them (second builder)
+  std::vector<int32_t> level_begin;  // first node of every level and nnodes at the end (nlevels + 1 entries, either builder)
   mg::KdView view() const {
     const char *b = (const char *)d_blob;
     mg::KdView v;

@@ -1006,8 +1006,7 @@ int build_tree_v2(mg_ctx *ctx, const double *d_pts, int64_t N, int D, const doub
                   mg_kdtree **out) {
   cudaStream_t s = ctx->stream;
   // the largest subtree whose key columns fit the shared memory of one SM
-  // (MCMC_GPU_KD_SMEM_KB caps the shared memory of a subtree CTA: ~110 lets two CTAs share an SM)
-  static const size_t smem_cap = [] { const char *e = getenv("MCMC_GPU_KD_SMEM_KB"); return (size_t)(e ? std::max(32, atoi(e)) : 224) * 1024; }();
+  constexpr size_t smem_cap = 224 * 1024;
   const int NMAX = v2_bottom_smem<2048, 1024>(D) <= smem_cap ? 2048 : v2_bottom_smem<1024, 1024>(D) <= smem_cap ? 1024
                    : v2_bottom_smem<512, 512>(D) <= smem_cap ? 512 : 256;
   if (N >= (1LL << 30)) return MG_V2_FALLBACK;
@@ -1138,11 +1137,8 @@ int build_tree_v2(mg_ctx *ctx, const double *d_pts, int64_t N, int D, const doub
     MG_CUDA(ctx, cudaMemcpyAsync(pout, pin, sizeof(int32_t) * N, cudaMemcpyDeviceToDevice, s));   // positions outside the subtrees
     a = V2Bottom{N, D, min_split, Lh, info.get(), nb.get(), ne.get(), Kin, pin, pout, l_dim.get(), l_child.get(), l_begin.get(),
                  l_end.get(), l_split.get(), cnt.get(), depth.get(), b_over.get()};
-    // MCMC_GPU_KD_BT: threads of a 1024-point subtree CTA (experiment; tools/kd_bottom_sweep.sh)
-    static const int bt1024 = [] { const char *e = getenv("MCMC_GPU_KD_BT"); return e ? atoi(e) : 1024; }();
     rc = NMAX == 2048 ? v2_launch_bottom<2048, 1024>(ctx, a, nsub, D)
-         : NMAX == 1024 ? (bt1024 == 256 ? v2_launch_bottom<1024, 256>(ctx, a, nsub, D) : bt1024 == 512 ? v2_launch_bottom<1024, 512>(ctx, a, nsub, D)
-                                         : v2_launch_bottom<1024, 1024>(ctx, a, nsub, D))
+         : NMAX == 1024 ? v2_launch_bottom<1024, 1024>(ctx, a, nsub, D)
          : NMAX == 512 ? v2_launch_bottom<512, 512>(ctx, a, nsub, D) : v2_launch_bottom<256, 256>(ctx, a, nsub, D);
     if (rc) return rc;
     v2_level_scan_kernel<<<V2_MAXL, 1024, 0, s>>>(cnt.get(), pre.get(), nsub, totals.get());

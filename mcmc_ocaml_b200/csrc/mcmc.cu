@@ -60,12 +60,7 @@ __global__ void to_chain_major_kernel(const double *__restrict__ src, int64_t ro
 int jit_launch_mh(mg_ctx *ctx, const DynFnParams &like, const DynFnParams &prior, const DynPropParams &prop,
                   const mg_mcmc_cfg *cfg, CallKey key, uint64_t t0, int record_first, double *d_state, double *d_samples, int32_t *d_accept);  // jit.cu
 int sample_block_stats(mg_ctx *ctx, const double *d_blk, int64_t n, int F, int64_t C, double *d_out);  // stats.cu
-int moments_grid(mg_ctx *ctx, int64_t n);
-int sample_block_moments_async(mg_ctx *ctx, cudaStream_t st, const double *blk_base, const double *seg, int64_t n,
-                               int F, int64_t C, int gx, double *partial);
 int chain_moments_finish(mg_ctx *ctx, cudaStream_t st, const double *mom, int F, int64_t C, int64_t n, double *d_out);
-int sample_block_moments_finish(mg_ctx *ctx, cudaStream_t st, const double *partial, int nseg, int gx, int F, double cnt,
-                                const double *blk_base, int64_t C, double *d_out);
 
 static int validate_cfg(mg_ctx *ctx, const mg_mcmc_cfg *cfg) {
   MG_REQUIRE(ctx, cfg != nullptr, "mcmc_array: null cfg");
@@ -251,75 +246,28 @@ extern "C" int mg_mcmc_array_resident(mg_ctx *ctx, const mg_logfn *like, const m
   MG_CUDA(ctx, cudaMemsetAsync(d_acc.get(), 0, sizeof(int32_t) * C, s));
   init_state_kernel<<<(unsigned)((C + 255) / 256), 256, 0, s>>>(d_x0.get(), cfg->x0_shared, D, C, d_state.get());
   MG_CHECK_LAUNCH(ctx);
-  // The run can be cut into segments with the Stats pass over segment k (an HBM-bound read) on a second
-  // stream while the sampler computes segment k+1.  Measured on B200 (profiles/r01_mh_ncu_summary.md): no
-  // gain -- the sampler's 4 warps x 122 registers fill every scheduler's 16K-register slice, so the Stats
-  // CTAs find no room until the segment ends.  One segment unless MCMC_GPU_STATS_SEGMENTS says otherwise.
+  // Statistics: the balanced sampler can keep per-chain running moments of the samples it records
+  // (ctx->mh_mom); any other path leaves mh_mom_done false and the block is read back once.  Overlapping that
+  // read with the sampler on a second stream gave no gain on B200 (profiles/r01_mh_ncu_summary.md): the sampler's
+  // 4 warps x 122 registers fill every scheduler's 16K-register slice, so the Stats CTAs find no room until it ends.
   const bool want_stats = (out_mean || out_std) && n > 0;
   std::vector<double> stats(2 * F);
-  {
-    const int64_t nrec = n > 0 ? n - 1 : 0;          // samples after slot 0
-    int nseg = 1;
-    if (const char *e = getenv("MCMC_GPU_STATS_SEGMENTS")) nseg = atoi(e);
-    if (nseg < 1 || !want_stats || nrec < 8 * (int64_t)nseg) nseg = 1;
-    const CallKey key = next_key(ctx);
-    DevBuf<double> d_partial;
-    std::vector<cudaEvent_t> evs;
-    int gx = 1;
-    if (want_stats) {
-      gx = moments_grid(ctx, (n + nseg - 1) / nseg);
-      MG_CUDA(ctx, d_partial.alloc((size_t)nseg * 2 * F * gx, s));
-      MG_CUDA(ctx, d_stats.alloc(2 * F, s));
-      if (!ctx->aux) MG_CUDA(ctx, cudaStreamCreateWithFlags(&ctx->aux, cudaStreamNonBlocking));
-    }
-    int64_t done = 0;                                 // recorded samples after slot 0 handled so far
-    bool fused_stats = false;
-    for (int k = 0; k < nseg; ++k) {
-      const int64_t m = nrec / nseg + (k < nrec % nseg ? 1 : 0);
-      mg_mcmc_cfg seg = *cfg;
-      seg.nbin = (k == 0) ? cfg->nbin : 0;
-      seg.n = (n > 0) ? m + 1 : 0;
-      const uint64_t t0 = (k == 0) ? 0 : (uint64_t)(cfg->nbin + done * cfg->nskip);
-      double *dst = d_samples ? d_samples + (size_t)((k == 0) ? 0 : 1 + done) * F * C : nullptr;
-      // one segment: ask the sampler for per-chain running moments (the balanced kernel provides them; any other
-      // path leaves mh_mom_done false and the block is read back below)
-      DevBuf<double> d_mom;
-      if (want_stats && nseg == 1) {
-        MG_CUDA(ctx, d_mom.alloc((size_t)3 * F * C, s));
-        MG_CUDA(ctx, cudaMemsetAsync(d_mom.get(), 0, sizeof(double) * 3 * F * C, s));
-        ctx->mh_mom = d_mom.get();
-      }
-      ctx->mh_mom_done = false;
-      rc = mcmc_launch_segment(ctx, like, prior, prop, &seg, key, t0, k == 0 ? 1 : 0, d_state.get(), dst, d_acc.get());
-      ctx->mh_mom = nullptr;
-      if (rc) return rc;
-      if (want_stats && ctx->mh_mom_done) {
-        if ((rc = chain_moments_finish(ctx, s, d_mom.get(), F, C, n, d_stats.get()))) return rc;
-        MG_CUDA(ctx, cudaMemcpyAsync(stats.data(), d_stats.get(), sizeof(double) * 2 * F, cudaMemcpyDeviceToHost, s));
-        fused_stats = true;
-      } else if (want_stats) {
-        cudaEvent_t e;
-        MG_CUDA(ctx, cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-        evs.push_back(e);
-        MG_CUDA(ctx, cudaEventRecord(e, s));
-        MG_CUDA(ctx, cudaStreamWaitEvent(ctx->aux, e, 0));
-        const int64_t cnt = (k == 0) ? m + 1 : m;     // segment 0 also holds slot 0
-        if ((rc = sample_block_moments_async(ctx, ctx->aux, d_samples, dst, cnt, F, C, gx,
-                                             d_partial.get() + (size_t)k * 2 * F * gx))) return rc;
-      }
-      done += m;
-    }
-    if (want_stats && !fused_stats) {
-      cudaEvent_t e;
-      MG_CUDA(ctx, cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-      evs.push_back(e);
-      MG_CUDA(ctx, cudaEventRecord(e, ctx->aux));
-      MG_CUDA(ctx, cudaStreamWaitEvent(s, e, 0));
-      if ((rc = sample_block_moments_finish(ctx, s, d_partial.get(), nseg, gx, F, (double)n * (double)C, d_samples, C,
-                                            d_stats.get()))) return rc;
-      MG_CUDA(ctx, cudaMemcpyAsync(stats.data(), d_stats.get(), sizeof(double) * 2 * F, cudaMemcpyDeviceToHost, s));
-    }
-    for (cudaEvent_t e : evs) cudaEventDestroy(e);    // released once the recorded work has completed
+  DevBuf<double> d_mom;
+  if (want_stats) {
+    MG_CUDA(ctx, d_stats.alloc(2 * F, s));
+    MG_CUDA(ctx, d_mom.alloc((size_t)3 * F * C, s));
+    MG_CUDA(ctx, cudaMemsetAsync(d_mom.get(), 0, sizeof(double) * 3 * F * C, s));
+    ctx->mh_mom = d_mom.get();
+  }
+  ctx->mh_mom_done = false;
+  rc = mcmc_launch_segment(ctx, like, prior, prop, cfg, next_key(ctx), 0, 1, d_state.get(), d_samples, d_acc.get());
+  ctx->mh_mom = nullptr;
+  if (rc) return rc;
+  if (want_stats) {
+    if (ctx->mh_mom_done) rc = chain_moments_finish(ctx, s, d_mom.get(), F, C, n, d_stats.get());
+    else rc = sample_block_stats(ctx, d_samples, n, F, C, d_stats.get());
+    if (rc) return rc;
+    MG_CUDA(ctx, cudaMemcpyAsync(stats.data(), d_stats.get(), sizeof(double) * 2 * F, cudaMemcpyDeviceToHost, s));
   }
   if (out_final) {
     MG_CUDA(ctx, d_final.alloc((size_t)F * C, s));

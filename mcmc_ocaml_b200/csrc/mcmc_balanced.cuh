@@ -62,7 +62,6 @@ struct MhQueue {
   unsigned long long *ring;  // [cap]: (ticket + 1) << 32 | group; 0 = empty
   unsigned int *ctr;         // [0] next pop ticket, [1] next push ticket
   int32_t *seg_next;         // [ngroups] next segment of each group
-  long long *prof;           // debug: [grid][4] cycles waiting / loading / stepping / releasing, or null
   uint32_t cap;              // power of two >= 2 * ngroups
   uint32_t ngroups;
   uint32_t total;            // ngroups * nseg tickets
@@ -114,7 +113,6 @@ mh_balanced_kernel(const __grid_constant__ MhArgs<Like, Prior, Prop, D> a, const
   __shared__ double s_piv[kMom ? (D + 2) * MH_BLOCK : 1];   // [field][lane]
   for (;;) {
     // ---- take a ticket and wait for its group
-    const long long tp0 = clock64();
     unsigned long long e = 0ull;
     if (lane == 0) {
       const unsigned ticket = atomicAdd(&q.ctr[0], 1u);
@@ -140,7 +138,6 @@ mh_balanced_kernel(const __grid_constant__ MhArgs<Like, Prior, Prop, D> a, const
     e = __shfl_sync(0xffffffffu, e, 0);
     if (e == ~0ull) break;
     const uint32_t grp = (uint32_t)e;
-    const long long tp1 = clock64();
     int64_t c = (int64_t)grp * MH_BLOCK + lane;
     const bool live = c < C;
     if (!live) c = C - 1;
@@ -208,7 +205,6 @@ mh_balanced_kernel(const __grid_constant__ MhArgs<Like, Prior, Prop, D> a, const
         accumulate(dd + 1, lp, first);
       }
     };
-    const long long tp2 = clock64();
     int nacc = 0;
     uint64_t t;
     if (k < q.nseg_burn) {  // :63-65 burn-in, nothing recorded until its last step
@@ -252,7 +248,6 @@ mh_balanced_kernel(const __grid_constant__ MhArgs<Like, Prior, Prop, D> a, const
       }
     }
 
-    const long long tp3 = clock64();
     // ---- state back, group released for its next segment
     if (live) {
 #pragma unroll
@@ -288,10 +283,6 @@ mh_balanced_kernel(const __grid_constant__ MhArgs<Like, Prior, Prop, D> a, const
       if (ok) *slot2 = (((unsigned long long)t2 + 1ull) << 32) | grp;
     }
     __syncwarp();
-    if (q.prof && lane == 0) {
-      long long *pr = q.prof + (size_t)blockIdx.x * 4;
-      pr[0] += tp1 - tp0; pr[1] += tp2 - tp1; pr[2] += tp3 - tp2; pr[3] += clock64() - tp3;
-    }
   }
 }
 

@@ -50,12 +50,11 @@ template <class Like, class Prior, class Prop, int D>
 static int launch_mh(mg_ctx *ctx, const MhArgs<Like, Prior, Prop, D> &a) {
   const int64_t ngroups = (a.C + MH_BLOCK - 1) / MH_BLOCK;
   const int64_t total_steps = a.nbin + (a.n > 0 ? (a.n - 1) * a.nskip : 0);
-  static const bool want_balanced = [] { const char *e = getenv("MCMC_GPU_MH_BALANCED"); return e ? atoi(e) != 0 : true; }();
   // Dynamic hand-out pays when the warps do not divide evenly over the schedulers.  The persistent grid holds the
   // largest whole number of warps per scheduler that the ensemble can keep busy all the time (no warp ever waits for
   // work until the tail: a polling warp on a saturated scheduler is starved by the arbiter and picks its group up late).
   const int64_t nsched = (int64_t)ctx->sm_count * 4;
-  if (want_balanced && total_steps >= 4 * kSegSteps && ngroups > nsched && ngroups < (1ll << 30)) {
+  if (total_steps >= 4 * kSegSteps && ngroups > nsched && ngroups < (1ll << 30)) {
     // running moments requested (mg_mcmc_array_resident): that instantiation holds more registers per warp, so its
     // own occupancy sizes the persistent grid
     const bool with_mom = ctx->mh_mom != nullptr && a.t0 == 0 && a.record_first && a.samples != nullptr;
@@ -67,7 +66,6 @@ static int launch_mh(mg_ctx *ctx, const MhArgs<Like, Prior, Prop, D> &a) {
     if (grid != ngroups) {
     MhQueue q;
     q.seg_steps = kSegSteps;
-    if (const char *e = getenv("MCMC_GPU_MH_SEG")) q.seg_steps = std::max(1, atoi(e));
     const int64_t nrec = a.n > 1 ? a.n - 1 : 0;   // slots 1 .. n-1
     int64_t nseg;
     for (;; q.seg_steps *= 2) {
@@ -92,26 +90,17 @@ static int launch_mh(mg_ctx *ctx, const MhArgs<Like, Prior, Prop, D> &a) {
     q.err = ctx->d_devflag;
     q.wait_cycles = kQueueWaitCycles;
     if (const char *e = getenv("MCMC_GPU_WAIT_CYCLES")) q.wait_cycles = std::max(1ll, atoll(e));
-    DevBuf<long long> prof;
-    q.prof = nullptr;
-    if (getenv("MCMC_GPU_DEBUG")) {
-      MG_CUDA(ctx, prof.alloc((size_t)grid * 4, ctx->stream));
-      MG_CUDA(ctx, cudaMemsetAsync(prof.get(), 0, sizeof(long long) * grid * 4, ctx->stream));
-      q.prof = prof.get();
-    }
     mh_queue_init_kernel<<<(q.cap + 255u) / 256u, 256, 0, ctx->stream>>>(q);
     MG_CHECK_LAUNCH(ctx);
     // running moments of the recorded samples (requested through the context by mg_mcmc_array_resident): the
     // variant with the accumulators is a separate instantiation, the plain kernel does not pay for them
     // Recorded samples leave through the TMA (one bulk tensor store per kTmaSteps samples of a warp) when the block's
     // shape allows a tensor map (even C, compile-time dimension, a tile of at most 16 KB); plain stores otherwise.
-    // MCMC_GPU_MH_TMA=0 keeps the plain stores.
     CUtensorMap tmap;
     memset(&tmap, 0, sizeof tmap);
-    static const bool want_tma = [] { const char *e = getenv("MCMC_GPU_MH_TMA"); return e ? atoi(e) != 0 : true; }();
     const int F = (Prop::kStaticDim ? D : a.d) + 2;
     const int64_t slots = a.n - (a.record_first ? 0 : 1);
-    const bool use_tma = want_tma && Prop::kStaticDim && (D + 2) * kTmaSteps * MH_BLOCK * 8 <= 16 * 1024 && a.samples != nullptr &&
+    const bool use_tma = Prop::kStaticDim && (D + 2) * kTmaSteps * MH_BLOCK * 8 <= 16 * 1024 && a.samples != nullptr &&
                          make_sample_tensor_map(&tmap, a.samples, slots, F, a.C);
     time_begin(ctx);
     MhArgs<Like, Prior, Prop, D> am = a;
@@ -136,15 +125,6 @@ static int launch_mh(mg_ctx *ctx, const MhArgs<Like, Prior, Prop, D> &a) {
     kt_stop(ctx);
     MG_CHECK_LAUNCH(ctx);
     time_end(ctx);
-    if (q.prof) {
-      std::vector<long long> h((size_t)grid * 4);
-      MG_CUDA(ctx, cudaMemcpyAsync(h.data(), q.prof, sizeof(long long) * grid * 4, cudaMemcpyDeviceToHost, ctx->stream));
-      MG_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-      double sum[4] = {0, 0, 0, 0}, mx[4] = {0, 0, 0, 0};
-      for (int64_t w = 0; w < grid; ++w) for (int i = 0; i < 4; ++i) { sum[i] += (double)h[w * 4 + i]; mx[i] = std::max(mx[i], (double)h[w * 4 + i]); }
-      fprintf(stderr, "mh_balanced: mean cycles/warp wait %.3g load %.3g step %.3g release %.3g | max %.3g %.3g %.3g %.3g\n",
-              sum[0] / grid, sum[1] / grid, sum[2] / grid, sum[3] / grid, mx[0], mx[1], mx[2], mx[3]);
-    }
     return MG_OK;  // queue buffers are freed stream-ordered after the kernel
     }
   }

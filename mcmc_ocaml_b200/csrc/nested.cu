@@ -603,7 +603,7 @@ extern "C" int mg_nested_evidence(mg_ctx *ctx, const mg_logfn *like, const mg_lo
 
   const size_t row_smem = (size_t)2 * 2 * NEST_BLOCK * nest_row_stride(D) * sizeof(double);
   // the shell-in-a-box pair with its parameters in registers (see nest_replace_kernel, FAST)
-  const int fast = (like->kind == MG_FN_SHELL && like->scale == 1.0 && prior->scale == 1.0 && !getenv("MCMC_GPU_NEST_GENERIC"))
+  const int fast = (like->kind == MG_FN_SHELL && like->scale == 1.0 && prior->scale == 1.0)
                        ? (prior->kind == MG_FN_BOX_CLOSED ? 1 : (prior->kind == MG_FN_BOX_OPEN ? 2 : 0)) : 0;
 #define MG_NEST_CASE2(KERNEL, DM, GRID, BLOCK, ...)                                  \
   do {                                                                               \

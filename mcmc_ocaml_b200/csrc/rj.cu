@@ -33,6 +33,9 @@ rj_ensemble_k_kernel(const __grid_constant__ RjArgsT<MG_RJ_MAX_MODELS> a) {
 
 int jit_launch_rj(mg_ctx *ctx, const RjArgs &a, int Dm, unsigned grid, unsigned block, size_t smem);   // jit.cu
 
+// largest tree dimension for which a run enables the per-point draw cache by itself (include/mcmc_gpu.h)
+constexpr int kDrawCacheMaxDim = 8;
+
 template <int NM> static int rj_launch(mg_ctx *, const RjArgsT<NM> &, bool, int, unsigned, int, size_t, cudaStream_t);
 template <> int rj_launch<2>(mg_ctx *ctx, const RjArgsT<2> &a, bool any_user, int Dm, unsigned grid, int block, size_t smem,
                              cudaStream_t s) {
@@ -124,10 +127,8 @@ static int rj_run(mg_ctx *ctx, const mg_rj_model *const *M, int K, const mg_rjmc
     memset(&m.tree, 0, sizeof m.tree);
     if (m.into_kind == MG_INTO_INTERP) {
       // leaf-level Interp.draw through the per-point cell records (kdtree.cu: mg_kdtree_enable_draw_cache)
-      static const bool want_cache = [] { const char *e = getenv("MCMC_GPU_DRAW_CACHE"); return e ? atoi(e) != 0 : true; }();
       mg_kdtree *tr = const_cast<mg_kdtree *>(M[k]->into.tree);
-      static const int cache_maxd = [] { const char *e = getenv("MCMC_GPU_DRAW_CACHE_MAXD"); return e ? atoi(e) : 8; }();
-      if (want_cache && m.nstop == 0 && tr->h.D <= cache_maxd && !tr->d_draw_cache && tr->ctx == ctx && C * (cfg->nbin + n * cfg->nskip) >= tr->h.N) {
+      if (m.nstop == 0 && tr->h.D <= kDrawCacheMaxDim && !tr->d_draw_cache && tr->ctx == ctx && C * (cfg->nbin + n * cfg->nskip) >= tr->h.N) {
         if ((rc = mg_kdtree_enable_draw_cache(tr)) == MG_ENOMEM) rc = MG_OK;   // no room: descend as before
         if (rc) return rc;
       }

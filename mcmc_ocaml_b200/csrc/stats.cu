@@ -27,10 +27,10 @@ constexpr int RED_BLOCK = 256;
 // (tests/test_mcmc_gpu.py::test_resident_call_and_block_stats).
 constexpr int MOM_BLOCK = RED_BLOCK;
 __global__ void __launch_bounds__(MOM_BLOCK)
-block_field_moments_kernel(const double *__restrict__ pivot_src, const double *__restrict__ blk, int64_t n, int F,
-                           int64_t C, double *__restrict__ partial /* [2][F][gridDim.x] */) {
+block_field_moments_kernel(const double *__restrict__ blk, int64_t n, int F, int64_t C,
+                           double *__restrict__ partial /* [2][F][gridDim.x] */) {
   const int f = blockIdx.y;
-  const double sh = pivot_src[(int64_t)f * C];   // pivot: sample 0, chain 0 of the whole block
+  const double sh = blk[(int64_t)f * C];   // pivot: sample 0, chain 0 of the block
   Comp a1, a2;
   const int64_t nvec = C / 2;
   const bool vec_ok = (C % 2 == 0);
@@ -58,17 +58,16 @@ block_field_moments_kernel(const double *__restrict__ pivot_src, const double *_
   }
 }
 
-// partial: [nseg][2][F][nb]
-__global__ void finish_moments_kernel(const double *__restrict__ partial, int nseg, int nb, int F, double cnt,
+// partial: [2][F][nb]
+__global__ void finish_moments_kernel(const double *__restrict__ partial, int nb, int F, double cnt,
                                       const double *__restrict__ blk, int64_t C, double *__restrict__ out) {
   const int f = blockIdx.x * blockDim.x + threadIdx.x;
   if (f >= F) return;
   Comp s1, s2;
-  for (int g = 0; g < nseg; ++g)
-    for (int b = 0; b < nb; ++b) {
-      s1.add(partial[(((int64_t)g * 2 + 0) * F + f) * nb + b]);
-      s2.add(partial[(((int64_t)g * 2 + 1) * F + f) * nb + b]);
-    }
+  for (int b = 0; b < nb; ++b) {
+    s1.add(partial[(int64_t)f * nb + b]);
+    s2.add(partial[((int64_t)F + f) * nb + b]);
+  }
   const double sh = blk[(int64_t)f * C];
   const double S1 = s1.value(), S2 = s2.value();
   out[f] = sh + S1 / cnt;
@@ -136,8 +135,6 @@ static int grid_for(mg_ctx *ctx, int64_t work_items) {
   return (int)(g < 1 ? 1 : g);
 }
 
-int moments_grid(mg_ctx *ctx, int64_t n) { return grid_for(ctx, n); }
-
 // Pool the per-chain running moments of the balanced sampler (mcmc_balanced.cuh, kMom): chain c holds its pivot
 // p_c, S1_c = sum (v - p_c), S2_c = sum (v - p_c)^2 over its n recorded samples.  Chain mean m_c = p_c + S1_c / n,
 // chain M2_c = S2_c - S1_c^2 / n; pooled mean = sum_c m_c / C and M2 = sum_c M2_c + n sum_c (m_c - mean)^2
@@ -169,29 +166,17 @@ int chain_moments_finish(mg_ctx *ctx, cudaStream_t st, const double *mom, int F,
   return MG_OK;
 }
 
-// partial moments of the samples [seg, seg + n) about the block's pivot, on stream `st`
-int sample_block_moments_async(mg_ctx *ctx, cudaStream_t st, const double *blk_base, const double *seg, int64_t n,
-                               int F, int64_t C, int gx, double *partial) {
-  block_field_moments_kernel<<<dim3(gx, F), MOM_BLOCK, 0, st>>>(blk_base, seg, n, F, C, partial);
-  MG_CHECK_LAUNCH(ctx);
-  return MG_OK;
-}
-int sample_block_moments_finish(mg_ctx *ctx, cudaStream_t st, const double *partial, int nseg, int gx, int F, double cnt,
-                                const double *blk_base, int64_t C, double *d_out) {
-  finish_moments_kernel<<<(F + 63) / 64, 64, 0, st>>>(partial, nseg, gx, F, cnt, blk_base, C, d_out);
-  MG_CHECK_LAUNCH(ctx);
-  return MG_OK;
-}
-
 // per-field mean and std of a device sample block; results in d_out[0..F) (mean), d_out[F..2F) (std)
 int sample_block_stats(mg_ctx *ctx, const double *d_blk, int64_t n, int F, int64_t C, double *d_out) {
   cudaStream_t s = ctx->stream;
   const int gx = grid_for(ctx, n);
   DevBuf<double> partial;
   MG_CUDA(ctx, partial.alloc((size_t)2 * F * gx, s));
-  int rc = sample_block_moments_async(ctx, s, d_blk, d_blk, n, F, C, gx, partial.get());
-  if (rc) return rc;
-  return sample_block_moments_finish(ctx, s, partial.get(), 1, gx, F, (double)n * (double)C, d_blk, C, d_out);
+  block_field_moments_kernel<<<dim3(gx, F), MOM_BLOCK, 0, s>>>(d_blk, n, F, C, partial.get());
+  MG_CHECK_LAUNCH(ctx);
+  finish_moments_kernel<<<(F + 63) / 64, 64, 0, s>>>(partial.get(), gx, F, (double)n * (double)C, d_blk, C, d_out);
+  MG_CHECK_LAUNCH(ctx);
+  return MG_OK;
 }
 
 // column mean (pow 1) or std about `d_shift` (pow 2) of a device table [n][D]

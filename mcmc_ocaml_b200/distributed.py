@@ -128,7 +128,7 @@ def broadcast_tree(tree, src: int = 0, ctx=None):
 # ---- distributed kd-tree build: the numbering rule of mg_kdtree_build_distributed (csrc/comm.cu) on the host -------------
 def tree_levels(left: np.ndarray) -> list[int]:
     """First node of every level (and the node count at the end) of a breadth-first tree with adjacent children:
-    the next level ends two past the largest `left` of the level (``kdd_levels_kernel``)."""
+    the next level ends two past the largest `left` of the level."""
     lb, b, e = [0], 0, 1
     while b < e:
         last = int(left[b:e].max())

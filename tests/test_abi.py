@@ -157,3 +157,23 @@ def test_ocaml_externals_have_the_arity_of_their_stubs():
             assert len(stubs) == 1, f"external {name}: {arrows} arguments need no bytecode stub"
         checked += 1
     assert checked >= 20
+
+
+def test_environment_switches_match_design_table():
+    """the MCMC_GPU_* variables the package reads are exactly those DESIGN.md section 7a lists"""
+    import os
+    import re
+    pkg = os.path.dirname(os.path.abspath(_abi.__file__))
+    root = os.path.dirname(pkg)
+    read = set()
+    for d, dirs, files in os.walk(pkg):
+        dirs[:] = [x for x in dirs if x not in ("build", "__pycache__")]
+        for f in files:
+            if f.endswith((".py", ".cu", ".cuh", ".hpp", ".h")):
+                text = open(os.path.join(d, f), encoding="utf-8").read()
+                read |= set(re.findall(r'(?:getenv|os\.environ(?:\.get)?)\s*[(\[]\s*"(MCMC_GPU_\w+)"', text))
+    design = open(os.path.join(root, "DESIGN.md"), encoding="utf-8").read()
+    section = design[design.index("\n## 7a."):]
+    section = section[:section.index("\n## ", 1)]
+    listed = {m for line in section.splitlines() if line.startswith("|") for m in re.findall(r"MCMC_GPU_\w+", line)}
+    assert read == listed, f"read but not listed: {sorted(read - listed)}; listed but not read: {sorted(listed - read)}"

@@ -13,6 +13,8 @@ NCCL id and allocates the test data):
      every rank; both builds timed.
   7. ensemble diagnostics of the chains of step 4, sharded as there (mg_comm_chain_diagnostics): the same bytes on
      every rank, within 1e-12 of the one-GPU call on all chains.  It runs right after step 4, whose chains it uses.
+  8. step 6 on data whose subtree on one rank the second kd-tree builder hands back to the first (a block of
+     identical rows), so that the level table of that rank comes from the first builder.
 Prints one JSON line on rank 0."""
 from __future__ import annotations
 
@@ -195,7 +197,23 @@ def main():
                                          nlevels=int(td.nlevels), distributed_s=min(dt_d), single_gpu_s=min(dt_s),
                                          speedup=min(dt_s) / min(dt_d))
         td.close(); ts.close()
-    del dpts
+    # ---- 8. distributed build with one rank's subtree from the first builder ------------------------------------------
+    # uniform rows with a block of identical rows at 0.25 (left of the root's split, so on rank 0 only): the node that
+    # holds the block sheds only a few rows per level and stays larger than a shared-memory subtree (<= 2048 points)
+    # past the second builder's level budget, which hands the input back (MCMC_GPU_DEBUG=1 prints
+    # "second builder handed the input back" between the rank's "gather" and "subtree" phases)
+    tp = np.random.default_rng(11).random((N, Dm))
+    tp[:max(N // 128, 16384)] = 0.25
+    dtp = torch.from_numpy(tp).to(dev)
+    td = comm.build_tree(dtp.data_ptr(), N, Dm, lo_, hi_, min_split=2)
+    ts = kd_tree.KdTree.from_device(dtp.data_ptr(), N, Dm, lo_, hi_, min_split=2, ctx=ctx)
+    ad, as_ = td.export(), ts.export()
+    same = all(np.array_equal(ad[k_], as_[k_]) for k_ in as_) and td.nnodes == ts.nnodes and td.nlevels == ts.nlevels
+    flags = comm.allgather(np.array([1.0 if same else 0.0]))
+    out["dist_build_first_builder"] = dict(identical_to_single_gpu_on_every_rank=bool(flags.min() == 1.0),
+                                           nnodes=int(td.nnodes), nlevels=int(td.nlevels))
+    td.close(); ts.close()
+    del dpts, dtp
     if rank == 0:
         ctx.set_seed(4711)
         r1 = mcmc.rjmcmc_array(51, A, B, a0, a0, nskip=4, nchains=20000, record_model=False, ctx=ctx)
@@ -206,7 +224,8 @@ def main():
                          and out["harmonic_sharded_rel_err"] < 1e-14 and out["evidence_identical_on_all_ranks"]
                          and out["evidence_bit_identical_to_single_gpu"] and out["rj_counts_equal"]
                          and out["diagnostics_identical_on_all_ranks"] and out["diagnostics_within_1e12_of_single_gpu"]
-                         and all(out[f"dist_build_ms{ms}"]["identical_to_single_gpu_on_every_rank"] for ms in (2, 64)))
+                         and all(out[f"dist_build_ms{ms}"]["identical_to_single_gpu_on_every_rank"] for ms in (2, 64))
+                         and out["dist_build_first_builder"]["identical_to_single_gpu_on_every_rank"])
         s_ = json.dumps(out)
         print(s_)
         if a.out:
