@@ -6,7 +6,8 @@
 // compensated (Neumaier) partial, partials are combined in a fixed order
 // (warp shuffle tree, then one block-order pass), so the result is
 // deterministic and within a few ulp of the exactly rounded sum -- closer to
-// exact than the reference's own sequential sum.  Parity tolerance: 1e-12 rel.
+// exact than the reference's own sequential sum.  The tested error model is in
+// DESIGN.md section S (tests/test_stats_exact_gpu.py).
 // All kernels are HBM-bound: 8 bytes read per element per pass.
 #include "common.cuh"
 #include "models.cuh"
@@ -17,62 +18,162 @@ namespace mg {
 
 constexpr int RED_BLOCK = 256;
 
+// IEEE sum of a compensated accumulator: once an infinity enters, the compensation term turns NaN (inf - inf)
+// while the running sum holds the right +-inf (or NaN where both signs met), so the running sum is the answer.
+__device__ __forceinline__ double comp_sum(const Comp &a) { return isfinite(a.s) ? a.value() : a.s; }
+
+// sqrt of a variance: only a finite negative round-off is clamped to 0; NaN (a non-finite input, or 0/0 at N = 1)
+// stays NaN as in the reference's fold
+__device__ __forceinline__ double std_of_var(double var) { return sqrt(var < 0.0 ? 0.0 : var); }
+
 // ---- sample block [n][F][C] ---------------------------------------------------
-// One pass for both moments: sums of (x - s_f) and (x - s_f)^2 about a pivot
-// s_f (the field's first sample), so that
-//   mean = s + S1/N,   var = (S2 - S1^2/N) / (N - 1)
-// read the 62.9 GB sample block once instead of twice.  With the pivot inside
-// the distribution the subtraction loses less than a digit, and both sums are
-// compensated; agreement with Stats.multi_mean / multi_std stays within 1e-12
-// (tests/test_mcmc_gpu.py::test_resident_call_and_block_stats).
+// One pass for both moments: sums of a = x - p_f and a^2 about a pivot p_f, so that
+//   mean = p + S1/N,   var = (S2 - S1^2/N) / (N - 1)
+// read the 62.9 GB sample block once instead of twice.  S1 and S2 are compensated, so the error of var is
+// dominated by the cancellation in S2 - S1^2/N, about eps (mean - p)^2 / var relative.  The pivot is therefore
+// taken from the data: the finite value nearest the mean of a fixed, evenly spaced subsample of up to PIV_SAMPLES
+// values of the field (block_field_pivot_kernel), so |mean - p| is of order sigma / sqrt(PIV_SAMPLES) however far
+// out any single sample (say an outlying start point in slot 0) lies.  Being a sample, p makes every deviation of a
+// constant field exactly 0.
+// A CTA whose partial sums come out non-finite reads its rows once more to classify the non-finite values, so the
+// finish gives what the reference's fold gives: mean NaN with a NaN or with both infinities, else +-inf with one of them; std NaN with any non-finite
+// value, and NaN for N = 1.
 constexpr int MOM_BLOCK = RED_BLOCK;
-__global__ void __launch_bounds__(MOM_BLOCK)
-block_field_moments_kernel(const double *__restrict__ blk, int64_t n, int F, int64_t C,
-                           double *__restrict__ partial /* [2][F][gridDim.x] */) {
-  const int f = blockIdx.y;
-  const double sh = blk[(int64_t)f * C];   // pivot: sample 0, chain 0 of the block
-  Comp a1, a2;
+constexpr int64_t PIV_SAMPLES = 4096;
+constexpr unsigned NF_NAN = 1u, NF_PINF = 2u, NF_NINF = 4u;
+
+constexpr int64_t PIV_ROWS = 16;
+
+// Subsample value j < R * Q of field f: R = min(n, PIV_ROWS) evenly spaced rows (samples), Q evenly spaced chains in
+// each.  Whole rows keep the reads on a few pages: values scattered over a block of tens of GB cost a page-table
+// walk each.
+__device__ __forceinline__ double pivot_sample(const double *__restrict__ blk, int64_t n, int F, int f, int64_t C,
+                                               int64_t R, int64_t Q, int64_t j) {
+  const int64_t s = (j / Q) * n / R, c = (j % Q) * C / Q;   // products < 2^12 * n, 2^12 * C: no overflow
+  return blk[(s * F + f) * C + c];
+}
+
+// (d, j) lexicographic minimum; "none" is (inf, INT_MAX)
+__device__ __forceinline__ void take_nearer(double &bd, int &bj, double od, int oj) {
+  if (od < bd || (od == bd && oj < bj)) { bd = od; bj = oj; }
+}
+
+// One CTA per field (strided over grid x).  Reads at most 2 * PIV_SAMPLES values per field.
+__global__ void __launch_bounds__(RED_BLOCK)
+block_field_pivot_kernel(const double *__restrict__ blk, int64_t n, int F, int64_t C, double *__restrict__ pivot) {
+  __shared__ double s_mean, s_bd[RED_BLOCK / 32];
+  __shared__ int s_bj[RED_BLOCK / 32];
+  const int64_t R = n < PIV_ROWS ? n : PIV_ROWS, Q = C < PIV_SAMPLES / R ? C : PIV_SAMPLES / R, K = R * Q;
+  for (int f = blockIdx.x; f < F; f += gridDim.x) {
+    Comp sum, cnt;
+    for (int64_t j = threadIdx.x; j < K; j += RED_BLOCK) {
+      const double v = pivot_sample(blk, n, F, f, C, R, Q, j);
+      if (isfinite(v)) { sum.add(v); cnt.add(1.0); }
+    }
+    const double t = block_reduce_comp<RED_BLOCK>(sum);
+    const double m = block_reduce_comp<RED_BLOCK>(cnt);
+    if (threadIdx.x == 0) s_mean = (m > 0.0 && isfinite(t / m)) ? t / m : 0.0;
+    __syncthreads();
+    const double mean = s_mean;
+    double bd = INFINITY;
+    int bj = INT_MAX;
+    for (int64_t j = threadIdx.x; j < K; j += RED_BLOCK) {
+      const double v = pivot_sample(blk, n, F, f, C, R, Q, j);
+      if (isfinite(v)) take_nearer(bd, bj, fabs(v - mean), (int)j);
+    }
+#pragma unroll
+    for (int off = 16; off > 0; off >>= 1)
+      take_nearer(bd, bj, __shfl_down_sync(0xffffffffu, bd, off), __shfl_down_sync(0xffffffffu, bj, off));
+    if ((threadIdx.x & 31) == 0) { s_bd[threadIdx.x >> 5] = bd; s_bj[threadIdx.x >> 5] = bj; }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+      for (int w = 1; w < RED_BLOCK / 32; ++w) take_nearer(bd, bj, s_bd[w], s_bj[w]);
+      pivot[f] = bj == INT_MAX ? 0.0 : pivot_sample(blk, n, F, f, C, R, Q, bj);
+    }
+    __syncthreads();
+  }
+}
+
+// Visit the values of field f in the rows a CTA at grid x position bx owns.  The double2 path needs an even C (rows
+// then start on 16 bytes relative to the base) and a 16-byte aligned base: a caller may pass any device pointer.
+template <class Fn>
+__device__ __forceinline__ void for_each_owned_value(const double *__restrict__ blk, int64_t n, int F, int64_t C,
+                                                     int f, Fn fn) {
   const int64_t nvec = C / 2;
-  const bool vec_ok = (C % 2 == 0);
+  const bool vec_ok = (C % 2 == 0) && (reinterpret_cast<uintptr_t>(blk) % 16 == 0);
   for (int64_t s = blockIdx.x; s < n; s += gridDim.x) {
     const double *row = blk + (s * F + f) * C;
     if (vec_ok) {
       const double2 *row2 = reinterpret_cast<const double2 *>(row);
       for (int64_t c = threadIdx.x; c < nvec; c += MOM_BLOCK) {
         const double2 v = __ldcs(row2 + c);
-        const double a = v.x - sh, b = v.y - sh;
-        a1.add(a); a1.add(b); a2.add(a * a); a2.add(b * b);
+        fn(v.x); fn(v.y);
       }
     } else {
-      for (int64_t c = threadIdx.x; c < C; c += MOM_BLOCK) {
-        const double a = __ldcs(row + c) - sh;
-        a1.add(a); a2.add(a * a);
-      }
+      for (int64_t c = threadIdx.x; c < C; c += MOM_BLOCK) fn(__ldcs(row + c));
     }
-  }
-  const double t1 = block_reduce_comp<MOM_BLOCK>(a1);
-  const double t2 = block_reduce_comp<MOM_BLOCK>(a2);
-  if (threadIdx.x == 0) {
-    partial[(int64_t)f * gridDim.x + blockIdx.x] = t1;
-    partial[((int64_t)F + f) * gridDim.x + blockIdx.x] = t2;
   }
 }
 
-// partial: [2][F][nb]
+// Fields stride over grid y (F may exceed its 65535 limit).  A non-finite value makes the CTA's partials non-finite
+// (an inf or NaN never leaves a compensated sum), which block_field_classify_kernel then looks into.
+__global__ void __launch_bounds__(MOM_BLOCK)
+block_field_moments_kernel(const double *__restrict__ blk, int64_t n, int F, int64_t C,
+                           const double *__restrict__ pivot, double *__restrict__ partial /* [3][F][gridDim.x] */) {
+  for (int f = blockIdx.y; f < F; f += gridDim.y) {
+    const double sh = pivot[f];
+    Comp a1, a2;
+    for_each_owned_value(blk, n, F, C, f, [&](double v) {
+      const double a = v - sh;
+      a1.add(a); a2.add(a * a);
+    });
+    const double t1 = block_reduce_comp<MOM_BLOCK>(a1);
+    const double t2 = block_reduce_comp<MOM_BLOCK>(a2);
+    if (threadIdx.x == 0) {
+      partial[(int64_t)f * gridDim.x + blockIdx.x] = t1;
+      partial[((int64_t)F + f) * gridDim.x + blockIdx.x] = t2;
+    }
+  }
+}
+
+// Same grid as the moments kernel.  A CTA whose partials are finite saw only finite values and records class 0;
+// otherwise it reads its rows again and records which of NaN / +inf / -inf they hold.  The moments pass thus spends
+// nothing on the check, and the second read happens only for a field that holds a non-finite value.
+__global__ void __launch_bounds__(MOM_BLOCK)
+block_field_classify_kernel(const double *__restrict__ blk, int64_t n, int F, int64_t C,
+                            double *__restrict__ partial /* [3][F][gridDim.x] */) {
+  for (int f = blockIdx.y; f < F; f += gridDim.y) {
+    const int64_t i = (int64_t)f * gridDim.x + blockIdx.x;
+    unsigned cls = 0;
+    if (!isfinite(partial[i]) || !isfinite(partial[(int64_t)F * gridDim.x + i])) {
+      unsigned nf = 0;
+      for_each_owned_value(blk, n, F, C, f, [&](double v) {
+        if (!isfinite(v)) nf |= isnan(v) ? NF_NAN : (v > 0.0 ? NF_PINF : NF_NINF);
+      });
+      cls = (__syncthreads_or(nf & NF_NAN) ? NF_NAN : 0u) | (__syncthreads_or(nf & NF_PINF) ? NF_PINF : 0u) |
+            (__syncthreads_or(nf & NF_NINF) ? NF_NINF : 0u);
+    }
+    if (threadIdx.x == 0) partial[(int64_t)2 * F * gridDim.x + i] = (double)cls;
+  }
+}
+
+// partial: [3][F][nb]
 __global__ void finish_moments_kernel(const double *__restrict__ partial, int nb, int F, double cnt,
-                                      const double *__restrict__ blk, int64_t C, double *__restrict__ out) {
+                                      const double *__restrict__ pivot, double *__restrict__ out) {
   const int f = blockIdx.x * blockDim.x + threadIdx.x;
   if (f >= F) return;
   Comp s1, s2;
+  unsigned cls = 0;
   for (int b = 0; b < nb; ++b) {
     s1.add(partial[(int64_t)f * nb + b]);
     s2.add(partial[((int64_t)F + f) * nb + b]);
+    cls |= (unsigned)partial[((int64_t)2 * F + f) * nb + b];
   }
-  const double sh = blk[(int64_t)f * C];
   const double S1 = s1.value(), S2 = s2.value();
-  out[f] = sh + S1 / cnt;
-  const double var = (S2 - S1 * (S1 / cnt)) / (cnt - 1.0);
-  out[F + f] = sqrt(var > 0.0 ? var : 0.0);
+  if ((cls & NF_NAN) || (cls & (NF_PINF | NF_NINF)) == (NF_PINF | NF_NINF)) out[f] = NAN;
+  else if (cls) out[f] = (cls & NF_PINF) ? INFINITY : -INFINITY;
+  else out[f] = pivot[f] + S1 / cnt;
+  out[F + f] = cls ? NAN : std_of_var(fma(-S1, S1 / cnt, S2) / (cnt - 1.0));
 }
 
 // ---- row-major table [n][D]: column sums ----------------------------------
@@ -89,12 +190,12 @@ __global__ void table_col_reduce_kernel(const double *__restrict__ xs, int64_t t
     const double a = xs[k] - sh;
     acc.add(POW == 1 ? a : a * a);
   }
-  sm[threadIdx.x] = acc.value();
+  sm[threadIdx.x] = comp_sum(acc);
   __syncthreads();
   if ((int)threadIdx.x < D) {
     Comp t;
     for (int k = threadIdx.x; k < (int)blockDim.x; k += D) t.add(sm[k]);
-    partial[(int64_t)blockIdx.x * D + threadIdx.x] = t.value();
+    partial[(int64_t)blockIdx.x * D + threadIdx.x] = comp_sum(t);
   }
 }
 __global__ void finish_cols_kernel(const double *__restrict__ partial, int nb, int D, double denom, int do_sqrt,
@@ -103,22 +204,24 @@ __global__ void finish_cols_kernel(const double *__restrict__ partial, int nb, i
   if (d >= D) return;
   Comp acc;
   for (int b = 0; b < nb; ++b) acc.add(partial[(int64_t)b * D + d]);
-  const double v = acc.value() / denom;
+  const double v = comp_sum(acc) / denom;
   out[d] = do_sqrt ? sqrt(v) : v;
 }
 
-// ---- autocorrelation (stats.ml:223-238), one block row per lag -------------
+// ---- autocorrelation (stats.ml:223-238), lags strided over grid y (nslides may exceed its 65535 limit) ----
 __global__ void __launch_bounds__(RED_BLOCK)
-autocorr_kernel(const double *__restrict__ x, int64_t n, double mu, double sigma2, double *__restrict__ partial) {
-  const int lag = blockIdx.y;
-  Comp acc;
-  const int64_t m = n - lag;
-  for (int64_t j = (int64_t)blockIdx.x * RED_BLOCK + threadIdx.x; j < m; j += (int64_t)gridDim.x * RED_BLOCK) {
-    const double dx = x[j] - mu, dxs = x[j + lag] - mu;
-    acc.add(dx * dxs / sigma2);
+autocorr_kernel(const double *__restrict__ x, int64_t n, int nslides, double mu, double sigma2,
+                double *__restrict__ partial) {
+  for (int lag = blockIdx.y; lag < nslides; lag += gridDim.y) {
+    Comp acc;
+    const int64_t m = n - lag;
+    for (int64_t j = (int64_t)blockIdx.x * RED_BLOCK + threadIdx.x; j < m; j += (int64_t)gridDim.x * RED_BLOCK) {
+      const double dx = x[j] - mu, dxs = x[j + lag] - mu;
+      acc.add(dx * dxs / sigma2);
+    }
+    const double tot = block_reduce_comp<RED_BLOCK>(acc);
+    if (threadIdx.x == 0) partial[(int64_t)lag * gridDim.x + blockIdx.x] = tot;
   }
-  const double tot = block_reduce_comp<RED_BLOCK>(acc);
-  if (threadIdx.x == 0) partial[(int64_t)lag * gridDim.x + blockIdx.x] = tot;
 }
 __global__ void finish_autocorr_kernel(const double *__restrict__ partial, int nb, int nslides, int64_t n,
                                        double *__restrict__ out) {
@@ -128,6 +231,8 @@ __global__ void finish_autocorr_kernel(const double *__restrict__ partial, int n
   for (int b = 0; b < nb; ++b) acc.add(partial[(int64_t)lag * nb + b]);
   out[lag] = acc.value() / (double)(n - lag);
 }
+
+constexpr int64_t GRID_Y_MAX = 65535;
 
 static int grid_for(mg_ctx *ctx, int64_t work_items) {
   int64_t g = (int64_t)ctx->sm_count * 8;
@@ -157,7 +262,7 @@ chain_moments_finish_kernel(const double *__restrict__ mom, int F, int64_t C, do
     m2.add(n * d * d);
   }
   const double M2 = block_reduce_comp<RED_BLOCK>(m2);
-  if (threadIdx.x == 0) { out[f] = mu; out[F + f] = sqrt(M2 / (n * (double)C - 1.0)); }   // stats.ml:85 (n - 1)
+  if (threadIdx.x == 0) { out[f] = mu; out[F + f] = std_of_var(M2 / (n * (double)C - 1.0)); }   // stats.ml:85 (n - 1)
 }
 
 int chain_moments_finish(mg_ctx *ctx, cudaStream_t st, const double *mom, int F, int64_t C, int64_t n, double *d_out) {
@@ -170,11 +275,17 @@ int chain_moments_finish(mg_ctx *ctx, cudaStream_t st, const double *mom, int F,
 int sample_block_stats(mg_ctx *ctx, const double *d_blk, int64_t n, int F, int64_t C, double *d_out) {
   cudaStream_t s = ctx->stream;
   const int gx = grid_for(ctx, n);
-  DevBuf<double> partial;
-  MG_CUDA(ctx, partial.alloc((size_t)2 * F * gx, s));
-  block_field_moments_kernel<<<dim3(gx, F), MOM_BLOCK, 0, s>>>(d_blk, n, F, C, partial.get());
+  DevBuf<double> partial, pivot;
+  MG_CUDA(ctx, partial.alloc((size_t)3 * F * gx, s));
+  MG_CUDA(ctx, pivot.alloc((size_t)F, s));
+  block_field_pivot_kernel<<<F, RED_BLOCK, 0, s>>>(d_blk, n, F, C, pivot.get());
   MG_CHECK_LAUNCH(ctx);
-  finish_moments_kernel<<<(F + 63) / 64, 64, 0, s>>>(partial.get(), gx, F, (double)n * (double)C, d_blk, C, d_out);
+  const dim3 grid(gx, (unsigned)std::min<int64_t>(F, GRID_Y_MAX));
+  block_field_moments_kernel<<<grid, MOM_BLOCK, 0, s>>>(d_blk, n, F, C, pivot.get(), partial.get());
+  MG_CHECK_LAUNCH(ctx);
+  block_field_classify_kernel<<<grid, MOM_BLOCK, 0, s>>>(d_blk, n, F, C, partial.get());
+  MG_CHECK_LAUNCH(ctx);
+  finish_moments_kernel<<<(F + 63) / 64, 64, 0, s>>>(partial.get(), gx, F, (double)n * (double)C, pivot.get(), d_out);
   MG_CHECK_LAUNCH(ctx);
   return MG_OK;
 }
@@ -278,7 +389,8 @@ extern "C" int mg_stats_autocorrelation(mg_ctx *ctx, const double *x, int64_t n,
   const int gx = grid_for(ctx, (n + RED_BLOCK - 1) / RED_BLOCK);
   MG_CUDA(ctx, d_partial.alloc((size_t)gx * nslides, s));
   MG_CUDA(ctx, d_out.alloc(nslides, s));
-  autocorr_kernel<<<dim3(gx, nslides), RED_BLOCK, 0, s>>>(d_x.get(), n, ms[0], sigma2, d_partial.get());
+  autocorr_kernel<<<dim3(gx, (unsigned)std::min<int64_t>(nslides, GRID_Y_MAX)), RED_BLOCK, 0, s>>>(
+      d_x.get(), n, nslides, ms[0], sigma2, d_partial.get());
   MG_CHECK_LAUNCH(ctx);
   finish_autocorr_kernel<<<(nslides + 63) / 64, 64, 0, s>>>(d_partial.get(), gx, nslides, n, d_out.get());
   MG_CHECK_LAUNCH(ctx);
