@@ -225,14 +225,12 @@ extern "C" int mg_kdtree_broadcast(mg_comm *c, mg_kdtree *tree, int32_t root, mg
   // announced size if that is at all possible, then judge
   const bool sane = h.magic == KD_MAGIC && h.nbytes >= (int64_t)HB && h.nbytes < (1LL << 40);
   if (!sane) return set_err(ctx, MG_EFAIL, "kdtree_broadcast: the root sent no kd-tree header");
-  mg_kdtree *t = new mg_kdtree;
-  t->ctx = ctx; t->h = h;
-  cudaError_t e = cudaMallocAsync(&t->d_blob, (size_t)h.nbytes, s);
-  if (e != cudaSuccess) { delete t; return set_err(ctx, MG_ENOMEM, "cuda: %s (kd-tree blob of %lld bytes)", cudaGetErrorString(e), (long long)h.nbytes); }
+  KdTreePtr t;
+  if ((rc = kd_alloc(ctx, h, &t))) return rc;
   rc = comm_broadcast_dev(c, t->d_blob, (size_t)h.nbytes, root);
   if (rc == MG_OK) { tm.stop(); rc = validate_blob_header(ctx, h); }
-  if (rc) { cudaFreeAsync(t->d_blob, s); delete t; return rc; }
-  *out = t;
+  if (rc) return rc;
+  *out = t.release();
   return MG_OK;
 }
 
@@ -361,9 +359,6 @@ extern "C" int mg_comm_pool_moments(mg_comm *c, int64_t n_local, const double *m
 // 4096 points per rank or a rank count that is not a power of two are built by every rank for itself.
 namespace mg {
 
-int build_tree(mg_ctx *ctx, const double *d_pts, int64_t N, int D, const double *low, const double *high, int min_split,
-               mg_kdtree **out);   // kdtree.cu
-
 constexpr int KDD_MAXL = 96;         // levels of a subtree
 constexpr int KDD_MAXR = 64;         // ranks
 
@@ -407,24 +402,17 @@ __global__ void kdd_unpack_perm_kernel(const KddTables *__restrict__ T, int r, c
   perm[b + j] = top_perm[b + reinterpret_cast<const int32_t *>(chunk + T->off_perm[r])[j]];
 }
 
-struct KdGuard { mg_kdtree *t = nullptr; ~KdGuard() { if (t) mg_kdtree_destroy(t); } };
-
-}  // namespace mg
-
-extern "C" int mg_kdtree_build_distributed(mg_comm *c, const double *d_pts, int64_t N, int32_t D, const double *low,
-                                           const double *high, int32_t min_split, mg_kdtree **out) {
-  if (!c) return MG_EINVAL;
+int build_tree_distributed(mg_comm *c, const double *d_pts, int64_t N, int D, const double *low, const double *high,
+                           int min_split, bool with_pts, KdTreePtr *out) {
   mg_ctx *ctx = c->ctx;
-  MG_REQUIRE(ctx, d_pts && low && high && out, "kd-tree (distributed): null argument");
   MG_CUDA(ctx, cudaSetDevice(ctx->device));
-  *out = nullptr;
   if (min_split < 2) min_split = 2;
   const int R = c->nranks;
   int k = 0;
   while ((1 << k) < R) ++k;
   const int64_t ms_top = (N >> k) + 3;           // no node of level k reaches it, every node above does (without ties)
   const bool shard = R > 1 && (1 << k) == R && R <= KDD_MAXR && N / R >= 4096 && (int64_t)min_split < ms_top && ms_top < (1LL << 31);
-  if (!shard) return build_tree(ctx, d_pts, N, D, low, high, min_split, out);
+  if (!shard) return build_tree(ctx, d_pts, N, D, low, high, min_split, with_pts, out);
   cudaStream_t s = ctx->stream;
   int rc;
   static const bool dbg = getenv("MCMC_GPU_DEBUG") != nullptr;
@@ -449,40 +437,20 @@ extern "C" int mg_kdtree_build_distributed(mg_comm *c, const double *d_pts, int6
   // gets the block of its previous tree back, where a late request for 2 GB in one piece makes the stream-ordered
   // pool remap its fragments (measured: 15-180 ms).  Truncated trees (min_split > 16) are small next to that bound and
   // get an exact blob at the end instead.
-  auto al = [](int64_t x) { return (x + 255) & ~255LL; };
-  const bool result_with_pts = !ctx->kd_no_pts;    // (internal callers that keep the rows themselves)
-  auto layout = [&](KdHeader &h, int64_t node_cap) {
-    int64_t off = al(sizeof(KdHeader));
-    h.off_low = off; off = al(off + 8 * D);
-    h.off_high = off; off = al(off + 8 * D);
-    h.off_nodes = off; off = al(off + 16 * node_cap);
-    h.off_count = off; off = al(off + 4 * node_cap);
-    h.off_begin = off; off = al(off + 4 * node_cap);
-    h.off_perm = off; off = al(off + 4 * N);
-    h.off_pts = off; off = al(off + (result_with_pts ? 8 * N * D : 0));
-    h.nbytes = off;
-  };
-  KdGuard res;
+  KdTreePtr res;
   const bool early = min_split <= 16;
-  if (early) {
-    res.t = new mg_kdtree;
-    res.t->ctx = ctx;
-    layout(res.t->h, 2 * N);
-    cudaError_t e = cudaMallocAsync(&res.t->d_blob, (size_t)res.t->h.nbytes, s);
-    if (e != cudaSuccess) { res.t->d_blob = nullptr; return set_err(ctx, MG_ENOMEM, "cuda: %s (kd-tree blob of %lld bytes)", cudaGetErrorString(e), (long long)res.t->h.nbytes); }
-  }
+  if (early && (rc = kd_alloc(ctx, kd_layout(N, D, 2 * N, with_pts), &res))) return rc;
   // ---- 1. the top, on every rank ---------------------------------------------------------------------------------------
-  KdGuard top, sub;
   // (the top and the subtree are scaffolding: their blobs carry no copy of the points)
-  struct NoPts { mg_ctx *c; bool was; explicit NoPts(mg_ctx *c_) : c(c_), was(c_->kd_no_pts) { c->kd_no_pts = true; } ~NoPts() { c->kd_no_pts = was; } };
-  { NoPts np(ctx); rc = build_tree(ctx, d_pts, N, D, low, high, (int)ms_top, &top.t); }
+  KdTreePtr top, sub;
+  rc = build_tree(ctx, d_pts, N, D, low, high, (int)ms_top, false, &top);
   // A rank that fails here still takes part in the agreement below (as "not complete"): every rank then builds alone
   // and the failing rank reports its own error, instead of the others waiting in a collective for ever.
   const int rc_top = rc;
   phase("top build");
   static const KdHeader no_header{};
-  const KdHeader &th = rc_top == MG_OK ? top.t->h : no_header;
-  const char *tb = rc_top == MG_OK ? (const char *)top.t->d_blob : nullptr;
+  const KdHeader &th = rc_top == MG_OK ? top->h : no_header;
+  const char *tb = rc_top == MG_OK ? (const char *)top->d_blob : nullptr;
   std::vector<KdNode> tnodes((size_t)th.nnodes);
   std::vector<int32_t> tcount((size_t)th.nnodes), tbegin((size_t)th.nnodes);
   bool complete = rc_top == MG_OK && th.nnodes == 2 * (int64_t)R - 1;
@@ -502,7 +470,7 @@ extern "C" int mg_kdtree_build_distributed(mg_comm *c, const double *d_pts, int6
     if ((rc = mg_comm_allgather(c, &mine, all.data(), sizeof mine))) return rc;
     for (int r = 0; r < R; ++r) complete = complete && all[r] == 1;
   }
-  if (!complete) return rc_top != MG_OK ? rc_top : build_tree(ctx, d_pts, N, D, low, high, min_split, out);
+  if (!complete) return rc_top != MG_OK ? rc_top : build_tree(ctx, d_pts, N, D, low, high, min_split, with_pts, out);
   phase("top");
   // ---- 2. this rank's subtree -------------------------------------------------------------------------------------------
   const int me = c->rank;
@@ -513,15 +481,15 @@ extern "C" int mg_kdtree_build_distributed(mg_comm *c, const double *d_pts, int6
   kdd_gather_rows_kernel<<<(unsigned)(((int64_t)my_n * D + 255) / 256), 256, 0, s>>>(d_pts, top_perm + my_b, my_n, D, rows.get());
   MG_CHECK_LAUNCH(ctx);
   phase("gather");
-  { NoPts np(ctx); rc = build_tree(ctx, rows.get(), my_n, D, low, high, min_split, &sub.t); }
+  rc = build_tree(ctx, rows.get(), my_n, D, low, high, min_split, false, &sub);
   const int rc_sub = rc;                         // a failure travels in the record below, so that no rank is left waiting
   phase("subtree");
-  const KdHeader &sh = rc_sub == MG_OK ? sub.t->h : no_header;
-  const char *sb = rc_sub == MG_OK ? (const char *)sub.t->d_blob : nullptr;
+  const KdHeader &sh = rc_sub == MG_OK ? sub->h : no_header;
+  const char *sb = rc_sub == MG_OK ? (const char *)sub->d_blob : nullptr;
   struct Rec { int32_t nl, nn, npts, pbegin; int32_t lb[KDD_MAXL + 1]; int32_t bad; };
   Rec mine{};
   if (rc_sub == MG_OK) {                         // the builder's level table, cut at KDD_MAXL levels (then flagged below)
-    const std::vector<int32_t> &lvb = sub.t->level_begin;
+    const std::vector<int32_t> &lvb = sub->level_begin;
     mine.nl = (int32_t)std::min<size_t>(lvb.size() - 1, KDD_MAXL);
     for (int l = 0; l <= mine.nl; ++l) mine.lb[l] = lvb[l];
   }
@@ -543,9 +511,9 @@ extern "C" int mg_kdtree_build_distributed(mg_comm *c, const double *d_pts, int6
     memcpy(T.lb[r], q.lb, sizeof q.lb);
     for (int l = q.nl + 1; l <= KDD_MAXL; ++l) T.lb[r][l] = q.nn;
     maxl = std::max(maxl, (int)q.nl);
-    auto al = [](int64_t x) { return (x + 255) & ~255LL; };
-    T.off_count[r] = al(16LL * q.nn); T.off_begin[r] = al(T.off_count[r] + 4LL * q.nn); T.off_perm[r] = al(T.off_begin[r] + 4LL * q.nn);
-    chunk = std::max<int64_t>(chunk, al(T.off_perm[r] + 4LL * q.npts));
+    T.off_count[r] = align256(16LL * q.nn); T.off_begin[r] = align256(T.off_count[r] + 4LL * q.nn);
+    T.off_perm[r] = align256(T.off_begin[r] + 4LL * q.nn);
+    chunk = std::max<int64_t>(chunk, align256(T.off_perm[r] + 4LL * q.npts));
   }
   T.gbase[0] = R - 1;                               // level k of the whole tree starts after the 2^k - 1 nodes above it
   for (int l = 0; l <= maxl; ++l) {
@@ -569,22 +537,12 @@ extern "C" int mg_kdtree_build_distributed(mg_comm *c, const double *d_pts, int6
     tm.stop();
   }
   phase("allgather");
-  // ---- the blob (layout of the single-GPU builders) -----------------------------------------------------------------------
-  if (!early) {
-    res.t = new mg_kdtree;
-    res.t->ctx = ctx;
-    layout(res.t->h, nnodes);
-    cudaError_t e = cudaMallocAsync(&res.t->d_blob, (size_t)res.t->h.nbytes, s);
-    if (e != cudaSuccess) { res.t->d_blob = nullptr; return set_err(ctx, MG_ENOMEM, "cuda: %s (kd-tree blob of %lld bytes)", cudaGetErrorString(e), (long long)res.t->h.nbytes); }
-  }
-  mg_kdtree *tr = res.t;
-  KdHeader &h = tr->h;
-  h.magic = KD_MAGIC; h.N = N; h.nnodes = nnodes; h.D = D; h.nlevels = k + maxl; h.min_split = min_split;
-  char *blob = (char *)tr->d_blob;
+  // ---- the blob: the nodes of the top, then every rank's subtree ------------------------------------------------------------
+  if (!early && (rc = kd_alloc(ctx, kd_layout(N, D, nnodes, with_pts), &res))) return rc;
+  KdHeader &h = res->h;
+  h.nnodes = nnodes; h.nlevels = k + maxl; h.min_split = min_split;
+  char *blob = (char *)res->d_blob;
   phase("blob alloc");
-  MG_CUDA(ctx, cudaMemcpyAsync(blob, &tr->h, sizeof(KdHeader), cudaMemcpyHostToDevice, s));
-  MG_CUDA(ctx, cudaMemcpyAsync(blob + h.off_low, low, 8 * D, cudaMemcpyHostToDevice, s));
-  MG_CUDA(ctx, cudaMemcpyAsync(blob + h.off_high, high, 8 * D, cudaMemcpyHostToDevice, s));
   // the 2^k - 1 nodes above the subtrees: numbers, counts and positions are those of the top tree
   MG_CUDA(ctx, cudaMemcpyAsync(blob + h.off_nodes, tb + th.off_nodes, 16 * (size_t)(R - 1), cudaMemcpyDeviceToDevice, s));
   MG_CUDA(ctx, cudaMemcpyAsync(blob + h.off_count, tb + th.off_count, 4 * (size_t)(R - 1), cudaMemcpyDeviceToDevice, s));
@@ -598,12 +556,21 @@ extern "C" int mg_kdtree_build_distributed(mg_comm *c, const double *d_pts, int6
     MG_CHECK_LAUNCH(ctx);
   }
   phase("unpack");
-  if (result_with_pts) MG_CUDA(ctx, cudaMemcpyAsync(blob + h.off_pts, d_pts, 8 * (size_t)N * D, cudaMemcpyDeviceToDevice, s));
-  MG_CUDA(ctx, cudaStreamSynchronize(s));
-  phase("pts copy");
-  res.t = nullptr;
-  *out = tr;
-  return MG_OK;
+  rc = kd_finish(ctx, std::move(res), low, high, d_pts, out);
+  phase("finish");
+  return rc;
+}
+
+}  // namespace mg
+
+extern "C" int mg_kdtree_build_distributed(mg_comm *c, const double *d_pts, int64_t N, int32_t D, const double *low,
+                                           const double *high, int32_t min_split, mg_kdtree **out) {
+  if (!c) return MG_EINVAL;
+  MG_REQUIRE(c->ctx, d_pts && low && high && out, "kd-tree (distributed): null argument");
+  KdTreePtr t;
+  const int rc = build_tree_distributed(c, d_pts, N, D, low, high, min_split, true, &t);
+  *out = t.release();
+  return rc;
 }
 
 // Ensemble diagnostics (diagnostics.cu) of chains sharded over the ranks: every rank runs the local pass on its own

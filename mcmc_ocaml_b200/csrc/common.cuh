@@ -27,8 +27,6 @@ struct mg_ctx {
   int64_t naccept = 0, nreject = 0;  // Mcmc.get_counters (mcmc.ml:27-35)
   int64_t rj_cross[2] = {0, 0};      // last mg_rjmcmc_array: cross-model proposals, of which accepted
   int sm_count = 148;
-  double *mh_mom = nullptr;        // request: per-chain running moments from the next MH launch (mcmc_balanced.cuh)
-  bool mh_mom_done = false;        // answer: the launch produced them
   // per-launch timing of the dominant kernel of the last call (bench.py roofline): event pairs on the context's
   // stream around EVERY launch of that kernel, collected lazily by mg_ctx_last_kernel_stats
   std::vector<cudaEvent_t> kt_ev;
@@ -40,7 +38,6 @@ struct mg_ctx {
   mg_nested_observer nest_observer = nullptr;   // Nested ?observer (nested.ml:123-125)
   void *nest_observer_user = nullptr;
   int *d_devflag = nullptr;        // device word set by a kernel whose bounded spin-wait ran out (MG_DEVERR_*)
-  bool kd_no_pts = false;          // internal (distributed build): the next kd-tree blob carries no copy of the points
   int sticky = MG_OK;              // a device-side failure that every later call reports until mg_ctx_clear_error
   std::string err;
 };

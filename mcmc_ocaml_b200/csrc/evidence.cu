@@ -27,9 +27,6 @@
 
 namespace mg {
 
-int build_tree(mg_ctx *ctx, const double *d_pts, int64_t N, int D, const double *low, const double *high,
-               int min_split, mg_kdtree **out);  // kdtree.cu
-
 __global__ void neg_ll_keys_kernel(const double *__restrict__ ll, int64_t n, uint64_t *__restrict__ keys,
                                    int32_t *__restrict__ vals) {
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
@@ -250,24 +247,17 @@ int sum_terms(mg_ctx *ctx, const double *d_terms, int64_t nn, double *out) {
   return reduce_sum(ctx, nn, [d_terms] __device__(int64_t i) { return d_terms[i]; }, out);
 }
 
-// tree of the survivors (not split below nmax)
-static int survivors_tree(mg_ctx *ctx, const Survivors &sv, int D, int nmax, mg_kdtree **t) {
-  std::vector<double> zeros(D, 0.0);
-  // The root box (bounds_of_objects, evidence.ml:164,206) does not influence
-  // any split nor the tight per-cell volumes, so it is not computed.
-  // (the tree is scaffolding here: the cell terms read the survivors' own rows, so the blob carries no copy of them)
-  ctx->kd_no_pts = true;
-  const int rc = build_tree(ctx, sv.pts.get(), sv.K, D, zeros.data(), zeros.data(), nmax < 2 ? 2 : nmax, t);
-  ctx->kd_no_pts = false;
-  return rc;
-}
-
 // tree of the survivors and the sum of the per-cell terms
 template <int MODE>
 static int integrate_cells(mg_ctx *ctx, const Survivors &sv, int D, int nmax, double *out, int64_t *ncells_out) {
   cudaStream_t s = ctx->stream;
-  mg_kdtree *t = nullptr;
-  int rc = survivors_tree(ctx, sv, D, nmax, &t);
+  // The root box (bounds_of_objects, evidence.ml:164,206) does not influence
+  // any split nor the tight per-cell volumes, so it is not computed.
+  // The tree is not split below nmax objects, and it is scaffolding: the cell terms read the survivors' own rows, so
+  // its blob carries no copy of them.
+  std::vector<double> zeros(D, 0.0);
+  KdTreePtr t;
+  int rc = build_tree(ctx, sv.pts.get(), sv.K, D, zeros.data(), zeros.data(), nmax < 2 ? 2 : nmax, false, &t);
   if (rc) return rc;
   const int64_t nn = t->h.nnodes;
   DevBuf<double> terms;
@@ -275,8 +265,8 @@ static int integrate_cells(mg_ctx *ctx, const Survivors &sv, int D, int nmax, do
   cudaError_t e = terms.alloc((size_t)nn, s);
   if (e == cudaSuccess) e = ncells.alloc(1, s);
   if (e == cudaSuccess) e = cudaMemsetAsync(ncells.get(), 0, 8, s);
-  if (e != cudaSuccess) { mg_kdtree_destroy(t); return set_err(ctx, MG_ECUDA, "cuda: %s", cudaGetErrorString(e)); }
-  rc = cell_terms_range<MODE>(ctx, t, sv.pts.get(), sv.ll.get(), sv.lp.get(), nmax, 0, nn, terms.get(), ncells.get());
+  if (e != cudaSuccess) return set_err(ctx, MG_ECUDA, "cuda: %s", cudaGetErrorString(e));
+  rc = cell_terms_range<MODE>(ctx, t.get(), sv.pts.get(), sv.ll.get(), sv.lp.get(), nmax, 0, nn, terms.get(), ncells.get());
   if (rc == MG_OK) rc = sum_terms(ctx, terms.get(), nn, out);
   unsigned long long nc = 0;
   if (rc == MG_OK && ncells_out) {
@@ -285,7 +275,6 @@ static int integrate_cells(mg_ctx *ctx, const Survivors &sv, int D, int nmax, do
     if (e != cudaSuccess) rc = set_err(ctx, MG_ECUDA, "cuda: %s (evidence cells)", cudaGetErrorString(e));
     *ncells_out = (int64_t)nc;
   }
-  mg_kdtree_destroy(t);
   return rc;
 }
 
@@ -475,7 +464,6 @@ static int evidence_sharded(mg_comm *c, int which, int32_t root, const double *d
   int rc = MG_OK;
   Survivors sv;
   double head[3] = {0.0, 0.0, 0.0};   // {mean 1/L of the kept prefix, status of the root's preparation, survivors}
-  mg_kdtree *t = nullptr;
   if (rank == root) {
     double mean_il = 1.0;
     rc = which == 0 ? lebesgue_prepare(ctx, d_pts, d_ll, d_lp, N, D, n, eps, sv, &mean_il)
@@ -493,7 +481,7 @@ static int evidence_sharded(mg_comm *c, int which, int32_t root, const double *d
   if (head[1] != 0.0)
     return rank == root ? rc : set_err(ctx, (int)head[1], "evidence (sharded): the root rank failed to prepare the samples");
   // the survivors (rows, lp, and ll for the direct estimator) go to every rank; the tree over them is then built by
-  // all ranks together (mg_kdtree_build_distributed: top levels everywhere, one subtree per rank, one all-gather)
+  // all ranks together (build_tree_distributed: top levels everywhere, one subtree per rank, one all-gather)
   const int64_t K = (int64_t)head[2];
   if (rank != root) {
     sv.K = K;
@@ -506,12 +494,11 @@ static int evidence_sharded(mg_comm *c, int which, int32_t root, const double *d
   if (rc == MG_OK) rc = comm_broadcast_dev(c, sv.lp.get(), sizeof(double) * (size_t)K, root);
   if (rc == MG_OK && which == 1) rc = comm_broadcast_dev(c, sv.ll.get(), sizeof(double) * (size_t)K, root);
   if (rc) return rc;
+  KdTreePtr t;
   {
-    std::vector<double> zeros(D, 0.0);            // the root box takes no part in the evidence (see survivors_tree)
-    ctx->kd_no_pts = true;                        // the cell terms read the survivors' rows, not a copy inside the blob
-    rc = mg_kdtree_build_distributed(c, sv.pts.get(), K, D, zeros.data(), zeros.data(), n < 2 ? 2 : n, &t);
-    ctx->kd_no_pts = false;
-    if (rc) return rc;
+    std::vector<double> zeros(D, 0.0);            // the root box takes no part in the evidence (see integrate_cells)
+    // the cell terms read the survivors' rows, not a copy inside the blob
+    if ((rc = build_tree_distributed(c, sv.pts.get(), K, D, zeros.data(), zeros.data(), n < 2 ? 2 : n, false, &t))) return rc;
   }
   const int64_t nn = t->h.nnodes;
   const double *sll = sv.ll.get(), *slp = sv.lp.get();
@@ -528,12 +515,11 @@ static int evidence_sharded(mg_comm *c, int which, int32_t root, const double *d
     if (e != cudaSuccess) rc = set_err(ctx, MG_ENOMEM, "cuda: %s", cudaGetErrorString(e));
   }
   if (rc == MG_OK)
-    rc = which == 0 ? cell_terms_range<0>(ctx, t, sv.pts.get(), sll, slp, n, n0, n1, terms.get(), ncells.get())
-                    : cell_terms_range<1>(ctx, t, sv.pts.get(), sll, slp, n, n0, n1, terms.get(), ncells.get());
+    rc = which == 0 ? cell_terms_range<0>(ctx, t.get(), sv.pts.get(), sll, slp, n, n0, n1, terms.get(), ncells.get())
+                    : cell_terms_range<1>(ctx, t.get(), sv.pts.get(), sll, slp, n, n0, n1, terms.get(), ncells.get());
   if (rc == MG_OK) rc = comm_allgather_dev(c, terms.get() + (size_t)rank * slice, terms.get(), sizeof(double) * (size_t)slice);
   double total = 0.0;
   if (rc == MG_OK) rc = sum_terms(ctx, terms.get(), nn, &total);
-  mg_kdtree_destroy(t);
   if (rc) return rc;
   *out = which == 0 ? total / head[0] : total;
   return MG_OK;

@@ -155,17 +155,16 @@ static int get_module(mg_ctx *ctx, int dmax, JitMod *out) {
 
 static int dmax_for(int D) { return D <= 2 ? 2 : D <= 4 ? 4 : D <= 8 ? 8 : D <= 16 ? 16 : D <= 32 ? 32 : 64; }
 
-// MH ensemble with user-registered log-densities (called from mg_mcmc_array_dev)
-int jit_launch_mh(mg_ctx *ctx, const DynFnParams &like, const DynFnParams &prior, const DynPropParams &prop,
-                  const mg_mcmc_cfg *cfg, CallKey key, uint64_t t0, int record_first, double *d_state, double *d_samples, int32_t *d_accept) {
-  const int dmax = dmax_for(cfg->dim);
+// MH ensemble with user-registered log-densities (called from mg_mcmc_array_dev); it keeps no running moments
+int jit_launch_mh(mg_ctx *ctx, const DynFnParams &like, const DynFnParams &prior, const DynPropParams &prop, const MhLaunch &L) {
+  const int dmax = dmax_for(L.cfg->dim);
   JitMod m;
   int rc = get_module(ctx, dmax, &m);
   if (rc) return rc;
   // MhArgs has the same layout for every DMAX (the template parameter only sizes registers)
   MhArgs<DynFn, DynFn, DynProp, 2> a;
   a.like = like; a.prior = prior; a.prop = prop;
-  fill_common(a, cfg, key, t0, record_first, d_state, d_samples, d_accept);
+  fill_common(a, L);
   void *params[] = {&a};
   const unsigned grid = (unsigned)((a.C + MH_BLOCK - 1) / MH_BLOCK);
   time_begin(ctx);

@@ -321,15 +321,53 @@ static inline unsigned grid1d(mg_ctx *ctx, int64_t n, int block = KB) {
   if (g > cap) g = cap;
   return (unsigned)(g < 1 ? 1 : g);
 }
-static inline int64_t align256(int64_t x) { return (x + 255) & ~255LL; }
 
-int build_tree_v2(mg_ctx *ctx, const double *d_pts, int64_t N, int D, const double *low, const double *high, int min_split,
-                  mg_kdtree **out);   // kdtree_build2.cu
+KdHeader kd_layout(int64_t N, int D, int64_t node_cap, bool with_pts) {
+  KdHeader h{};
+  h.magic = KD_MAGIC; h.N = N; h.nnodes = node_cap; h.D = D;
+  int64_t off = align256(sizeof(KdHeader));
+  h.off_low = off; off = align256(off + 8 * D);
+  h.off_high = off; off = align256(off + 8 * D);
+  h.off_nodes = off; off = align256(off + 16 * node_cap);
+  h.off_count = off; off = align256(off + 4 * node_cap);
+  h.off_begin = off; off = align256(off + 4 * node_cap);
+  h.off_perm = off; off = align256(off + 4 * N);
+  h.off_pts = off; off = align256(off + (with_pts ? 8 * N * D : 0));
+  h.nbytes = off;
+  return h;
+}
+
+int kd_alloc(mg_ctx *ctx, const KdHeader &h, KdTreePtr *out) {
+  // from the stream-ordered pool (kept cached between builds: a synchronous cudaMalloc / cudaFree of a 2 GB blob
+  // costs 0.1-0.4 s now and then and synchronises the device)
+  void *blob = nullptr;
+  const cudaError_t e = cudaMallocAsync(&blob, (size_t)h.nbytes, ctx->stream);
+  if (e != cudaSuccess) return set_err(ctx, MG_ENOMEM, "cuda: %s (kd-tree blob of %lld bytes)", cudaGetErrorString(e), (long long)h.nbytes);
+  out->reset(new mg_kdtree);
+  (*out)->ctx = ctx; (*out)->d_blob = blob; (*out)->h = h;
+  return MG_OK;
+}
+
+int kd_finish(mg_ctx *ctx, KdTreePtr t, const double *low, const double *high, const double *d_pts, KdTreePtr *out) {
+  cudaStream_t s = ctx->stream;
+  const KdHeader &h = t->h;
+  char *blob = (char *)t->d_blob;
+  MG_CUDA(ctx, cudaMemcpyAsync(blob, &h, sizeof(KdHeader), cudaMemcpyHostToDevice, s));
+  MG_CUDA(ctx, cudaMemcpyAsync(blob + h.off_low, low, 8 * h.D, cudaMemcpyHostToDevice, s));
+  MG_CUDA(ctx, cudaMemcpyAsync(blob + h.off_high, high, 8 * h.D, cudaMemcpyHostToDevice, s));
+  if (h.off_pts < h.nbytes) MG_CUDA(ctx, cudaMemcpyAsync(blob + h.off_pts, d_pts, 8 * h.N * h.D, cudaMemcpyDeviceToDevice, s));
+  const cudaError_t e = cudaStreamSynchronize(s);
+  if (e != cudaSuccess) return set_err(ctx, MG_ECUDA, "cuda: %s (kd-tree build)", cudaGetErrorString(e));
+  if (int rc = poll_device_error(ctx)) return rc;
+  *out = std::move(t);
+  return MG_OK;
+}
+
 static int build_tree_v1(mg_ctx *ctx, const double *d_pts, int64_t N, int D, const double *low, const double *high,
-                         int min_split, mg_kdtree **out);
+                         int min_split, bool with_pts, KdTreePtr *out);
 
 int build_tree(mg_ctx *ctx, const double *d_pts, int64_t N, int D, const double *low, const double *high,
-                      int min_split, mg_kdtree **out) {
+               int min_split, bool with_pts, KdTreePtr *out) {
   cudaStream_t s = ctx->stream;
   MG_REQUIRE(ctx, N >= 1, "tree_of_objects: no objects");
   MG_REQUIRE(ctx, D >= 1 && D <= 64, "kd-tree: dim must be in 1..64");
@@ -337,7 +375,7 @@ int build_tree(mg_ctx *ctx, const double *d_pts, int64_t N, int D, const double 
   if (min_split < 2) min_split = 2;
   // The second builder (key columns moved level by level, subtrees finished in shared memory) hands inputs it is not
   // made for back to the first one (presorted index lists)
-  const int rc = build_tree_v2(ctx, d_pts, N, D, low, high, min_split, out);
+  const int rc = build_tree_v2(ctx, d_pts, N, D, low, high, min_split, with_pts, out);
   if (rc != MG_V2_FALLBACK) return rc;
   if (getenv("MCMC_GPU_DEBUG")) fprintf(stderr, "kd-tree: second builder handed the input back (ties / depth), first builder runs\n");
   // NaN coordinates are rejected (Pervasives.compare orders them, IEEE does not)
@@ -350,11 +388,11 @@ int build_tree(mg_ctx *ctx, const double *d_pts, int64_t N, int D, const double 
   MG_CUDA(ctx, cudaMemcpyAsync(&h_flag, d_flag.get(), sizeof(int), cudaMemcpyDeviceToHost, s));
   MG_CUDA(ctx, cudaStreamSynchronize(s));
   MG_REQUIRE(ctx, h_flag == 0, "kd-tree: NaN coordinate");
-  return build_tree_v1(ctx, d_pts, N, D, low, high, min_split, out);
+  return build_tree_v1(ctx, d_pts, N, D, low, high, min_split, with_pts, out);
 }
 
 static int build_tree_v1(mg_ctx *ctx, const double *d_pts, int64_t N, int D, const double *low, const double *high,
-                         int min_split, mg_kdtree **out) {
+                         int min_split, bool with_pts, KdTreePtr *out) {
   cudaStream_t s = ctx->stream;
   time_begin(ctx);
   kt_reset(ctx, N % 4 == 0 ? (const void *)part_fused_kernel<true> : (const void *)part_fused_kernel<false>);
@@ -487,40 +525,18 @@ static int build_tree_v1(mg_ctx *ctx, const double *d_pts, int64_t N, int D, con
     lb = le; le = nnodes + 2 * nsplit; nnodes = le;
   }
   level_begin.push_back((int32_t)nnodes);
-  // ---- assemble the blob ----------------------------------------------------
-  KdHeader h{};
-  h.magic = KD_MAGIC; h.N = N; h.nnodes = nnodes; h.D = D; h.nlevels = nlevels; h.min_split = min_split;
-  int64_t off = align256(sizeof(KdHeader));
-  h.off_low = off; off = align256(off + 8 * D);
-  h.off_high = off; off = align256(off + 8 * D);
-  h.off_nodes = off; off = align256(off + 16 * nnodes);
-  h.off_count = off; off = align256(off + 4 * nnodes);
-  h.off_begin = off; off = align256(off + 4 * nnodes);
-  h.off_perm = off; off = align256(off + 4 * N);
-  const bool with_pts = !ctx->kd_no_pts;
-  h.off_pts = off; off = align256(off + (with_pts ? 8 * N * D : 0));
-  h.nbytes = off;
-  mg_kdtree *t = new mg_kdtree;
-  t->ctx = ctx; t->h = h; t->level_begin = std::move(level_begin);
-  // from the stream-ordered pool (kept cached between builds: a synchronous cudaMalloc / cudaFree of a 2 GB blob
-  // costs 0.1-0.4 s now and then and synchronises the device)
-  cudaError_t e = cudaMallocAsync(&t->d_blob, (size_t)h.nbytes, s);
-  if (e != cudaSuccess) { delete t; return set_err(ctx, MG_ENOMEM, "cuda: %s (kd-tree blob of %lld bytes)", cudaGetErrorString(e), (long long)h.nbytes); }
+  // ---- the blob: nodes, counts, begins and the order of the points are this builder's ------------------------------
+  KdTreePtr t;
+  if (int rc = kd_alloc(ctx, kd_layout(N, D, nnodes, with_pts), &t)) return rc;
+  t->h.nlevels = nlevels; t->h.min_split = min_split; t->level_begin = std::move(level_begin);
+  const KdHeader &h = t->h;
   char *blob = (char *)t->d_blob;
-  cudaMemcpyAsync(blob, &t->h, sizeof(KdHeader), cudaMemcpyHostToDevice, s);
-  cudaMemcpyAsync(blob + h.off_low, low, 8 * D, cudaMemcpyHostToDevice, s);
-  cudaMemcpyAsync(blob + h.off_high, high, 8 * D, cudaMemcpyHostToDevice, s);
   pack_nodes_kernel<<<grid1d(ctx, nnodes), KB, 0, s>>>(a, nnodes, (KdNode *)(blob + h.off_nodes),
                                                       (int32_t *)(blob + h.off_count), (int32_t *)(blob + h.off_begin));
-  ctx->launches++;
-  cudaMemcpyAsync(blob + h.off_perm, lin + (int64_t)D * N, 4 * N, cudaMemcpyDeviceToDevice, s);
-  if (with_pts) cudaMemcpyAsync(blob + h.off_pts, d_pts, 8 * N * D, cudaMemcpyDeviceToDevice, s);
+  MG_CHECK_LAUNCH(ctx);
+  MG_CUDA(ctx, cudaMemcpyAsync(blob + h.off_perm, lin + (int64_t)D * N, 4 * N, cudaMemcpyDeviceToDevice, s));
   time_end(ctx);
-  e = cudaStreamSynchronize(s);
-  if (e != cudaSuccess) { cudaFreeAsync(t->d_blob, s); delete t; return set_err(ctx, MG_ECUDA, "cuda: %s (kd-tree build)", cudaGetErrorString(e)); }
-  if (int rc = poll_device_error(ctx)) { cudaFreeAsync(t->d_blob, s); delete t; return rc; }
-  *out = t;
-  return MG_OK;
+  return kd_finish(ctx, std::move(t), low, high, d_pts, out);
 }
 
 // ---- Interpolate_pdf kernels ------------------------------------------------
@@ -580,8 +596,10 @@ extern "C" int mg_kdtree_build_dev(mg_ctx *ctx, const double *d_pts, int64_t N, 
   if (!ctx) return MG_EINVAL;
   MG_REQUIRE(ctx, d_pts && low && high && out, "kd-tree: null argument");
   MG_CUDA(ctx, cudaSetDevice(ctx->device));
-  *out = nullptr;
-  return build_tree(ctx, d_pts, N, D, low, high, min_split, out);
+  KdTreePtr t;
+  const int rc = build_tree(ctx, d_pts, N, D, low, high, min_split, true, &t);
+  *out = t.release();
+  return rc;
 }
 
 extern "C" int mg_kdtree_build(mg_ctx *ctx, const double *pts, int64_t N, int32_t D, const double *low,
@@ -593,8 +611,10 @@ extern "C" int mg_kdtree_build(mg_ctx *ctx, const double *pts, int64_t N, int32_
   MG_CUDA(ctx, cudaSetDevice(ctx->device));
   DevBuf<double> d_pts;
   MG_CUDA(ctx, upload(d_pts, pts, (size_t)N * D, ctx->stream));
-  *out = nullptr;
-  return build_tree(ctx, d_pts.get(), N, D, low, high, min_split, out);
+  KdTreePtr t;
+  const int rc = build_tree(ctx, d_pts.get(), N, D, low, high, min_split, true, &t);
+  *out = t.release();
+  return rc;
 }
 
 extern "C" void mg_kdtree_destroy(mg_kdtree *t) {
@@ -697,19 +717,14 @@ extern "C" int mg_kdtree_from_blob_dev(mg_ctx *ctx, const void *d_blob, int64_t 
   MG_CUDA(ctx, cudaMemcpyAsync(&h, d_blob, sizeof h, cudaMemcpyDeviceToHost, ctx->stream));
   MG_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
   MG_REQUIRE(ctx, h.magic == KD_MAGIC && h.nbytes == nbytes, "kd-tree: blob header mismatch");
+  KdTreePtr t;
   int rc = validate_blob_header(ctx, h);
+  if (rc == MG_OK) rc = kd_alloc(ctx, h, &t);
   if (rc) return rc;
-  mg_kdtree *t = new mg_kdtree;
-  t->ctx = ctx; t->h = h;
-  cudaError_t e = cudaMallocAsync(&t->d_blob, (size_t)nbytes, ctx->stream);
-  if (e != cudaSuccess) { delete t; return set_err(ctx, MG_ENOMEM, "cuda: %s", cudaGetErrorString(e)); }
-  e = cudaMemcpyAsync(t->d_blob, d_blob, (size_t)nbytes, cudaMemcpyDeviceToDevice, ctx->stream);
+  cudaError_t e = cudaMemcpyAsync(t->d_blob, d_blob, (size_t)nbytes, cudaMemcpyDeviceToDevice, ctx->stream);
   if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
-  if (e != cudaSuccess) {
-    cudaFreeAsync(t->d_blob, ctx->stream); delete t;
-    return set_err(ctx, MG_ECUDA, "cuda: %s (kd-tree from blob)", cudaGetErrorString(e));
-  }
-  *out = t;
+  if (e != cudaSuccess) return set_err(ctx, MG_ECUDA, "cuda: %s (kd-tree from blob)", cudaGetErrorString(e));
+  *out = t.release();
   return MG_OK;
 }
 

@@ -35,10 +35,6 @@ struct KdHeader {
   int64_t off_low, off_high, off_nodes, off_count, off_begin, off_perm, off_pts;
 };
 constexpr uint64_t KD_MAGIC = 0x6b64747265653031ull;  // "kdtree01"
-#ifndef __CUDACC_RTC__
-int validate_blob_header(struct ::mg_ctx *ctx, const KdHeader &h);   // kdtree.cu
-#endif
-constexpr int MG_V2_FALLBACK = -1000;   // build_tree_v2: this input is for the first builder (not an error)
 
 struct KdView {
   const KdNode *nodes;
@@ -163,6 +159,7 @@ __device__ __forceinline__ bool kd_draw(const KdView &t, const KdScratch &s, int
 }  // namespace mg
 
 #ifndef __CUDACC_RTC__
+#include <memory>
 #include <vector>
 // host-side handle
 struct mg_kdtree {
@@ -185,4 +182,38 @@ struct mg_kdtree {
     return v;
   }
 };
+
+namespace mg {
+
+// A tree this code still owns (being built, or not yet handed to the caller): destroyed with its blob unless released.
+struct KdTreeDelete { void operator()(mg_kdtree *t) const { mg_kdtree_destroy(t); } };
+using KdTreePtr = std::unique_ptr<mg_kdtree, KdTreeDelete>;
+
+inline int64_t align256(int64_t x) { return (x + 255) & ~255LL; }
+
+// ---- the blob (kdtree.cu) ----------------------------------------------------------------------------------------------
+// kd_layout is the one place that states the section order and alignment.  It leaves room for node_cap nodes and sets
+// h.nnodes = node_cap (a builder that fills fewer sets h.nnodes itself); without the points, off_pts == nbytes.
+KdHeader kd_layout(int64_t N, int D, int64_t node_cap, bool with_pts);
+// a handle that owns a fresh blob of h.nbytes bytes and holds h
+int kd_alloc(mg_ctx *ctx, const KdHeader &h, KdTreePtr *out);
+// Writes the header, the root box and, where the layout has room for them, the points into t's blob, then waits for
+// the stream: a failed copy, kernel or device-side wait is reported and t is freed; otherwise t moves to *out.
+int kd_finish(mg_ctx *ctx, KdTreePtr t, const double *low, const double *high, const double *d_pts, KdTreePtr *out);
+// checks a blob that arrives from another process before any kernel indexes with it
+int validate_blob_header(mg_ctx *ctx, const KdHeader &h);
+
+// Kd_tree.tree_of_objects.  with_pts: the blob carries a copy of the points (Interpolate_pdf draws from it; callers
+// that keep the rows themselves leave it out).
+int build_tree(mg_ctx *ctx, const double *d_pts, int64_t N, int D, const double *low, const double *high,
+               int min_split, bool with_pts, KdTreePtr *out);
+// the second builder (kdtree_build2.cu); MG_V2_FALLBACK: this input is for the first builder (not an error)
+constexpr int MG_V2_FALLBACK = -1000;
+int build_tree_v2(mg_ctx *ctx, const double *d_pts, int64_t N, int D, const double *low, const double *high,
+                  int min_split, bool with_pts, KdTreePtr *out);
+// the same tree of the N points every rank holds, built by all ranks of c together (comm.cu)
+int build_tree_distributed(mg_comm *c, const double *d_pts, int64_t N, int D, const double *low, const double *high,
+                           int min_split, bool with_pts, KdTreePtr *out);
+
+}  // namespace mg
 #endif  // !__CUDACC_RTC__

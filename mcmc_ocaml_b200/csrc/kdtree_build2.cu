@@ -990,8 +990,6 @@ v2_emit_bottom_kernel(V2Bottom a, const int32_t *__restrict__ pre, V2LevelBase l
   }
 }
 
-static inline int64_t v2_align256(int64_t x) { return (x + 255) & ~255LL; }
-
 template <int NMAX, int BT>
 static int v2_launch_bottom(mg_ctx *ctx, const V2Bottom &a, int nsub, int D) {
   const size_t smem = v2_bottom_smem<NMAX, BT>(D);
@@ -1003,7 +1001,7 @@ static int v2_launch_bottom(mg_ctx *ctx, const V2Bottom &a, int nsub, int D) {
 
 // Returns MG_OK, an error, or MG_V2_FALLBACK (the caller then runs the first builder).
 int build_tree_v2(mg_ctx *ctx, const double *d_pts, int64_t N, int D, const double *low, const double *high, int min_split,
-                  mg_kdtree **out) {
+                  bool with_pts, KdTreePtr *out) {
   cudaStream_t s = ctx->stream;
   // the largest subtree whose key columns fit the shared memory of one SM
   constexpr size_t smem_cap = 224 * 1024;
@@ -1159,48 +1157,27 @@ int build_tree_v2(mg_ctx *ctx, const double *d_pts, int64_t N, int D, const doub
     std::swap(pin, pout);                           // pin = final order
   }
   if (nnodes > 2 * N) return set_err(ctx, MG_EFAIL, "kd-tree: node capacity exceeded");
-  // ---- assemble the blob (same layout as the first builder) ----------------------------------------------------------
-  KdHeader h{};
-  h.magic = KD_MAGIC; h.N = N; h.nnodes = nnodes; h.D = D; h.nlevels = nlevels; h.min_split = min_split;
-  int64_t off = v2_align256(sizeof(KdHeader));
-  h.off_low = off; off = v2_align256(off + 8 * D);
-  h.off_high = off; off = v2_align256(off + 8 * D);
-  h.off_nodes = off; off = v2_align256(off + 16 * nnodes);
-  h.off_count = off; off = v2_align256(off + 4 * nnodes);
-  h.off_begin = off; off = v2_align256(off + 4 * nnodes);
-  h.off_perm = off; off = v2_align256(off + 4 * N);
-  const bool with_pts = !ctx->kd_no_pts;
-  h.off_pts = off; off = v2_align256(off + (with_pts ? 8 * N * D : 0));
-  h.nbytes = off;
-  mg_kdtree *tr = new mg_kdtree;
-  tr->ctx = ctx; tr->h = h;
+  // ---- the blob: nodes, counts, begins and the order of the points are this builder's --------------------------------
+  KdTreePtr tr;
+  if ((rc = kd_alloc(ctx, kd_layout(N, D, nnodes, with_pts), &tr))) return rc;
+  tr->h.nlevels = nlevels; tr->h.min_split = min_split;
   // first node of every level: the top levels as the level loop numbered them, the subtree levels from the scan
   for (int L = 0; L <= Lh && L < nlevels; ++L) tr->level_begin.push_back(h_info.lvl[L].lb);
   for (int l = 1; Lh + l < nlevels; ++l) tr->level_begin.push_back(lbase.base[l]);
   tr->level_begin.push_back((int32_t)nnodes);
-  cudaError_t e = cudaMallocAsync(&tr->d_blob, (size_t)h.nbytes, s);
-  if (e != cudaSuccess) { delete tr; return set_err(ctx, MG_ENOMEM, "cuda: %s (kd-tree blob of %lld bytes)", cudaGetErrorString(e), (long long)h.nbytes); }
+  const KdHeader &h = tr->h;
   char *blob = (char *)tr->d_blob;
-  cudaMemcpyAsync(blob, &tr->h, sizeof(KdHeader), cudaMemcpyHostToDevice, s);
-  cudaMemcpyAsync(blob + h.off_low, low, 8 * D, cudaMemcpyHostToDevice, s);
-  cudaMemcpyAsync(blob + h.off_high, high, 8 * D, cudaMemcpyHostToDevice, s);
   KdNode *nodes = (KdNode *)(blob + h.off_nodes);
   int32_t *count = (int32_t *)(blob + h.off_count), *begin_out = (int32_t *)(blob + h.off_begin);
   v2_emit_top_kernel<<<(unsigned)std::min<int64_t>((nn_top + 255) / 256, 4096), 256, 0, s>>>(t, nn_top, nodes, count, begin_out);
-  ctx->launches++;
+  MG_CHECK_LAUNCH(ctx);
   if (nsub > 0) {
     v2_emit_bottom_kernel<<<(unsigned)nsub, 256, 0, s>>>(a, pre.get(), lbase, nodes, count, begin_out);
-    ctx->launches++;
+    MG_CHECK_LAUNCH(ctx);
   }
-  cudaMemcpyAsync(blob + h.off_perm, pin, 4 * N, cudaMemcpyDeviceToDevice, s);
-  if (with_pts) cudaMemcpyAsync(blob + h.off_pts, d_pts, 8 * N * D, cudaMemcpyDeviceToDevice, s);
+  MG_CUDA(ctx, cudaMemcpyAsync(blob + h.off_perm, pin, 4 * N, cudaMemcpyDeviceToDevice, s));
   time_end(ctx);
-  e = cudaGetLastError();
-  if (e == cudaSuccess) e = cudaStreamSynchronize(s);
-  if (e != cudaSuccess) { cudaFreeAsync(tr->d_blob, s); delete tr; return set_err(ctx, MG_ECUDA, "cuda: %s (kd-tree build)", cudaGetErrorString(e)); }
-  if (int rc2 = poll_device_error(ctx)) { cudaFreeAsync(tr->d_blob, s); delete tr; return rc2; }
-  *out = tr;
-  return MG_OK;
+  return kd_finish(ctx, std::move(tr), low, high, d_pts, out);
 }
 
 }  // namespace mg

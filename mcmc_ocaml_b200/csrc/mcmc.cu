@@ -22,12 +22,9 @@ namespace mg {
 // instantiations live in mcmc_static.cu / mcmc_dyn.cu (one object per dimension)
 #define MG_STATIC_DIMS(X) X(2) X(4) X(8) X(10) X(16) X(20) X(32)
 #define MG_DYN_DIMS(X) X(2) X(4) X(8) X(16) X(32) X(64)
-#define MG_DECL_STATIC(DD)                                                                         \
-  int mh_static_gauss_##DD(mg_ctx *, const mg_logfn *, const mg_proposal *, const mg_mcmc_cfg *, \
-                           CallKey, uint64_t, int, double *, double *, int32_t *);
-#define MG_DECL_DYN(DD)                                                                          \
-  int mh_dyn_##DD(mg_ctx *, const DynFnParams &, const DynFnParams &, const DynPropParams &,     \
-                  const mg_mcmc_cfg *, CallKey, uint64_t, int, double *, double *, int32_t *);
+#define MG_DECL_STATIC(DD) int mh_static_gauss_##DD(mg_ctx *, const mg_logfn *, const mg_proposal *, const MhLaunch &, bool *);
+#define MG_DECL_DYN(DD)                                                                                          \
+  int mh_dyn_##DD(mg_ctx *, const DynFnParams &, const DynFnParams &, const DynPropParams &, const MhLaunch &, bool *);
 MG_STATIC_DIMS(MG_DECL_STATIC)
 MG_DYN_DIMS(MG_DECL_DYN)
 
@@ -58,7 +55,7 @@ __global__ void to_chain_major_kernel(const double *__restrict__ src, int64_t ro
 }
 
 int jit_launch_mh(mg_ctx *ctx, const DynFnParams &like, const DynFnParams &prior, const DynPropParams &prop,
-                  const mg_mcmc_cfg *cfg, CallKey key, uint64_t t0, int record_first, double *d_state, double *d_samples, int32_t *d_accept);  // jit.cu
+                  const MhLaunch &L);  // jit.cu
 int sample_block_stats(mg_ctx *ctx, const double *d_blk, int64_t n, int F, int64_t C, double *d_out);  // stats.cu
 int chain_moments_finish(mg_ctx *ctx, cudaStream_t st, const double *mom, int F, int64_t C, int64_t n, double *d_out);
 
@@ -82,23 +79,24 @@ static int validate_cfg(mg_ctx *ctx, const mg_mcmc_cfg *cfg) {
 
 using namespace mg;
 
-// One launch of the ensemble kernel: steps t0 .. of the run keyed by `key`.
+// One launch of the ensemble kernel.  *mom_done (mom_done may be null where L.mom is): it kept the running moments.
 static int mcmc_launch_segment(mg_ctx *ctx, const mg_logfn *like, const mg_logfn *prior, const mg_proposal *prop,
-                               const mg_mcmc_cfg *cfg, CallKey key, uint64_t t0, int record_first, double *d_state,
-                               double *d_samples, int32_t *d_accept) {
+                               const MhLaunch &L, bool *mom_done) {
+  const mg_mcmc_cfg *cfg = L.cfg;
   int rc;
+  if (mom_done) *mom_done = false;
   if ((rc = validate_cfg(ctx, cfg))) return rc;
   if ((rc = validate_logfn(ctx, like, cfg->dim, "log_likelihood"))) return rc;
   if ((rc = validate_logfn(ctx, prior, cfg->dim, "log_prior"))) return rc;
   if ((rc = validate_proposal(ctx, prop, cfg->dim))) return rc;
-  MG_REQUIRE(ctx, d_state != nullptr, "mcmc_array: null state");
+  MG_REQUIRE(ctx, L.state != nullptr, "mcmc_array: null state");
   MG_CUDA(ctx, cudaSetDevice(ctx->device));
   const int D = cfg->dim;
 
   if (like->kind == MG_FN_GAUSS_CORR && like->scale == 1.0 && prior->kind == MG_FN_ZERO &&
       prop->kind == MG_PROP_BOX) {
     switch (D) {
-#define MG_CASE(DD) case DD: return mh_static_gauss_##DD(ctx, like, prop, cfg, key, t0, record_first, d_state, d_samples, d_accept);
+#define MG_CASE(DD) case DD: return mh_static_gauss_##DD(ctx, like, prop, L, mom_done);
       MG_STATIC_DIMS(MG_CASE)
 #undef MG_CASE
       default: break;
@@ -109,8 +107,8 @@ static int mcmc_launch_segment(mg_ctx *ctx, const mg_logfn *like, const mg_logfn
   MG_CUDA(ctx, dp.upload_from(prior, ctx->stream));
   MG_CUDA(ctx, dj.upload_from(prop, ctx->stream));
   if (like->kind >= MG_FN_USER || prior->kind >= MG_FN_USER)  // user plugins: kernel compiled at run time
-    return jit_launch_mh(ctx, dl.params, dp.params, dj.params, cfg, key, t0, record_first, d_state, d_samples, d_accept);
-#define MG_TRY(DD) if (D <= DD) rc = mh_dyn_##DD(ctx, dl.params, dp.params, dj.params, cfg, key, t0, record_first, d_state, d_samples, d_accept); else
+    return jit_launch_mh(ctx, dl.params, dp.params, dj.params, L);
+#define MG_TRY(DD) if (D <= DD) rc = mh_dyn_##DD(ctx, dl.params, dp.params, dj.params, L, mom_done); else
   MG_DYN_DIMS(MG_TRY) rc = set_err(ctx, MG_EINVAL, "mcmc_array: dim too large");
 #undef MG_TRY
   return rc;  // parameter blobs are freed stream-ordered after the kernel
@@ -122,7 +120,8 @@ extern "C" int mg_mcmc_array_dev(mg_ctx *ctx, const mg_logfn *like, const mg_log
   if (!ctx) return MG_EINVAL;
   int rc;
   if ((rc = validate_cfg(ctx, cfg))) return rc;
-  return mcmc_launch_segment(ctx, like, prior, prop, cfg, next_key(ctx), 0, 1, d_state, d_samples, d_accept);
+  return mcmc_launch_segment(ctx, like, prior, prop, MhLaunch{cfg, next_key(ctx), 0, 1, d_state, d_samples, d_accept, nullptr},
+                             nullptr);
 }
 
 extern "C" int mg_mcmc_array(mg_ctx *ctx, const mg_logfn *like, const mg_logfn *prior, const mg_proposal *prop,
@@ -178,7 +177,8 @@ extern "C" int mg_mcmc_array(mg_ctx *ctx, const mg_logfn *like, const mg_logfn *
       const uint64_t t0 = (k == 0) ? 0 : (uint64_t)(cfg->nbin + done * cfg->nskip);
       first[k] = (k == 0) ? 0 : 1 + done; count[k] = (k == 0) ? m + 1 : m;
       double *dst = d_samples.get() + (size_t)first[k] * F * C;
-      int r = mcmc_launch_segment(ctx, like, prior, prop, &seg, key, t0, k == 0 ? 1 : 0, d_state.get(), dst, d_acc.get());
+      int r = mcmc_launch_segment(ctx, like, prior, prop, MhLaunch{&seg, key, t0, k == 0 ? 1 : 0, d_state.get(), dst, d_acc.get(), nullptr},
+                                  nullptr);
       if (r) return r;
       MG_CUDA(ctx, cudaEventCreateWithFlags(&evs[k], cudaEventDisableTiming));
       MG_CUDA(ctx, cudaEventRecord(evs[k], s));
@@ -246,10 +246,10 @@ extern "C" int mg_mcmc_array_resident(mg_ctx *ctx, const mg_logfn *like, const m
   MG_CUDA(ctx, cudaMemsetAsync(d_acc.get(), 0, sizeof(int32_t) * C, s));
   init_state_kernel<<<(unsigned)((C + 255) / 256), 256, 0, s>>>(d_x0.get(), cfg->x0_shared, D, C, d_state.get());
   MG_CHECK_LAUNCH(ctx);
-  // Statistics: the balanced sampler can keep per-chain running moments of the samples it records
-  // (ctx->mh_mom); any other path leaves mh_mom_done false and the block is read back once.  Overlapping that
-  // read with the sampler on a second stream gave no gain on B200 (profiles/r01_mh_ncu_summary.md): the sampler's
-  // 4 warps x 122 registers fill every scheduler's 16K-register slice, so the Stats CTAs find no room until it ends.
+  // Statistics: the balanced sampler can keep per-chain running moments of the samples it records (d_mom); where the
+  // launch reports that it did not, the block is read back once.  Overlapping that read with the sampler on a second
+  // stream gave no gain on B200 (profiles/r01_mh_ncu_summary.md): the sampler's 4 warps x 122 registers fill every
+  // scheduler's 16K-register slice, so the Stats CTAs find no room until it ends.
   const bool want_stats = (out_mean || out_std) && n > 0;
   std::vector<double> stats(2 * F);
   DevBuf<double> d_mom;
@@ -257,14 +257,13 @@ extern "C" int mg_mcmc_array_resident(mg_ctx *ctx, const mg_logfn *like, const m
     MG_CUDA(ctx, d_stats.alloc(2 * F, s));
     MG_CUDA(ctx, d_mom.alloc((size_t)3 * F * C, s));
     MG_CUDA(ctx, cudaMemsetAsync(d_mom.get(), 0, sizeof(double) * 3 * F * C, s));
-    ctx->mh_mom = d_mom.get();
   }
-  ctx->mh_mom_done = false;
-  rc = mcmc_launch_segment(ctx, like, prior, prop, cfg, next_key(ctx), 0, 1, d_state.get(), d_samples, d_acc.get());
-  ctx->mh_mom = nullptr;
+  bool mom_done = false;
+  rc = mcmc_launch_segment(ctx, like, prior, prop,
+                           MhLaunch{cfg, next_key(ctx), 0, 1, d_state.get(), d_samples, d_acc.get(), d_mom.get()}, &mom_done);
   if (rc) return rc;
   if (want_stats) {
-    if (ctx->mh_mom_done) rc = chain_moments_finish(ctx, s, d_mom.get(), F, C, n, d_stats.get());
+    if (mom_done) rc = chain_moments_finish(ctx, s, d_mom.get(), F, C, n, d_stats.get());
     else rc = sample_block_stats(ctx, d_samples, n, F, C, d_stats.get());
     if (rc) return rc;
     MG_CUDA(ctx, cudaMemcpyAsync(stats.data(), d_stats.get(), sizeof(double) * 2 * F, cudaMemcpyDeviceToHost, s));

@@ -10,12 +10,11 @@
 #define MG_CAT(a, b) MG_CAT2(a, b)
 
 namespace mg {
-int MG_CAT(mh_dyn_, MG_DMAX)(mg_ctx *ctx, const DynFnParams &like, const DynFnParams &prior,
-                             const DynPropParams &prop, const mg_mcmc_cfg *cfg, CallKey key, uint64_t t0, int record_first, double *d_state,
-                             double *d_samples, int32_t *d_accept) {
+int MG_CAT(mh_dyn_, MG_DMAX)(mg_ctx *ctx, const DynFnParams &like, const DynFnParams &prior, const DynPropParams &prop,
+                             const MhLaunch &L, bool *mom_done) {
   MhArgs<DynFn, DynFn, DynProp, MG_DMAX> a;
   a.like = like; a.prior = prior; a.prop = prop;
-  fill_common(a, cfg, key, t0, record_first, d_state, d_samples, d_accept);
-  return launch_mh(ctx, a);
+  fill_common(a, L);
+  return launch_mh(ctx, a, L.mom, mom_done);
 }
 }  // namespace mg

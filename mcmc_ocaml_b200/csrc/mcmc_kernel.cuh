@@ -46,8 +46,21 @@ static inline bool make_sample_tensor_map(CUtensorMap *tm, double *samples, int6
              CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_NONE, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 
+// One launch of the ensemble kernel: steps t0 .. of the run keyed by `key`.
+struct MhLaunch {
+  const mg_mcmc_cfg *cfg;
+  CallKey key;
+  uint64_t t0;
+  int record_first;
+  double *state, *samples;
+  int32_t *accept;
+  double *mom;   // [3][D+2][C], zeroed: per-chain running moments of the recorded samples are wanted; or null
+};
+
+// mom (may be null): where to keep the running moments of the recorded samples.  Only the balanced kernel keeps
+// them, over a run that records from slot 0; *mom_done (non-null where mom is) tells whether this launch did.
 template <class Like, class Prior, class Prop, int D>
-static int launch_mh(mg_ctx *ctx, const MhArgs<Like, Prior, Prop, D> &a) {
+static int launch_mh(mg_ctx *ctx, const MhArgs<Like, Prior, Prop, D> &a, double *mom, bool *mom_done) {
   const int64_t ngroups = (a.C + MH_BLOCK - 1) / MH_BLOCK;
   const int64_t total_steps = a.nbin + (a.n > 0 ? (a.n - 1) * a.nskip : 0);
   // Dynamic hand-out pays when the warps do not divide evenly over the schedulers.  The persistent grid holds the
@@ -55,9 +68,9 @@ static int launch_mh(mg_ctx *ctx, const MhArgs<Like, Prior, Prop, D> &a) {
   // work until the tail: a polling warp on a saturated scheduler is starved by the arbiter and picks its group up late).
   const int64_t nsched = (int64_t)ctx->sm_count * 4;
   if (total_steps >= 4 * kSegSteps && ngroups > nsched && ngroups < (1ll << 30)) {
-    // running moments requested (mg_mcmc_array_resident): that instantiation holds more registers per warp, so its
-    // own occupancy sizes the persistent grid
-    const bool with_mom = ctx->mh_mom != nullptr && a.t0 == 0 && a.record_first && a.samples != nullptr;
+    // running moments requested: that instantiation holds more registers per warp, so its own occupancy sizes the
+    // persistent grid
+    const bool with_mom = mom != nullptr && a.t0 == 0 && a.record_first && a.samples != nullptr;
     int occ = 0;
     if (with_mom) MG_CUDA(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, mh_balanced_kernel<Like, Prior, Prop, D, true, false>, MH_BLOCK, 0));
     else MG_CUDA(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, mh_balanced_kernel<Like, Prior, Prop, D, false, false>, MH_BLOCK, 0));
@@ -92,8 +105,8 @@ static int launch_mh(mg_ctx *ctx, const MhArgs<Like, Prior, Prop, D> &a) {
     if (const char *e = getenv("MCMC_GPU_WAIT_CYCLES")) q.wait_cycles = std::max(1ll, atoll(e));
     mh_queue_init_kernel<<<(q.cap + 255u) / 256u, 256, 0, ctx->stream>>>(q);
     MG_CHECK_LAUNCH(ctx);
-    // running moments of the recorded samples (requested through the context by mg_mcmc_array_resident): the
-    // variant with the accumulators is a separate instantiation, the plain kernel does not pay for them
+    // running moments of the recorded samples: the variant with the accumulators is a separate instantiation, the
+    // plain kernel does not pay for them
     // Recorded samples leave through the TMA (one bulk tensor store per kTmaSteps samples of a warp) when the block's
     // shape allows a tensor map (even C, compile-time dimension, a tile of at most 16 KB); plain stores otherwise.
     CUtensorMap tmap;
@@ -104,7 +117,7 @@ static int launch_mh(mg_ctx *ctx, const MhArgs<Like, Prior, Prop, D> &a) {
                          make_sample_tensor_map(&tmap, a.samples, slots, F, a.C);
     time_begin(ctx);
     MhArgs<Like, Prior, Prop, D> am = a;
-    if (with_mom) { am.mom = ctx->mh_mom; ctx->mh_mom_done = true; }
+    if (with_mom) { am.mom = mom; *mom_done = true; }
     const void *fn;
 #define MG_MHB_LAUNCH(MOM, TMA)                                                                         \
     do {                                                                                                \
@@ -139,14 +152,15 @@ static int launch_mh(mg_ctx *ctx, const MhArgs<Like, Prior, Prop, D> &a) {
   return MG_OK;
 }
 
+// everything but the plugin parameters; a.mom is set by launch_mh for the kernel that keeps the moments
 template <class A>
-static void fill_common(A &a, const mg_mcmc_cfg *cfg, CallKey key, uint64_t t0, int record_first, double *d_state, double *d_samples,
-                        int32_t *d_accept) {
+static void fill_common(A &a, const MhLaunch &L) {
+  const mg_mcmc_cfg *cfg = L.cfg;
   a.d = cfg->dim; a.pad = 0; a.C = cfg->nchains; a.chain_offset = cfg->chain_offset;
-  a.nbin = cfg->nbin; a.nskip = cfg->nskip; a.n = cfg->n; a.key = key;
-  a.t0 = t0; a.record_first = record_first; a.pad2 = 0;
-  a.rk = make_round_keys(key);
-  a.state = d_state; a.samples = d_samples; a.accept = d_accept; a.mom = nullptr;
+  a.nbin = cfg->nbin; a.nskip = cfg->nskip; a.n = cfg->n; a.key = L.key;
+  a.t0 = L.t0; a.record_first = L.record_first; a.pad2 = 0;
+  a.rk = make_round_keys(L.key);
+  a.state = L.state; a.samples = L.samples; a.accept = L.accept; a.mom = nullptr;
 }
 
 }  // namespace mg

@@ -13,14 +13,13 @@
 #define MG_CAT(a, b) MG_CAT2(a, b)
 
 namespace mg {
-int MG_CAT(mh_static_gauss_, MG_SD)(mg_ctx *ctx, const mg_logfn *like, const mg_proposal *prop,
-                                    const mg_mcmc_cfg *cfg, CallKey key, uint64_t t0, int record_first, double *d_state, double *d_samples,
-                                    int32_t *d_accept) {
+int MG_CAT(mh_static_gauss_, MG_SD)(mg_ctx *ctx, const mg_logfn *like, const mg_proposal *prop, const MhLaunch &L,
+                                    bool *mom_done) {
   constexpr int D = MG_SD;
   MhArgs<GaussCorr<D>, ZeroFn, BoxProp<D>, D> a;
   GaussCorr<D>::pack(like->params, like->params + D, like->params[D + D * (D + 1) / 2], a.like);
   BoxProp<D>::pack(prop->params, a.prop);
-  fill_common(a, cfg, key, t0, record_first, d_state, d_samples, d_accept);
-  return launch_mh(ctx, a);
+  fill_common(a, L);
+  return launch_mh(ctx, a, L.mom, mom_done);
 }
 }  // namespace mg
