@@ -554,6 +554,45 @@ int mg_stats_chain_diagnostics(mg_ctx *ctx, const double *samples,
                                int32_t *out_window_closed, double *out_rho,
                                double *seq_tau);
 
+/* Exact per-field order statistics and quantiles of a sample block (Stats
+ * order statistics, stats.mli:19-110; DESIGN.md 4c).  Block x[s][f][c],
+ * s < n, f < F = D+2, c < C.  For each field f, the pool is the N = n*C values
+ * x[s][f][c] (all chains pooled, as mg_stats_sample_block_dev pools them).
+ * Order is the total order of f64_to_ordered: -inf is the smallest value and
+ * +inf the largest; -0.0 equals +0.0, and a zero is returned as +0.0.
+ * To drop a burn-in, pass d_samples + r*F*C and n - r (the block base need
+ * only be 8-byte aligned).
+ * Order statistic of rank k (0 <= k < N, 0-based: k = 0 is the minimum): the
+ *   k-th smallest value of the pool, exact (one of the block's values, bit for
+ *   bit, except for the sign of a zero).
+ * Quantile at p in [0, 1] (numpy's default "linear" rule, Hyndman-Fan 7, with
+ *   one rounding):
+ *   h = (double)(N-1) * p, lo = floor(h), g = h - lo, a = x_(lo),
+ *   b = x_(min(lo+1, N-1));
+ *   if g = 0 or a = b, q = a;
+ *   else if a = -inf: q = NaN when b = +inf, and -inf otherwise;
+ *   else if b = +inf, q = +inf;
+ *   otherwise q = a + g*(b - a), evaluated exactly as written (the library
+ *   builds with -fmad=false).
+ * NaN: if a field holds any NaN, every output for that field is NaN; other
+ *   fields are unaffected.
+ * MG_EINVAL: null pointers, n < 1, C < 1, D < 1, nq (or nk) outside
+ *   [1, MG_QUANT_MAX], a p outside [0, 1] or NaN, a k outside [0, N).
+ * The device block is read and never modified.  out: host [D+2][nq]
+ * ([D+2][nk] for order statistics). */
+#define MG_QUANT_MAX 64
+int mg_stats_quantiles_dev(mg_ctx *ctx, const double *d_samples, int64_t n,
+                           int32_t D, int64_t C, const double *probs,
+                           int32_t nq, double *out);
+/* the same on a host block [n][D+2][C] */
+int mg_stats_quantiles(mg_ctx *ctx, const double *samples, int64_t n,
+                       int32_t D, int64_t C, const double *probs, int32_t nq,
+                       double *out);
+int mg_stats_order_statistics_dev(mg_ctx *ctx, const double *d_samples,
+                                  int64_t n, int32_t D, int64_t C,
+                                  const int64_t *ranks, int32_t nk,
+                                  double *out);
+
 /* Stats.draw_uniform a b / draw_gaussian mu sigma / draw_cauchy x0 gamma
  * (stats.ml:126-128, 113-124 [Leva's ratio of uniforms], 89-91), n draws at
  * once.  Draw i comes from the call's Philox stream; the reference's global
@@ -702,6 +741,15 @@ int mg_comm_chain_diagnostics(mg_comm *comm, const double *d_samples_local,
                               double *out_ess, double *out_tau,
                               int32_t *out_window_closed, double *out_rho,
                               double *d_seq_tau);
+/* mg_stats_quantiles_dev of the union of every rank's block: each rank passes
+ * its own [n][D+2][C_r] block (same n, D, nq and probs on every rank, C_r of
+ * its own).  The result is the same on every rank and bit-identical to
+ * mg_stats_quantiles_dev on the concatenated block.  Arguments that differ
+ * between ranks, or a failure on one rank, are reported as an error on every
+ * rank. */
+int mg_comm_quantiles(mg_comm *comm, const double *d_samples_local, int64_t n,
+                      int32_t D, int64_t C_local, const double *probs,
+                      int32_t nq, double *out);
 
 /* ------------------------------------------------------------------ */
 /* Read_write: the text format of the reference's tools (host only)    */

@@ -72,6 +72,7 @@ class mg_diag_cfg(C.Structure):
 
 
 DIAG_MAXLAG = 256   # MG_DIAG_MAXLAG
+QUANT_MAX = 64      # MG_QUANT_MAX
 
 
 def as_f64(a, shape=None) -> np.ndarray:
@@ -140,6 +141,11 @@ def load_library() -> C.CDLL:
         lib.mg_ellipse_tree_destroy.argtypes = [C.c_void_p]
         lib.mg_ellipse_tree_info.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
         lib.mg_ellipse_tree_export.argtypes = [C.c_void_p] + [C.c_void_p] * 10
+    for name in ("mg_stats_quantiles_dev", "mg_stats_quantiles", "mg_stats_order_statistics_dev", "mg_comm_quantiles"):
+        fn = getattr(lib, name)
+        fn.restype = C.c_int
+        items = c_int64_p if name == "mg_stats_order_statistics_dev" else c_double_p
+        fn.argtypes = [C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_int64, items, C.c_int32, c_double_p]
     _lib = lib
     return lib
 

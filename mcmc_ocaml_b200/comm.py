@@ -180,3 +180,13 @@ class Comm:
         self.ctx.check(stats._diag_call(self.ctx.lib.mg_comm_chain_diagnostics, self.h, C.c_void_p(samples_ptr), cfg,
                                         outs, C.c_void_p(seq_tau_ptr) if seq_tau_ptr else None))
         return stats.ChainDiagnostics(*outs)
+
+    def quantiles(self, samples_ptr: int, n: int, D: int, nchains_local: int, probs) -> np.ndarray:
+        """``stats.quantiles_dev`` of the union of every rank's device block [n][D+2][C_r] (same n, D and probs on
+        every rank); the result [D+2][nq] is the same bytes on every rank."""
+        from . import stats
+        p = stats._probs(probs)
+        out = np.empty((D + 2, p.size))
+        self.ctx.check(self.ctx.lib.mg_comm_quantiles(self.h, samples_ptr, n, D, nchains_local, _abi.ptr(p), p.size,
+                                                      _abi.ptr(out)))
+        return out

@@ -621,3 +621,52 @@ extern "C" int mg_comm_chain_diagnostics(mg_comm *c, const double *d_samples_loc
   diag_finish(recs.data(), c->nranks, F, L, N, out_rhat, out_ess, out_tau, out_window_closed, out_rho);
   return MG_OK;
 }
+
+// Quantiles (quantiles.cu) of the union of every rank's block: one header exchange checks that n, D and the probs
+// agree and gives the pooled size; the order statistics then run on every rank with their exchanges (brackets, region
+// counts, select histograms) summed in rank order, so every rank gets the same bytes and one rank the single-GPU bits.
+namespace mg {
+int qt_check(mg_ctx *ctx, const void *x, int64_t n, int32_t D, int64_t C, const void *list, int32_t nq,
+             const double *out);
+int qt_prob_ranks(mg_ctx *ctx, const double *probs, int32_t nq, int64_t N, std::vector<int64_t> &ranks);
+int qt_order_keys(mg_ctx *ctx, mg_comm *comm, const double *d_x, int64_t n, int32_t D, int64_t C, int64_t N,
+                  const std::vector<int64_t> &ranks, std::vector<uint64_t> &keys, std::vector<int> &nan_f);
+void qt_finish_quantiles(const double *probs, int32_t nq, int64_t N, int F, const std::vector<int64_t> &ranks,
+                         const std::vector<uint64_t> &keys, const std::vector<int> &nan_f, double *out);
+}  // namespace mg
+
+extern "C" int mg_comm_quantiles(mg_comm *c, const double *d_samples_local, int64_t n, int32_t D, int64_t C_local,
+                                 const double *probs, int32_t nq, double *out) {
+  if (!c) return MG_EINVAL;
+  mg_ctx *ctx = c->ctx;
+  std::vector<int64_t> ranks;
+  int rc = qt_check(ctx, d_samples_local, n, D, C_local, probs, nq, out);
+  if (rc == MG_OK) rc = qt_prob_ranks(ctx, probs, nq, n * C_local, ranks);
+  if (rc == MG_OK && cudaSetDevice(ctx->device) != cudaSuccess) rc = set_err(ctx, MG_ECUDA, "cuda: cannot select the device");
+  // header: status, n, D, C_r, nq, the bits of probs
+  const size_t H = 5 + MG_QUANT_MAX;
+  std::vector<uint64_t> mine(H, 0), all(H * c->nranks);
+  mine[0] = (uint64_t)rc;
+  if (rc == MG_OK) {
+    mine[1] = (uint64_t)n; mine[2] = (uint64_t)D; mine[3] = (uint64_t)C_local; mine[4] = (uint64_t)nq;
+    memcpy(&mine[5], probs, sizeof(double) * nq);
+  }
+  const int rc2 = mg_comm_allgather(c, mine.data(), all.data(), (int64_t)(sizeof(uint64_t) * H));
+  if (rc) return rc;
+  if (rc2) return rc2;
+  int64_t Ctot = 0;
+  for (int r = 0; r < c->nranks; ++r) {
+    const uint64_t *q = all.data() + H * r;
+    if (q[0] != 0) return set_err(ctx, (int)q[0], "quantiles (comm): rank %d failed", r);
+    if (!std::equal(q + 1, q + 3, mine.begin() + 1) || !std::equal(q + 4, q + H, mine.begin() + 4))
+      return set_err(ctx, MG_EINVAL, "quantiles (comm): rank %d has another n, D or probs", r);
+    Ctot += (int64_t)q[3];
+  }
+  const int64_t N = n * Ctot;
+  if ((rc = qt_prob_ranks(ctx, probs, nq, N, ranks))) return rc;
+  std::vector<uint64_t> keys;
+  std::vector<int> nan_f;
+  if ((rc = qt_order_keys(ctx, c, d_samples_local, n, D, C_local, N, ranks, keys, nan_f))) return rc;
+  qt_finish_quantiles(probs, nq, N, D + 2, ranks, keys, nan_f, out);
+  return MG_OK;
+}

@@ -140,6 +140,58 @@ def chain_diagnostics_dev(samples_ptr: int, n: int, D: int, nchains: int, maxlag
     return ChainDiagnostics(*outs)
 
 
+# --- order statistics and quantiles of a sample block (DESIGN.md 4c) ------------------------------------------------
+
+QUANT_MAX = _abi.QUANT_MAX
+
+
+def _probs(probs) -> np.ndarray:
+    p = _abi.as_f64(probs).ravel()
+    if not 1 <= p.size <= QUANT_MAX:
+        raise _abi.InvalidArgument(f"quantiles: need 1 to {QUANT_MAX} probabilities")
+    return p
+
+
+def quantiles(samples, probs, *, ctx: Context | None = None) -> np.ndarray:
+    """Exact per-field quantiles [D+2][nq] of a host sample block: an ``McmcSamples`` (a chain-major block is
+    transposed here) or an array [n][D+2][C]; all chains pooled, numpy's "linear" rule (include/mcmc_gpu.h)."""
+    ctx = ctx or default_context()
+    if hasattr(samples, "layout"):
+        blk = samples.block if samples.layout == "step" else np.transpose(samples.block, (1, 2, 0))
+    else:
+        blk = samples
+    blk = _abi.as_f64(blk)
+    if blk.ndim != 3 or blk.shape[1] < 3:
+        raise _abi.InvalidArgument("quantiles: the block must be [n][D+2][C] with D >= 1")
+    n, F, nc = blk.shape
+    p = _probs(probs)
+    out = np.empty((F, p.size))
+    ctx.check(ctx.lib.mg_stats_quantiles(ctx.h, _abi.ptr(blk), n, F - 2, nc, _abi.ptr(p), p.size, _abi.ptr(out)))
+    return out
+
+
+def quantiles_dev(samples_ptr: int, n: int, D: int, nchains: int, probs, *, ctx: Context | None = None) -> np.ndarray:
+    """The same over a device sample block [n][D+2][C] (``mg_mcmc_array_dev`` / ``_resident``), which is not modified."""
+    ctx = ctx or default_context()
+    p = _probs(probs)
+    out = np.empty((D + 2, p.size))
+    ctx.check(ctx.lib.mg_stats_quantiles_dev(ctx.h, samples_ptr, n, D, nchains, _abi.ptr(p), p.size, _abi.ptr(out)))
+    return out
+
+
+def order_statistics_dev(samples_ptr: int, n: int, D: int, nchains: int, ranks, *,
+                         ctx: Context | None = None) -> np.ndarray:
+    """Exact order statistics [D+2][nk] (0-based ranks into the n C pooled values of each field) of a device block."""
+    ctx = ctx or default_context()
+    r = np.ascontiguousarray(ranks, dtype=np.int64).ravel()
+    if not 1 <= r.size <= QUANT_MAX:
+        raise _abi.InvalidArgument(f"order_statistics: need 1 to {QUANT_MAX} ranks")
+    out = np.empty((D + 2, r.size))
+    ctx.check(ctx.lib.mg_stats_order_statistics_dev(ctx.h, samples_ptr, n, D, nchains, _abi.ptr(r, _abi.c_int64_p),
+                                                    r.size, _abi.ptr(out)))
+    return out
+
+
 # --- draws and densities (stats.ml:89-128, 240-248) ------------------------------------------------------------
 
 DRAW_UNIFORM, DRAW_GAUSSIAN, DRAW_CAUCHY = 0, 1, 2

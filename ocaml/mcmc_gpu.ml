@@ -49,6 +49,12 @@ external chain_diagnostics_dev_raw :
   ctx -> int64 -> int -> int -> int -> int -> int -> (float, float64_elt, c_layout) Array2.t ->
   (float, float64_elt, c_layout) Array2.t -> int64 -> unit
   = "mcmcgpu_chain_diagnostics_dev_bytecode" "mcmcgpu_chain_diagnostics_dev_native"
+external quantiles_raw :
+  ctx -> (float, float64_elt, c_layout) Array3.t -> (float, float64_elt, c_layout) Array1.t ->
+  (float, float64_elt, c_layout) Array2.t -> unit = "mcmcgpu_quantiles"
+external quantiles_dev_raw :
+  ctx -> int64 -> int -> int -> int -> (float, float64_elt, c_layout) Array1.t -> (float, float64_elt, c_layout) Array2.t ->
+  unit = "mcmcgpu_quantiles_dev_bytecode" "mcmcgpu_quantiles_dev_native"
 (* the record the stub reads field by field (rj_of_value in mcmc_gpu_stubs.c) *)
 type rj_model_raw = {
   r_like : logfn; r_prior : logfn; r_prop : proposal; r_into : tree option;
@@ -210,6 +216,20 @@ let chain_diagnostics_dev ctx ?(split = true) ?(seq_tau = 0L) ~maxlag ~n ~dim ~n
   let out = Array2.create float64 c_layout 4 f and rho = Array2.create float64 c_layout f maxlag in
   chain_diagnostics_dev_raw ctx block n dim nchains maxlag (if split then 1 else 0) out rho seq_tau;
   diag_result f maxlag out rho None
+
+(* Exact per-field quantiles of a sample block [n][D+2][C], chains pooled (include/mcmc_gpu.h) *)
+let quantiles_result f probs out =
+  Array.init f (fun i -> Array.init (Array.length probs) (fun k -> out.{i, k}))
+let quantiles ctx ~probs (block : (float, float64_elt, c_layout) Array3.t) =
+  let f = Array3.dim2 block in
+  let out = Array2.create float64 c_layout f (Array.length probs) in
+  quantiles_raw ctx block (Array1.of_array float64 c_layout probs) out;
+  quantiles_result f probs out
+let quantiles_dev ctx ~probs ~n ~dim ~nchains (block : int64) =
+  let f = dim + 2 in
+  let out = Array2.create float64 c_layout f (Array.length probs) in
+  quantiles_dev_raw ctx block n dim nchains (Array1.of_array float64 c_layout probs) out;
+  quantiles_result f probs out
 
 (* Nested.nested_evidence ?epsrel ?nmcmc ?nlive ?mode_hopping_frac (nested.ml:122-146; nested.mli:50-61) with draw_prior
    uniform on [prior_low, prior_high]; ?batch live points are replaced per iteration (1 = the reference's schedule).

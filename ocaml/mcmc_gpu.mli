@@ -109,6 +109,13 @@ val chain_diagnostics_dev :
   ctx -> ?split:bool -> ?seq_tau:int64 -> maxlag:int -> n:int -> dim:int -> nchains:int -> int64 ->
   chain_diagnostics
 (** The same on a device block (its address); [?seq_tau] is the device address of a [D+2][M] float64 array. *)
+val quantiles :
+  ctx -> probs:float array -> (float, Bigarray.float64_elt, Bigarray.c_layout) Bigarray.Array3.t -> float array array
+(** Exact quantiles [D+2][nq] of a sample block [n][D+2][C], all chains pooled: numpy's "linear" rule on the exact
+    order statistics; a field holding a NaN gives NaN.  Definitions in mcmc_gpu.h.  [Invalid_argument] for no probs or
+    more than 64, or a p outside [0, 1]. *)
+val quantiles_dev : ctx -> probs:float array -> n:int -> dim:int -> nchains:int -> int64 -> float array array
+(** The same on a device block (its address), which is not modified. *)
 
 (** {2 Nested (nested.mli:50-69)} *)
 val nested_evidence :

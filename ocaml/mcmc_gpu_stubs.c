@@ -329,6 +329,47 @@ CAMLprim value mcmcgpu_chain_diagnostics_dev_bytecode(value *a, int argn) {
   return mcmcgpu_chain_diagnostics_dev_native(a[0], a[1], a[2], a[3], a[4], a[5], a[6], a[7], a[8], a[9]);
 }
 
+/* ---- exact quantiles of a sample block (mg_stats_quantiles*) ------------------------------------------------
+ * external quantiles : ctx -> (float, float64_elt, c_layout) Array3.t (* block [n][D+2][C] *) ->
+ *   Array1.t (* probs *) -> Array2.t (* out [D+2][nq] *) -> unit */
+CAMLprim value mcmcgpu_quantiles(value ctx, value blk, value probs, value out) {
+  CAMLparam4(ctx, blk, probs, out);
+  struct caml_ba_array *b = Caml_ba_array_val(blk);
+  mg_ctx *c = Ctx_val(ctx);
+  const double *x = (const double *)Caml_ba_data_val(blk), *p = (const double *)Caml_ba_data_val(probs);
+  double *o = (double *)Caml_ba_data_val(out);
+  const int64_t n = b->dim[0], C = b->dim[2];
+  const int32_t D = (int32_t)b->dim[1] - 2, nq = (int32_t)Caml_ba_array_val(probs)->dim[0];
+  caml_release_runtime_system();
+  int rc = mg_stats_quantiles(c, x, n, D, C, p, nq, o);
+  caml_acquire_runtime_system();
+  check(c, rc);
+  CAMLreturn(Val_unit);
+}
+/* the same on a device block (its device address as int64)
+ * external quantiles_dev : ctx -> int64 -> int (* n *) -> int (* dim *) -> int (* nchains *) -> Array1.t (* probs *) ->
+ *   Array2.t (* out *) -> unit */
+CAMLprim value mcmcgpu_quantiles_dev_native(value ctx, value ptr, value n, value dim, value nchains, value probs,
+                                            value out) {
+  CAMLparam5(ctx, ptr, n, dim, nchains);
+  CAMLxparam2(probs, out);
+  mg_ctx *c = Ctx_val(ctx);
+  const double *x = (const double *)(intptr_t)Int64_val(ptr), *p = (const double *)Caml_ba_data_val(probs);
+  double *o = (double *)Caml_ba_data_val(out);
+  const int32_t nq = (int32_t)Caml_ba_array_val(probs)->dim[0];
+  const int64_t nn = Long_val(n), C = Long_val(nchains);
+  const int32_t D = Int_val(dim);
+  caml_release_runtime_system();
+  int rc = mg_stats_quantiles_dev(c, x, nn, D, C, p, nq, o);
+  caml_acquire_runtime_system();
+  check(c, rc);
+  CAMLreturn(Val_unit);
+}
+CAMLprim value mcmcgpu_quantiles_dev_bytecode(value *a, int argn) {
+  (void)argn;
+  return mcmcgpu_quantiles_dev_native(a[0], a[1], a[2], a[3], a[4], a[5], a[6]);
+}
+
 /* ---- Stats.draw_uniform / draw_gaussian / draw_cauchy (stats.ml:89-91,113-128), n draws per call ----------
  * external stats_draw : ctx -> int -> float -> float -> (float, float64_elt, c_layout) Array1.t -> unit
  * kind: 0 uniform a b | 1 gaussian mu sigma | 2 cauchy x0 gamma (MG_DRAW_*) */

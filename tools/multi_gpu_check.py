@@ -15,6 +15,8 @@ NCCL id and allocates the test data):
      every rank, within 1e-12 of the one-GPU call on all chains.  It runs right after step 4, whose chains it uses.
   8. step 6 on data whose subtree on one rank the second kd-tree builder hands back to the first (a block of
      identical rows), so that the level table of that rank comes from the first builder.
+  9. exact quantiles of a seeded block whose chains are shared unevenly over the ranks (mg_comm_quantiles): the same
+     bytes on every rank, equal to the single-GPU call on the whole block.
 Prints one JSON line on rank 0."""
 from __future__ import annotations
 
@@ -157,6 +159,26 @@ def main():
         out["diagnostics_identical_on_all_ranks"] = bool(all(np.array_equal(allv[r_], allv[0], equal_nan=True)
                                                              for r_ in range(world)))
         out["diagnostics_within_1e12_of_single_gpu"] = bool(np.allclose(vec, ov, rtol=1e-12, atol=1e-12, equal_nan=True))
+    # ---- 9. quantiles of chains sharded unevenly (mg_comm_quantiles) ----------------------------------
+    # the same seeded block on every rank; rank r holds a share of the chains proportional to r + 1.  The result must be
+    # the same bytes on every rank and equal to the single-GPU call on the whole block
+    nq_, Dq, Cq = 300, 3, 1537
+    xq = np.random.default_rng(1234).standard_normal((nq_, Dq + 2, Cq))
+    xq[:, 1] *= 1e-3
+    xq[:, 1] += 1e8
+    xq[5, 2, 7] = np.nan
+    xq[:, 3, :Cq // 2] = 0.5
+    edges = [Cq * r_ * (r_ + 1) // (world * (world + 1)) for r_ in range(world + 1)]
+    qb, qe = edges[rank], edges[rank + 1]
+    probs = [0.0, 0.025, 0.16, 0.5, 0.84, 0.975, 1.0]
+    dq = torch.as_tensor(np.ascontiguousarray(xq[:, :, qb:qe]), device=dev); torch.cuda.synchronize()
+    qv = comm.quantiles(dq.data_ptr(), nq_, Dq, qe - qb, probs)
+    allq = np.asarray(comm.allgather(qv.ravel().view(np.int64))).reshape(world, -1)
+    del dq
+    if rank == 0:
+        one = stats.quantiles(xq, probs, ctx=ctx)
+        out["quantiles_identical_on_all_ranks"] = bool(all(np.array_equal(allq[r_], allq[0]) for r_ in range(world)))
+        out["quantiles_bit_identical_to_single_gpu"] = bool(np.array_equal(qv.view(np.int64), one.view(np.int64)))
     # ---- 5. sharded RJMCMC over the broadcast tree(s) ----------------------------
     d2 = Dm
     likeA = P.gauss_diag(np.full(d2, 0.5), np.full(d2, 0.08)); priorA = P.box(np.zeros(d2), np.ones(d2), 0.0)
@@ -224,6 +246,7 @@ def main():
                          and out["harmonic_sharded_rel_err"] < 1e-14 and out["evidence_identical_on_all_ranks"]
                          and out["evidence_bit_identical_to_single_gpu"] and out["rj_counts_equal"]
                          and out["diagnostics_identical_on_all_ranks"] and out["diagnostics_within_1e12_of_single_gpu"]
+                         and out["quantiles_identical_on_all_ranks"] and out["quantiles_bit_identical_to_single_gpu"]
                          and all(out[f"dist_build_ms{ms}"]["identical_to_single_gpu_on_every_rank"] for ms in (2, 64))
                          and out["dist_build_first_builder"]["identical_to_single_gpu_on_every_rank"])
         s_ = json.dumps(out)
