@@ -659,7 +659,14 @@ double mg_nested_log_total_error(double log_ev, double log_dev, int32_t nlive);
  * one rank and replicated, per-rank statistics and per-cell evidence terms are
  * gathered and combined in a fixed order.  NCCL is loaded at run time
  * (libnccl.so.2); without it only the entry points below fail (MG_EFAIL).
- * Every entry point here is COLLECTIVE: all ranks of the communicator call it. */
+ * Every entry point here is COLLECTIVE: all ranks of the communicator call it.
+ * The rank-pooled calls (the sharded evidence estimators, the distributed
+ * kd-tree build, mg_rjmcmc_array_sharded, mg_comm_pool_moments,
+ * mg_comm_chain_diagnostics and mg_comm_quantiles) exchange every rank's status
+ * before they use another rank's data: an argument error or a failure on any
+ * rank is returned on every rank, and the arguments that must be the same on
+ * every rank are checked ("rank r has another ..." is MG_EINVAL).  A null comm
+ * returns MG_EINVAL at once. */
 #define MG_COMM_ID_BYTES 128
 /* ncclGetUniqueId: called by one rank, which hands the 128 bytes to the others
  * through any channel of the host program (a file, a socket, MPI, ...). */
@@ -680,7 +687,8 @@ int mg_comm_allgather(mg_comm *comm, const void *send, void *recv, int64_t nbyte
 /* Interp.make on `root`, used everywhere: ONE ncclBroadcast of the tree's
  * contiguous device blob, from the builder's blob straight into the receivers'
  * (no staging copy).  tree: the root's tree (ignored elsewhere, may be NULL).
- * *out: on the root `tree` itself, on the other ranks a new tree (destroy it). */
+ * *out: on the root `tree` itself, on the other ranks a new tree (destroy it).
+ * An argument error on one rank is not propagated to the others. */
 int mg_kdtree_broadcast(mg_comm *comm, mg_kdtree *tree, int32_t root,
                         mg_kdtree **out);
 /* Kd_tree.tree_of_objects (kd_tree.ml:155-175) built by all ranks together
@@ -690,7 +698,8 @@ int mg_kdtree_broadcast(mg_comm *comm, mg_kdtree *tree, int32_t root,
  * subtrees; every rank receives the whole tree, bit-identical to
  * mg_kdtree_build_dev on one GPU.  A rank count that is not a power of two,
  * fewer than 4096 points per rank, min_split above N / nranks or ties that keep
- * the top from being a complete tree make every rank build the tree alone. */
+ * the top from being a complete tree make every rank build the tree alone.
+ * An argument error on one rank is not propagated to the others. */
 int mg_kdtree_build_distributed(mg_comm *comm, const double *d_pts, int64_t N,
                                 int32_t D, const double *low, const double *high,
                                 int32_t min_split, mg_kdtree **out);
@@ -723,19 +732,14 @@ int mg_rjmcmc_array_sharded(mg_comm *comm, const mg_rj_model *A,
                             int64_t out_counts[2], int64_t *shard_begin,
                             int64_t *shard_count);
 /* Stats.multi_mean / multi_std of samples held by several ranks, pooled from
- * each rank's (count, mean[F], std[F]) in rank order. */
+ * each rank's (count, mean[F], std[F]) in rank order (same F on every rank). */
 int mg_comm_pool_moments(mg_comm *comm, int64_t n_local, const double *mean_local,
                          const double *std_local, int32_t F, int64_t *n_total,
                          double *out_mean, double *out_std);
 /* mg_stats_chain_diagnostics_dev over chains sharded across the ranks: each
  * rank passes its own [n][D+2][C_r] block (same n, dim, maxlag and split on
  * every rank).  The pooled outputs are identical on every rank (one rank: the
- * bits of the single-GPU call); d_seq_tau covers the local sequences [D+2][M_r].
- * dim and maxlag size the exchanged record, so they MUST agree on every rank: a
- * rank whose dim or maxlag is out of range returns before the collective, and
- * ranks that disagree enter it with different sizes; in both cases the other
- * ranks wait for ever (as in mg_comm_pool_moments).  A differing n or split,
- * or a failure of the local pass, is reported as an error on every rank. */
+ * bits of the single-GPU call); d_seq_tau covers the local sequences [D+2][M_r]. */
 int mg_comm_chain_diagnostics(mg_comm *comm, const double *d_samples_local,
                               const mg_diag_cfg *cfg_local, double *out_rhat,
                               double *out_ess, double *out_tau,
@@ -744,9 +748,7 @@ int mg_comm_chain_diagnostics(mg_comm *comm, const double *d_samples_local,
 /* mg_stats_quantiles_dev of the union of every rank's block: each rank passes
  * its own [n][D+2][C_r] block (same n, D, nq and probs on every rank, C_r of
  * its own).  The result is the same on every rank and bit-identical to
- * mg_stats_quantiles_dev on the concatenated block.  Arguments that differ
- * between ranks, or a failure on one rank, are reported as an error on every
- * rank. */
+ * mg_stats_quantiles_dev on the concatenated block. */
 int mg_comm_quantiles(mg_comm *comm, const double *d_samples_local, int64_t n,
                       int32_t D, int64_t C_local, const double *probs,
                       int32_t nq, double *out);

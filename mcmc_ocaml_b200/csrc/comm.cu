@@ -15,7 +15,7 @@
 #include <algorithm>
 #include <vector>
 
-#include "common.cuh"
+#include "comm.cuh"
 #include "kdtree.cuh"
 
 static_assert(sizeof(ncclUniqueId) == MG_COMM_ID_BYTES, "ncclUniqueId is 128 bytes");
@@ -191,6 +191,31 @@ extern "C" int mg_comm_barrier(mg_comm *c) {
   return mg_comm_allgather(c, &one, all.data(), 1);
 }
 
+namespace mg {
+
+mg_ctx *mg_comm_ctx(const mg_comm *c) { return c ? c->ctx : nullptr; }
+
+int comm_gather(mg_comm *c, int rc, const void *rec, size_t nbytes, std::vector<uint8_t> &all, const char *what) {
+  const size_t W = sizeof(int64_t) + nbytes;
+  std::vector<uint8_t> mine(W, 0), got(W * c->nranks);
+  const int64_t status = rc;
+  memcpy(mine.data(), &status, sizeof status);
+  if (rc == MG_OK && nbytes) memcpy(mine.data() + sizeof status, rec, nbytes);
+  const int rc2 = mg_comm_allgather(c, mine.data(), got.data(), (int64_t)W);
+  if (rc) return rc;
+  if (rc2) return rc2;
+  all.resize(nbytes * c->nranks);
+  for (int r = 0; r < c->nranks; ++r) {
+    int64_t s;
+    memcpy(&s, got.data() + W * r, sizeof s);
+    if (s != MG_OK) return set_err(c->ctx, (int)s, "%s: rank %d failed", what, r);
+    if (nbytes) memcpy(all.data() + nbytes * r, got.data() + W * r + sizeof s, nbytes);
+  }
+  return MG_OK;
+}
+
+}  // namespace mg
+
 // Kd-tree built on `root`, replicated on every rank: the header first (sizes), then ONE broadcast of the blob from the
 // builder's blob straight into each receiver's freshly allocated blob.  On the root *out is `tree` itself.
 extern "C" int mg_kdtree_broadcast(mg_comm *c, mg_kdtree *tree, int32_t root, mg_kdtree **out) {
@@ -231,113 +256,6 @@ extern "C" int mg_kdtree_broadcast(mg_comm *c, mg_kdtree *tree, int32_t root, mg
   if (rc == MG_OK) { tm.stop(); rc = validate_blob_header(ctx, h); }
   if (rc) return rc;
   *out = t.release();
-  return MG_OK;
-}
-
-mg_ctx *mg_comm_ctx(const mg_comm *c) { return c ? c->ctx : nullptr; }
-
-#include "reduce_sum.cuh"
-
-// Evidence.evidence_harmonic_mean (evidence.ml:101-107) over samples SHARDED across ranks: every rank reduces the
-// 1/L of its own shard (compensated), the (count, sum) pairs are all-gathered and folded in rank order.  Agrees with
-// the single-GPU value to the rounding of the compensated sums (<= 2 ulp); identical on every rank.
-extern "C" int mg_evidence_harmonic_mean_sharded(mg_comm *c, const double *d_ll_shard, int64_t n_shard, double *out) {
-  if (!c) return MG_EINVAL;
-  mg_ctx *ctx = c->ctx;
-  MG_REQUIRE(ctx, out && n_shard >= 0 && (d_ll_shard || n_shard == 0), "evidence_harmonic_mean (sharded): bad arguments");
-  MG_CUDA(ctx, cudaSetDevice(ctx->device));
-  double mine[2] = {(double)n_shard, 0.0};
-  if (n_shard > 0) {
-    int rc = reduce_sum(ctx, n_shard, [d_ll_shard] __device__(int64_t i) { return 1.0 / exp(d_ll_shard[i]); }, &mine[1]);
-    if (rc) return rc;
-  }
-  std::vector<double> all((size_t)2 * c->nranks);
-  int rc = mg_comm_allgather(c, mine, all.data(), sizeof mine);
-  if (rc) return rc;
-  Comp linv; double n = 0.0;
-  for (int r = 0; r < c->nranks; ++r) { n += all[2 * r]; linv.add(all[2 * r + 1]); }
-  MG_REQUIRE(ctx, n >= 1.0, "evidence_harmonic_mean (sharded): no samples on any rank");
-  *out = n / linv.value();
-  return MG_OK;
-}
-
-// Mcmc.rjmcmc_array (mcmc.ml:121-139) with the ensemble's chains cut into contiguous ranges, one per rank: rank r runs
-// the global chain ids cfg->chain_offset + [b_r, e_r) (the Philox stream is addressed by the global id, so the
-// chains do not depend on the number of ranks), then rjmcmc_model_counts (mcmc.ml:141-149) and the accept / jump
-// counters of all ranks are all-gathered and summed.  out_model / out_samples receive this rank's shard only
-// ([n][C_r], [n][Dmax+2][C_r]); *shard_begin / *shard_count tell which chains those are.
-extern "C" int mg_rjmcmc_array_sharded(mg_comm *c, const mg_rj_model *A, const mg_rj_model *B, const mg_rjmcmc_cfg *cfg,
-                                       const double *a0, const double *b0, uint8_t *out_model, double *out_samples,
-                                       int64_t out_counts[2], int64_t *shard_begin, int64_t *shard_count) {
-  if (!c) return MG_EINVAL;
-  mg_ctx *ctx = c->ctx;
-  MG_REQUIRE(ctx, cfg && out_counts, "rjmcmc_array (sharded): null argument");
-  const int64_t C = cfg->nchains, base = C / c->nranks, rem = C % c->nranks;
-  const int64_t b = (int64_t)c->rank * base + std::min<int64_t>(c->rank, rem), cnt = base + (c->rank < rem ? 1 : 0);
-  if (shard_begin) *shard_begin = b;
-  if (shard_count) *shard_count = cnt;
-  int64_t mine[5] = {0, 0, 0, 0, 0};          // #A, #B, accepted, cross-model proposed, cross-model accepted
-  int rc = MG_OK;
-  if (cnt > 0) {
-    mg_rjmcmc_cfg local = *cfg;
-    local.nchains = cnt; local.chain_offset = cfg->chain_offset + (uint64_t)b;
-    const int64_t acc0 = ctx->naccept;
-    rc = mg_rjmcmc_array(ctx, A, B, &local, a0, b0, out_model, out_samples, mine);
-    mine[2] = ctx->naccept - acc0; mine[3] = ctx->rj_cross[0]; mine[4] = ctx->rj_cross[1];
-  } else {
-    ctx->epoch++;                              // every rank consumes the same epoch of its context's key
-  }
-  int64_t status = rc;
-  std::vector<int64_t> all((size_t)6 * c->nranks);
-  int64_t rec[6] = {mine[0], mine[1], mine[2], mine[3], mine[4], status};
-  int rc2 = mg_comm_allgather(c, rec, all.data(), sizeof rec);
-  if (rc) return rc;
-  if (rc2) return rc2;
-  int64_t tot[5] = {0, 0, 0, 0, 0};
-  for (int r = 0; r < c->nranks; ++r) {
-    if (all[6 * r + 5] != 0) return set_err(ctx, (int)all[6 * r + 5], "rjmcmc_array (sharded): rank %d failed", r);
-    for (int k = 0; k < 5; ++k) tot[k] += all[6 * r + k];
-  }
-  out_counts[0] = tot[0]; out_counts[1] = tot[1];
-  ctx->rj_cross[0] = tot[3]; ctx->rj_cross[1] = tot[4];
-  return MG_OK;
-}
-
-// Stats.multi_mean / multi_std (stats.ml:58-87) of samples held by several ranks, from each rank's own
-// (count, mean[F], std[F]): the pairs are all-gathered and pooled in rank order with the parallel-variance update
-// (Chan et al.), std with n - 1 as the reference.  Every rank receives the same values.
-extern "C" int mg_comm_pool_moments(mg_comm *c, int64_t n_local, const double *mean_local, const double *std_local,
-                                    int32_t F, int64_t *n_total, double *out_mean, double *out_std) {
-  if (!c) return MG_EINVAL;
-  mg_ctx *ctx = c->ctx;
-  MG_REQUIRE(ctx, mean_local && std_local && F >= 1 && F <= 4096 && n_local >= 0, "pool_moments: bad arguments");
-  std::vector<double> mine((size_t)1 + 2 * F), all(((size_t)1 + 2 * F) * c->nranks);
-  mine[0] = (double)n_local;
-  for (int i = 0; i < F; ++i) {
-    mine[1 + i] = mean_local[i];
-    mine[1 + F + i] = n_local > 1 ? std_local[i] * std_local[i] * ((double)n_local - 1.0) : 0.0;   // sum of squared deviations
-  }
-  int rc = mg_comm_allgather(c, mine.data(), all.data(), (int64_t)(sizeof(double) * mine.size()));
-  if (rc) return rc;
-  double n = 0.0;
-  std::vector<double> mean(F, 0.0), m2(F, 0.0);
-  for (int r = 0; r < c->nranks; ++r) {
-    const double *rec = all.data() + (size_t)r * mine.size();
-    const double cnt = rec[0];
-    if (cnt == 0.0) continue;
-    const double tot = n + cnt;
-    for (int i = 0; i < F; ++i) {
-      const double delta = rec[1 + i] - mean[i];
-      mean[i] = mean[i] + delta * (cnt / tot);
-      m2[i] = m2[i] + rec[1 + F + i] + delta * delta * (n * cnt / tot);
-    }
-    n = tot;
-  }
-  if (n_total) *n_total = (int64_t)n;
-  for (int i = 0; i < F; ++i) {
-    if (out_mean) out_mean[i] = mean[i];
-    if (out_std) out_std[i] = n > 1.0 ? sqrt(m2[i] / (n - 1.0)) : 0.0;
-  }
   return MG_OK;
 }
 
@@ -482,21 +400,21 @@ int build_tree_distributed(mg_comm *c, const double *d_pts, int64_t N, int D, co
   MG_CHECK_LAUNCH(ctx);
   phase("gather");
   rc = build_tree(ctx, rows.get(), my_n, D, low, high, min_split, false, &sub);
-  const int rc_sub = rc;                         // a failure travels in the record below, so that no rank is left waiting
   phase("subtree");
-  const KdHeader &sh = rc_sub == MG_OK ? sub->h : no_header;
-  const char *sb = rc_sub == MG_OK ? (const char *)sub->d_blob : nullptr;
-  struct Rec { int32_t nl, nn, npts, pbegin; int32_t lb[KDD_MAXL + 1]; int32_t bad; };
-  Rec mine{};
-  if (rc_sub == MG_OK) {                         // the builder's level table, cut at KDD_MAXL levels (then flagged below)
+  struct Rec { int32_t nl, nn, npts, pbegin; int32_t lb[KDD_MAXL + 1]; int32_t deep; };
+  std::vector<Rec> mine(1), recs;
+  if (rc == MG_OK) {                             // the builder's level table, cut at KDD_MAXL levels (then flagged)
+    Rec &m = mine[0];
     const std::vector<int32_t> &lvb = sub->level_begin;
-    mine.nl = (int32_t)std::min<size_t>(lvb.size() - 1, KDD_MAXL);
-    for (int l = 0; l <= mine.nl; ++l) mine.lb[l] = lvb[l];
+    m.nl = (int32_t)std::min<size_t>(lvb.size() - 1, KDD_MAXL);
+    for (int l = 0; l <= m.nl; ++l) m.lb[l] = lvb[l];
+    m.nn = (int32_t)sub->h.nnodes; m.npts = my_n; m.pbegin = my_b;
+    m.deep = m.nl >= KDD_MAXL || m.lb[m.nl] != m.nn;
   }
-  mine.nn = (int32_t)sh.nnodes; mine.npts = my_n; mine.pbegin = my_b;
-  mine.bad = rc_sub != MG_OK ? 2 : ((mine.nl >= KDD_MAXL || mine.lb[mine.nl] != mine.nn) ? 1 : 0);
-  std::vector<Rec> recs((size_t)R);
-  if ((rc = mg_comm_allgather(c, &mine, recs.data(), sizeof mine))) return rc;
+  // a failure travels as the record's status, so that no rank is left waiting
+  if ((rc = comm_gather(c, rc, mine, recs, "kd-tree (distributed)"))) return rc;
+  const KdHeader &sh = sub->h;
+  const char *sb = (const char *)sub->d_blob;
   phase("tables");
   // ---- 3. numbering of the whole tree and the exchange -------------------------------------------------------------------
   std::vector<KddTables> Tv(1);
@@ -505,8 +423,7 @@ int build_tree_distributed(mg_comm *c, const double *d_pts, int64_t N, int D, co
   int maxl = 0; int64_t chunk = 0;
   for (int r = 0; r < R; ++r) {
     const Rec &q = recs[r];
-    if (q.bad == 2) return (r == c->rank) ? rc_sub : set_err(ctx, MG_EFAIL, "kd-tree (distributed): rank %d failed to build its subtree", r);
-    if (q.bad) return set_err(ctx, MG_EFAIL, "kd-tree (distributed): rank %d built a subtree deeper than %d levels", r, KDD_MAXL);
+    if (q.deep) return set_err(ctx, MG_EFAIL, "kd-tree (distributed): rank %d built a subtree deeper than %d levels", r, KDD_MAXL);
     T.nl[r] = q.nl; T.nn[r] = q.nn; T.npts[r] = q.npts; T.pbegin[r] = q.pbegin;
     memcpy(T.lb[r], q.lb, sizeof q.lb);
     for (int l = q.nl + 1; l <= KDD_MAXL; ++l) T.lb[r][l] = q.nn;
@@ -571,102 +488,4 @@ extern "C" int mg_kdtree_build_distributed(mg_comm *c, const double *d_pts, int6
   const int rc = build_tree_distributed(c, d_pts, N, D, low, high, min_split, true, &t);
   *out = t.release();
   return rc;
-}
-
-// Ensemble diagnostics (diagnostics.cu) of chains sharded over the ranks: every rank runs the local pass on its own
-// [n][D+2][C_r] block and pools it into one record per field, (count, mean and M2 of the sequence means, sum s_m^2,
-// sum_m gamma_m(t)) = F (L + 4) doubles, plus its status; the records are all-gathered and folded in rank order by the
-// same host step as the single-GPU call, so every rank gets the same bytes and one rank gives the single-GPU bits.
-namespace mg {
-int diag_check_cfg(mg_ctx *ctx, const mg_diag_cfg *cfg);
-int diag_local_record(mg_ctx *ctx, const double *d_x, const mg_diag_cfg *cfg, double *d_seq_tau, std::vector<double> &rec);
-void diag_finish(const double *recs, int R, int F, int L, int64_t N, double *rhat, double *ess, double *tau,
-                 int32_t *closed, double *rho);
-}  // namespace mg
-
-extern "C" int mg_comm_chain_diagnostics(mg_comm *c, const double *d_samples_local, const mg_diag_cfg *cfg_local,
-                                         double *out_rhat, double *out_ess, double *out_tau, int32_t *out_window_closed,
-                                         double *out_rho, double *d_seq_tau) {
-  if (!c) return MG_EINVAL;
-  mg_ctx *ctx = c->ctx;
-  // dim and maxlag size the exchanged record: every rank must pass the same values (include/mcmc_gpu.h).  A rank that
-  // fails this check returns before the collective and the others wait for it, as in mg_comm_pool_moments; every
-  // later failure (other checks, the local pass) still takes part in the all-gather and is reported on every rank.
-  MG_REQUIRE(ctx, cfg_local && cfg_local->dim >= 1 && cfg_local->maxlag >= 2 && cfg_local->maxlag <= MG_DIAG_MAXLAG,
-             "chain_diagnostics (comm): bad configuration");
-  MG_CUDA(ctx, cudaSetDevice(ctx->device));
-  const int F = cfg_local->dim + 2, L = cfg_local->maxlag, W = L + 4;
-  int rc = diag_check_cfg(ctx, cfg_local);
-  if (rc == MG_OK && !(d_samples_local && out_rhat && out_ess && out_tau && out_window_closed))
-    rc = set_err(ctx, MG_EINVAL, "chain_diagnostics (comm): null argument");
-  std::vector<double> rec;
-  if (rc == MG_OK) rc = diag_local_record(ctx, d_samples_local, cfg_local, d_seq_tau, rec);
-  std::vector<double> mine((size_t)F * W + 3, 0.0), all(mine.size() * c->nranks);
-  if (rc == MG_OK) std::copy(rec.begin(), rec.end(), mine.begin());
-  const int64_t N = cfg_local->split ? cfg_local->n / 2 : cfg_local->n;
-  mine[(size_t)F * W] = (double)rc;
-  mine[(size_t)F * W + 1] = (double)N;
-  mine[(size_t)F * W + 2] = (double)cfg_local->split;
-  const int rc2 = mg_comm_allgather(c, mine.data(), all.data(), (int64_t)(sizeof(double) * mine.size()));
-  if (rc) return rc;
-  if (rc2) return rc2;
-  std::vector<double> recs((size_t)F * W * c->nranks);
-  for (int r = 0; r < c->nranks; ++r) {
-    const double *q = all.data() + mine.size() * r;
-    if (q[(size_t)F * W] != 0.0) return set_err(ctx, (int)q[(size_t)F * W], "chain_diagnostics (comm): rank %d failed", r);
-    if (q[(size_t)F * W + 1] != (double)N || q[(size_t)F * W + 2] != (double)cfg_local->split)
-      return set_err(ctx, MG_EINVAL, "chain_diagnostics (comm): rank %d has another n or split", r);
-    std::copy(q, q + (size_t)F * W, recs.begin() + (size_t)F * W * r);
-  }
-  diag_finish(recs.data(), c->nranks, F, L, N, out_rhat, out_ess, out_tau, out_window_closed, out_rho);
-  return MG_OK;
-}
-
-// Quantiles (quantiles.cu) of the union of every rank's block: one header exchange checks that n, D and the probs
-// agree and gives the pooled size; the order statistics then run on every rank with their exchanges (brackets, region
-// counts, select histograms) summed in rank order, so every rank gets the same bytes and one rank the single-GPU bits.
-namespace mg {
-int qt_check(mg_ctx *ctx, const void *x, int64_t n, int32_t D, int64_t C, const void *list, int32_t nq,
-             const double *out);
-int qt_prob_ranks(mg_ctx *ctx, const double *probs, int32_t nq, int64_t N, std::vector<int64_t> &ranks);
-int qt_order_keys(mg_ctx *ctx, mg_comm *comm, const double *d_x, int64_t n, int32_t D, int64_t C, int64_t N,
-                  const std::vector<int64_t> &ranks, std::vector<uint64_t> &keys, std::vector<int> &nan_f);
-void qt_finish_quantiles(const double *probs, int32_t nq, int64_t N, int F, const std::vector<int64_t> &ranks,
-                         const std::vector<uint64_t> &keys, const std::vector<int> &nan_f, double *out);
-}  // namespace mg
-
-extern "C" int mg_comm_quantiles(mg_comm *c, const double *d_samples_local, int64_t n, int32_t D, int64_t C_local,
-                                 const double *probs, int32_t nq, double *out) {
-  if (!c) return MG_EINVAL;
-  mg_ctx *ctx = c->ctx;
-  std::vector<int64_t> ranks;
-  int rc = qt_check(ctx, d_samples_local, n, D, C_local, probs, nq, out);
-  if (rc == MG_OK) rc = qt_prob_ranks(ctx, probs, nq, n * C_local, ranks);
-  if (rc == MG_OK && cudaSetDevice(ctx->device) != cudaSuccess) rc = set_err(ctx, MG_ECUDA, "cuda: cannot select the device");
-  // header: status, n, D, C_r, nq, the bits of probs
-  const size_t H = 5 + MG_QUANT_MAX;
-  std::vector<uint64_t> mine(H, 0), all(H * c->nranks);
-  mine[0] = (uint64_t)rc;
-  if (rc == MG_OK) {
-    mine[1] = (uint64_t)n; mine[2] = (uint64_t)D; mine[3] = (uint64_t)C_local; mine[4] = (uint64_t)nq;
-    memcpy(&mine[5], probs, sizeof(double) * nq);
-  }
-  const int rc2 = mg_comm_allgather(c, mine.data(), all.data(), (int64_t)(sizeof(uint64_t) * H));
-  if (rc) return rc;
-  if (rc2) return rc2;
-  int64_t Ctot = 0;
-  for (int r = 0; r < c->nranks; ++r) {
-    const uint64_t *q = all.data() + H * r;
-    if (q[0] != 0) return set_err(ctx, (int)q[0], "quantiles (comm): rank %d failed", r);
-    if (!std::equal(q + 1, q + 3, mine.begin() + 1) || !std::equal(q + 4, q + H, mine.begin() + 4))
-      return set_err(ctx, MG_EINVAL, "quantiles (comm): rank %d has another n, D or probs", r);
-    Ctot += (int64_t)q[3];
-  }
-  const int64_t N = n * Ctot;
-  if ((rc = qt_prob_ranks(ctx, probs, nq, N, ranks))) return rc;
-  std::vector<uint64_t> keys;
-  std::vector<int> nan_f;
-  if ((rc = qt_order_keys(ctx, c, d_samples_local, n, D, C_local, N, ranks, keys, nan_f))) return rc;
-  qt_finish_quantiles(probs, nq, N, D + 2, ranks, keys, nan_f, out);
-  return MG_OK;
 }

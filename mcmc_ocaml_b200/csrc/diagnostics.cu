@@ -18,12 +18,13 @@
 // then tau_m per sequence (Geyer), and one record per CTA: (count, mean and M2 of the sequence means, sum s_m^2,
 // sum_m gamma_m(t)).  A pool kernel folds the records of a field in a fixed order (Chan's update for the means,
 // compensated sums for the rest); the host turns the pooled record into Rhat, rho, tau, ESS.  The same host step pools
-// the records of several ranks (comm.cu), so one rank and one GPU give the same bits.
+// the records of several ranks (mg_comm_chain_diagnostics), so one rank and one GPU give the same bits.
 #include <math_constants.h>
 
+#include <algorithm>
 #include <cmath>
 
-#include "common.cuh"
+#include "comm.cuh"
 #include "reduce.cuh"
 
 namespace mg {
@@ -220,7 +221,7 @@ __global__ void __launch_bounds__(DG_POOL) diag_pool_kernel(const double *__rest
   }
 }
 
-int diag_check_cfg(mg_ctx *ctx, const mg_diag_cfg *cfg) {
+static int diag_check_cfg(mg_ctx *ctx, const mg_diag_cfg *cfg) {
   MG_REQUIRE(ctx, cfg, "chain_diagnostics: null configuration");
   MG_REQUIRE(ctx, cfg->n >= 1 && cfg->nchains >= 1 && cfg->dim >= 1, "chain_diagnostics: bad block shape");
   MG_REQUIRE(ctx, cfg->split == 0 || cfg->split == 1, "chain_diagnostics: split is 0 or 1");
@@ -234,7 +235,7 @@ int diag_check_cfg(mg_ctx *ctx, const mg_diag_cfg *cfg) {
 }
 
 // The local pass: d_pooled [F][L + 4] = this block's pooled record of every field; d_seq_tau [F][M] or null.
-int diag_local(mg_ctx *ctx, const double *d_x, const mg_diag_cfg *cfg, double *d_pooled, double *d_seq_tau) {
+static int diag_local(mg_ctx *ctx, const double *d_x, const mg_diag_cfg *cfg, double *d_pooled, double *d_seq_tau) {
   cudaStream_t st = ctx->stream;
   const int F = cfg->dim + 2, L = cfg->maxlag, nblk = (L + DG_LB - 1) / DG_LB;
   DgArgs a;
@@ -265,8 +266,8 @@ int diag_local(mg_ctx *ctx, const double *d_x, const mg_diag_cfg *cfg, double *d
 }
 
 // Pooled records of R ranks (host [R][F][L + 4], rank order) -> the outputs; the same arithmetic on every rank.
-void diag_finish(const double *recs, int R, int F, int L, int64_t N, double *rhat, double *ess, double *tau,
-                 int32_t *closed, double *rho) {
+static void diag_finish(const double *recs, int R, int F, int L, int64_t N, double *rhat, double *ess, double *tau,
+                        int32_t *closed, double *rho) {
   const int W = L + 4;
   const double nan = std::nan(""), Nd = (double)N;
   std::vector<double> gbar(L);
@@ -318,7 +319,8 @@ void diag_finish(const double *recs, int R, int F, int L, int64_t N, double *rha
 }
 
 // local pass + pooled record to the host
-int diag_local_record(mg_ctx *ctx, const double *d_x, const mg_diag_cfg *cfg, double *d_seq_tau, std::vector<double> &rec) {
+static int diag_local_record(mg_ctx *ctx, const double *d_x, const mg_diag_cfg *cfg, double *d_seq_tau,
+                             std::vector<double> &rec) {
   const int F = cfg->dim + 2, W = cfg->maxlag + 4;
   DevBuf<double> pooled;
   MG_CUDA(ctx, pooled.alloc((size_t)F * W, ctx->stream));
@@ -368,5 +370,33 @@ extern "C" int mg_stats_chain_diagnostics(mg_ctx *ctx, const double *samples, co
     MG_CUDA(ctx, cudaMemcpyAsync(seq_tau, d_tau.get(), sizeof(double) * F * M, cudaMemcpyDeviceToHost, ctx->stream));
     MG_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
   }
+  return MG_OK;
+}
+
+// Chains sharded over the ranks: every rank runs the local pass on its own [n][D+2][C_r] block and pools it into one
+// record per field, F (L + 4) doubles; the records are all-gathered and folded in rank order by the same host step as
+// the single-GPU call, so every rank gets the same bytes and one rank gives the single-GPU bits.  A header exchange
+// first checks that dim and maxlag, which size the records, and n and split agree.
+extern "C" int mg_comm_chain_diagnostics(mg_comm *c, const double *d_samples_local, const mg_diag_cfg *cfg_local,
+                                         double *out_rhat, double *out_ess, double *out_tau, int32_t *out_window_closed,
+                                         double *out_rho, double *d_seq_tau) {
+  if (!c) return MG_EINVAL;
+  mg_ctx *ctx = mg_comm_ctx(c);
+  int rc = diag_check_cfg(ctx, cfg_local);
+  if (rc == MG_OK && !(d_samples_local && out_rhat && out_ess && out_tau && out_window_closed))
+    rc = set_err(ctx, MG_EINVAL, "chain_diagnostics (comm): null argument");
+  if (rc == MG_OK && cudaSetDevice(ctx->device) != cudaSuccess) rc = set_err(ctx, MG_ECUDA, "cuda: cannot select the device");
+  std::vector<int64_t> hdr(4, 0), hdrs;
+  if (rc == MG_OK) hdr = {cfg_local->dim, cfg_local->maxlag, cfg_local->n, cfg_local->split};
+  if ((rc = comm_gather(c, rc, hdr, hdrs, "chain_diagnostics (comm)"))) return rc;
+  for (int r = 0; r < mg_comm_size(c); ++r)
+    if (!std::equal(hdr.begin(), hdr.end(), hdrs.begin() + 4 * r))
+      return set_err(ctx, MG_EINVAL, "chain_diagnostics (comm): rank %d has another dim, maxlag, n or split", r);
+  const int F = cfg_local->dim + 2, L = cfg_local->maxlag;
+  std::vector<double> rec((size_t)F * (L + 4)), recs;
+  rc = diag_local_record(ctx, d_samples_local, cfg_local, d_seq_tau, rec);
+  if ((rc = comm_gather(c, rc, rec, recs, "chain_diagnostics (comm)"))) return rc;
+  const int64_t N = cfg_local->split ? cfg_local->n / 2 : cfg_local->n;
+  diag_finish(recs.data(), mg_comm_size(c), F, L, N, out_rhat, out_ess, out_tau, out_window_closed, out_rho);
   return MG_OK;
 }

@@ -18,7 +18,7 @@
 //             (:122-124,150-160).
 // Per-cell terms are bit-exact up to exp(); the sum over cells is compensated,
 // i.e. closer to the exact sum than the reference's left-to-right fold.
-#include "common.cuh"
+#include "comm.cuh"
 #include "kdtree.cuh"
 #include "radix_sort.cuh"
 #include "reduce.cuh"
@@ -304,6 +304,27 @@ extern "C" int mg_evidence_harmonic_mean(mg_ctx *ctx, const double *ll, int64_t 
   return mg_evidence_harmonic_mean_dev(ctx, d_ll.get(), N, out);
 }
 
+// The same over samples SHARDED across ranks: every rank reduces the 1/L of its own shard (compensated), the
+// (count, sum) pairs are all-gathered and folded in rank order.  Agrees with the single-GPU value to the rounding of
+// the compensated sums (<= 2 ulp); identical on every rank.
+extern "C" int mg_evidence_harmonic_mean_sharded(mg_comm *c, const double *d_ll_shard, int64_t n_shard, double *out) {
+  if (!c) return MG_EINVAL;
+  mg_ctx *ctx = mg_comm_ctx(c);
+  int rc = MG_OK;
+  if (!(out && n_shard >= 0 && (d_ll_shard || n_shard == 0)))
+    rc = set_err(ctx, MG_EINVAL, "evidence_harmonic_mean (sharded): bad arguments");
+  if (rc == MG_OK && cudaSetDevice(ctx->device) != cudaSuccess) rc = set_err(ctx, MG_ECUDA, "cuda: cannot select the device");
+  std::vector<double> mine = {(double)n_shard, 0.0}, all;
+  if (rc == MG_OK && n_shard > 0)
+    rc = reduce_sum(ctx, n_shard, [d_ll_shard] __device__(int64_t i) { return 1.0 / exp(d_ll_shard[i]); }, &mine[1]);
+  if ((rc = comm_gather(c, rc, mine, all, "evidence_harmonic_mean (sharded)"))) return rc;
+  Comp linv; double n = 0.0;
+  for (int r = 0; r < mg_comm_size(c); ++r) { n += all[2 * r]; linv.add(all[2 * r + 1]); }
+  MG_REQUIRE(ctx, n >= 1.0, "evidence_harmonic_mean (sharded): no samples on any rank");
+  *out = n / linv.value();
+  return MG_OK;
+}
+
 // evidence.ml:202-205: the kept prefix, its mean 1/L, and the survivors of remove_dups_rev (reversed)
 static int lebesgue_prepare(mg_ctx *ctx, const double *d_pts, const double *d_ll, const double *d_lp, int64_t N, int32_t D,
                             int32_t n, double eps, Survivors &sv, double *mean_il_out) {
@@ -443,46 +464,33 @@ extern "C" int mg_evidence_direct_dev(mg_ctx *ctx, const double *d_pts, const do
 // contiguous ranges, one per rank, each rank evaluates the cell terms of its range; the per-node terms are
 // all-gathered (ncclAllGather, in place) and every rank runs the SAME deterministic reduction over the complete
 // array -- the result is bit-identical on every rank and to the single-GPU call.
-struct mg_comm;
-namespace mg {
-int comm_broadcast_dev(mg_comm *c, void *d_buf, size_t nbytes, int root);
-int comm_allgather_dev(mg_comm *c, const void *d_send, void *d_recv, size_t nbytes_per_rank);
-}
-extern "C" int mg_kdtree_broadcast(mg_comm *c, mg_kdtree *tree, int32_t root, mg_kdtree **out);
-extern "C" int32_t mg_comm_rank(const mg_comm *c);
-extern "C" int32_t mg_comm_size(const mg_comm *c);
-mg_ctx *mg_comm_ctx(const mg_comm *c);   // comm.cu
-
 static int evidence_sharded(mg_comm *c, int which, int32_t root, const double *d_pts, const double *d_ll, const double *d_lp,
                             int64_t N, int32_t D, int32_t n, double eps, double *out) {
   if (!c) return MG_EINVAL;
   mg_ctx *ctx = mg_comm_ctx(c);
   const int R = mg_comm_size(c), rank = mg_comm_rank(c);
-  MG_REQUIRE(ctx, out && root >= 0 && root < R && n >= 1, "evidence (sharded): bad arguments");
-  MG_CUDA(ctx, cudaSetDevice(ctx->device));
-  cudaStream_t s = ctx->stream;
   int rc = MG_OK;
+  if (!(out && root >= 0 && root < R && n >= 1)) rc = set_err(ctx, MG_EINVAL, "evidence (sharded): bad arguments");
+  if (rc == MG_OK && cudaSetDevice(ctx->device) != cudaSuccess) rc = set_err(ctx, MG_ECUDA, "cuda: cannot select the device");
+  cudaStream_t s = ctx->stream;
   Survivors sv;
-  double head[3] = {0.0, 0.0, 0.0};   // {mean 1/L of the kept prefix, status of the root's preparation, survivors}
-  if (rank == root) {
-    double mean_il = 1.0;
+  double mean_il = 1.0;                 // mean 1/L of the kept prefix (Lebesgue)
+  if (rc == MG_OK && rank == root)
     rc = which == 0 ? lebesgue_prepare(ctx, d_pts, d_ll, d_lp, N, D, n, eps, sv, &mean_il)
                     : direct_prepare(ctx, d_pts, d_ll, d_lp, N, D, n, sv);
-    head[0] = mean_il; head[1] = (double)rc; head[2] = (double)sv.K;
-  }
-  // the root's status travels first, so that a failure there ends the call on every rank instead of a hang
-  DevBuf<double> d_head;
-  MG_CUDA(ctx, d_head.alloc(3, s));
-  if (rank == root) MG_CUDA(ctx, cudaMemcpyAsync(d_head.get(), head, sizeof head, cudaMemcpyHostToDevice, s));
-  int rc2 = comm_broadcast_dev(c, d_head.get(), sizeof head, root);
-  if (rc2) return rc2;
-  MG_CUDA(ctx, cudaMemcpyAsync(head, d_head.get(), sizeof head, cudaMemcpyDeviceToHost, s));
-  MG_CUDA(ctx, cudaStreamSynchronize(s));
-  if (head[1] != 0.0)
-    return rank == root ? rc : set_err(ctx, (int)head[1], "evidence (sharded): the root rank failed to prepare the samples");
+  // one exchange: every rank's status (a failure anywhere ends the call on every rank instead of a hang), the
+  // arguments that must agree, and the root's mean 1/L and survivor count
+  struct Head { int64_t root, D, n; uint64_t eps; int64_t K; double mean_il; };
+  std::vector<Head> head(1), heads;
+  head[0] = {root, D, n, 0, sv.K, mean_il};
+  memcpy(&head[0].eps, &eps, sizeof eps);
+  if ((rc = comm_gather(c, rc, head, heads, "evidence (sharded)"))) return rc;
+  for (int r = 0; r < R; ++r)
+    if (heads[r].root != root || heads[r].D != D || heads[r].n != n || heads[r].eps != head[0].eps)
+      return set_err(ctx, MG_EINVAL, "evidence (sharded): rank %d has another root, D, n or eps", r);
   // the survivors (rows, lp, and ll for the direct estimator) go to every rank; the tree over them is then built by
   // all ranks together (build_tree_distributed: top levels everywhere, one subtree per rank, one all-gather)
-  const int64_t K = (int64_t)head[2];
+  const int64_t K = heads[root].K;
   if (rank != root) {
     sv.K = K;
     cudaError_t e = sv.pts.alloc((size_t)K * D, s);
@@ -521,7 +529,7 @@ static int evidence_sharded(mg_comm *c, int which, int32_t root, const double *d
   double total = 0.0;
   if (rc == MG_OK) rc = sum_terms(ctx, terms.get(), nn, &total);
   if (rc) return rc;
-  *out = which == 0 ? total / head[0] : total;
+  *out = which == 0 ? total / heads[root].mean_il : total;
   return MG_OK;
 }
 

@@ -30,7 +30,7 @@
 #include <cmath>
 #include <cstdlib>
 
-#include "common.cuh"
+#include "comm.cuh"
 #include "radix_sort.cuh"
 
 namespace mg {
@@ -206,30 +206,6 @@ __global__ void __launch_bounds__(QT_THREADS) qt_select_kernel(const QtSelArgs a
 
 // ---- host --------------------------------------------------------------------------------------------------------
 
-// Combine a host vector of integers over the ranks in rank order (op(i, acc, x)), carrying every rank's status: a
-// failure on any rank is returned on every rank.  Without a communicator only the local status is returned.
-template <class Op>
-static int qt_exchange(mg_ctx *ctx, mg_comm *comm, int rc, std::vector<uint64_t> &v, Op op) {
-  if (!comm) return rc;
-  const int R = mg_comm_size(comm);
-  const size_t W = v.size() + 1;
-  std::vector<uint64_t> mine(W, 0), all(W * R);
-  mine[0] = (uint64_t)rc;
-  if (rc == MG_OK) std::copy(v.begin(), v.end(), mine.begin() + 1);
-  const int rc2 = mg_comm_allgather(comm, mine.data(), all.data(), (int64_t)(sizeof(uint64_t) * W));
-  if (rc) return rc;
-  if (rc2) return rc2;
-  for (int r = 0; r < R; ++r)
-    if (all[W * r] != 0) return set_err(ctx, (int)all[W * r], "quantiles (comm): rank %d failed", r);
-  for (size_t i = 0; i < v.size(); ++i) {
-    uint64_t acc = all[1 + i];
-    for (int r = 1; r < R; ++r) acc = op(i, acc, all[W * r + 1 + i]);
-    v[i] = acc;
-  }
-  return MG_OK;
-}
-static uint64_t qt_sum(size_t, uint64_t a, uint64_t b) { return a + b; }
-
 static int64_t qt_chunks(mg_ctx *ctx, int64_t nslot, int64_t maxlen) {
   int64_t ch = std::max<int64_t>(1, ((int64_t)ctx->sm_count * 32 + nslot - 1) / nslot);
   ch = std::max(ch, (maxlen + QT_CHUNK_MAX - 1) / QT_CHUNK_MAX);
@@ -311,7 +287,14 @@ static int qt_select(mg_ctx *ctx, mg_comm *comm, bool keys, const void *base, in
     }
     if (rc == MG_OK) rc = local(pass);
     hist.resize((size_t)hoff[ns]);
-    if ((rc = qt_exchange(ctx, comm, rc, hist, qt_sum))) return rc;
+    if (comm) {                                     // the histograms of all ranks, summed in rank order
+      std::vector<uint64_t> all;
+      if ((rc = comm_gather(comm, rc, hist, all, "quantiles (comm)"))) return rc;
+      hist.assign(all.begin(), all.begin() + hist.size());
+      for (size_t r = 1; r < all.size() / hist.size(); ++r)
+        for (size_t i = 0; i < hist.size(); ++i) hist[i] += all[hist.size() * r + i];
+    }
+    if (rc) return rc;
     for (int64_t g = 0; g < ns; ++g)
       for (size_t t = 0; t < sl.rank[g].size(); ++t) {
         const uint64_t *h = hist.data() + hoff[g] + 256LL * tp[g][t];
@@ -329,8 +312,8 @@ static int qt_select(mg_ctx *ctx, mg_comm *comm, bool keys, const void *base, in
 
 // Order statistics of ascending, distinct global ranks (N = the pooled size over the ranks, C_local this rank's
 // chains) for every field: keys [F][K]; nan [F] = 1 where the field holds a NaN.
-int qt_order_keys(mg_ctx *ctx, mg_comm *comm, const double *d_x, int64_t n, int32_t D, int64_t C, int64_t N,
-                  const std::vector<int64_t> &ranks, std::vector<uint64_t> &keys, std::vector<int> &nan_f) {
+static int qt_order_keys(mg_ctx *ctx, mg_comm *comm, const double *d_x, int64_t n, int32_t D, int64_t C, int64_t N,
+                         const std::vector<int64_t> &ranks, std::vector<uint64_t> &keys, std::vector<int> &nan_f) {
   cudaStream_t st = ctx->stream;
   const int F = D + 2, K = (int)ranks.size();
   const int64_t Nl = n * C, rstride = (int64_t)F * C;
@@ -370,10 +353,15 @@ int qt_order_keys(mg_ctx *ctx, mg_comm *comm, const double *d_x, int64_t n, int3
     MG_CUDA(ctx, cudaStreamSynchronize(st));
     return MG_OK;
   }();
-  if ((rc = qt_exchange(ctx, comm, rc, br, [](size_t i, uint64_t a, uint64_t b) {
-         return (i & 1) ? std::max(a, b) : std::min(a, b);
-       })))
-    return rc;
+  if (comm) {                                        // the widest bracket of the ranks: min of lo, max of hi
+    std::vector<uint64_t> all;
+    if ((rc = comm_gather(comm, rc, br, all, "quantiles (comm)"))) return rc;
+    br.assign(all.begin(), all.begin() + br.size());
+    for (size_t r = 1; r < all.size() / br.size(); ++r)
+      for (size_t i = 0; i < br.size(); ++i)
+        br[i] = (i & 1) ? std::max(br[i], all[br.size() * r + i]) : std::min(br[i], all[br.size() * r + i]);
+  }
+  if (rc) return rc;
   // merge each field's overlapping brackets; tb[f][j] = bracket of target j
   std::vector<int> nb(F, 0);
   std::vector<uint64_t> blo((size_t)F * QT_MAXT), bhi((size_t)F * QT_MAXT);
@@ -430,7 +418,14 @@ int qt_order_keys(mg_ctx *ctx, mg_comm *comm, const double *d_x, int64_t n, int3
     }
     return MG_OK;
   }();
-  if ((rc = qt_exchange(ctx, comm, rc, tally, qt_sum))) return rc;
+  if (comm) {                                        // counts and flags of all ranks, summed in rank order
+    std::vector<uint64_t> all;
+    if ((rc = comm_gather(comm, rc, tally, all, "quantiles (comm)"))) return rc;
+    tally.assign(all.begin(), all.begin() + tally.size());
+    for (size_t r = 1; r < all.size() / tally.size(); ++r)
+      for (size_t i = 0; i < tally.size(); ++i) tally[i] += all[tally.size() * r + i];
+  }
+  if (rc) return rc;
   // 3. resolve: bracket value, candidate rank, or fallback
   keys.assign((size_t)F * K, 0);
   nan_f.assign(F, 0);
@@ -494,8 +489,8 @@ using namespace mg;
 
 namespace mg {
 
-int qt_check(mg_ctx *ctx, const void *x, int64_t n, int32_t D, int64_t C, const void *list, int32_t nq,
-             const double *out) {
+static int qt_check(mg_ctx *ctx, const void *x, int64_t n, int32_t D, int64_t C, const void *list, int32_t nq,
+                    const double *out) {
   MG_REQUIRE(ctx, x && list && out, "quantiles: null argument");
   MG_REQUIRE(ctx, n >= 1 && C >= 1 && D >= 1 && D <= INT32_MAX - 2, "quantiles: bad block shape");
   MG_REQUIRE(ctx, nq >= 1 && nq <= MG_QUANT_MAX, "quantiles: need 1 <= nq <= %d", MG_QUANT_MAX);
@@ -504,7 +499,7 @@ int qt_check(mg_ctx *ctx, const void *x, int64_t n, int32_t D, int64_t C, const 
 }
 
 // the ranks probs need (ascending, distinct); N = the pooled size
-int qt_prob_ranks(mg_ctx *ctx, const double *probs, int32_t nq, int64_t N, std::vector<int64_t> &ranks) {
+static int qt_prob_ranks(mg_ctx *ctx, const double *probs, int32_t nq, int64_t N, std::vector<int64_t> &ranks) {
   ranks.clear();
   for (int i = 0; i < nq; ++i) {
     const double p = probs[i];
@@ -529,8 +524,8 @@ static double qt_interp(double a, double b, double g) {
 }
 
 // keys [F][K] of ranks -> out [F][nq]
-void qt_finish_quantiles(const double *probs, int32_t nq, int64_t N, int F, const std::vector<int64_t> &ranks,
-                         const std::vector<uint64_t> &keys, const std::vector<int> &nan_f, double *out) {
+static void qt_finish_quantiles(const double *probs, int32_t nq, int64_t N, int F, const std::vector<int64_t> &ranks,
+                                const std::vector<uint64_t> &keys, const std::vector<int> &nan_f, double *out) {
   const int K = (int)ranks.size();
   auto x = [&](int f, int64_t k) {
     const int j = (int)(std::lower_bound(ranks.begin(), ranks.end(), k) - ranks.begin());
@@ -596,5 +591,39 @@ extern "C" int mg_stats_order_statistics_dev(mg_ctx *ctx, const double *d_sample
       const int j = (int)(std::lower_bound(rk.begin(), rk.end(), ranks[i]) - rk.begin());
       out[(size_t)f * nk + i] = nan_f[f] ? NAN : ordered_to_f64(keys[(size_t)f * K + j]);
     }
+  return MG_OK;
+}
+
+// The union of every rank's block: one header exchange checks that n, D and the probs agree and gives the pooled size;
+// the order statistics then run on every rank with their exchanges (brackets, region counts, select histograms) folded
+// in rank order, so every rank gets the same bytes and one rank the single-GPU bits.
+extern "C" int mg_comm_quantiles(mg_comm *c, const double *d_samples_local, int64_t n, int32_t D, int64_t C_local,
+                                 const double *probs, int32_t nq, double *out) {
+  if (!c) return MG_EINVAL;
+  mg_ctx *ctx = mg_comm_ctx(c);
+  std::vector<int64_t> ranks;
+  int rc = qt_check(ctx, d_samples_local, n, D, C_local, probs, nq, out);
+  if (rc == MG_OK) rc = qt_prob_ranks(ctx, probs, nq, n * C_local, ranks);
+  if (rc == MG_OK && cudaSetDevice(ctx->device) != cudaSuccess) rc = set_err(ctx, MG_ECUDA, "cuda: cannot select the device");
+  // header: n, D, C_r, nq, the bits of probs
+  std::vector<uint64_t> mine(4 + MG_QUANT_MAX, 0), all;
+  if (rc == MG_OK) {
+    mine[0] = (uint64_t)n; mine[1] = (uint64_t)D; mine[2] = (uint64_t)C_local; mine[3] = (uint64_t)nq;
+    memcpy(&mine[4], probs, sizeof(double) * nq);
+  }
+  if ((rc = comm_gather(c, rc, mine, all, "quantiles (comm)"))) return rc;
+  int64_t Ctot = 0;
+  for (int r = 0; r < mg_comm_size(c); ++r) {
+    const uint64_t *q = all.data() + mine.size() * r;
+    if (!std::equal(q, q + 2, mine.begin()) || !std::equal(q + 3, q + mine.size(), mine.begin() + 3))
+      return set_err(ctx, MG_EINVAL, "quantiles (comm): rank %d has another n, D or probs", r);
+    Ctot += (int64_t)q[2];
+  }
+  const int64_t N = n * Ctot;
+  if ((rc = qt_prob_ranks(ctx, probs, nq, N, ranks))) return rc;
+  std::vector<uint64_t> keys;
+  std::vector<int> nan_f;
+  if ((rc = qt_order_keys(ctx, c, d_samples_local, n, D, C_local, N, ranks, keys, nan_f))) return rc;
+  qt_finish_quantiles(probs, nq, N, D + 2, ranks, keys, nan_f, out);
   return MG_OK;
 }

@@ -11,7 +11,9 @@
 // (kdtree.cuh).  Traffic per step: 1 byte (model) or
 // 8 (Dmax+2) bytes (full sample) per recorded chain-step plus ~16 B per tree
 // level gathered through L2 -- latency-bound pointer chasing, not HBM-bound.
-#include "common.cuh"
+#include <algorithm>
+
+#include "comm.cuh"
 #include "host_plugins.hpp"
 
 #include "rj_kernel_dev.cuh"
@@ -206,6 +208,43 @@ extern "C" int mg_rjmcmc_array_k(mg_ctx *ctx, const mg_rj_model *models, int32_t
   }
   if (!(psum - 1.0 < sqrt(2.220446049250313e-16))) return set_err(ctx, MG_EFAIL, "Assert_failure mcmc.ml:90 (sum of the model priors)");
   return rj_run<MG_RJ_MAX_MODELS>(ctx, M, nmodels, cfg, starts, out_model, out_samples, out_counts);
+}
+
+// mg_rjmcmc_array with the ensemble's chains cut into contiguous ranges, one per rank: rank r runs the global chain ids
+// cfg->chain_offset + [b_r, e_r) (the Philox stream is addressed by the global id, so the chains do not depend on the
+// number of ranks), then rjmcmc_model_counts (mcmc.ml:141-149) and the accept / jump counters of all ranks are
+// all-gathered and summed.  out_model / out_samples receive this rank's shard only ([n][C_r], [n][Dmax+2][C_r]);
+// *shard_begin / *shard_count tell which chains those are.
+extern "C" int mg_rjmcmc_array_sharded(mg_comm *c, const mg_rj_model *A, const mg_rj_model *B, const mg_rjmcmc_cfg *cfg,
+                                       const double *a0, const double *b0, uint8_t *out_model, double *out_samples,
+                                       int64_t out_counts[2], int64_t *shard_begin, int64_t *shard_count) {
+  if (!c) return MG_EINVAL;
+  mg_ctx *ctx = mg_comm_ctx(c);
+  const int R = mg_comm_size(c), me = mg_comm_rank(c);
+  std::vector<int64_t> mine(5, 0), all;     // #A, #B, accepted, cross-model proposed, cross-model accepted
+  int rc = cfg && out_counts ? MG_OK : set_err(ctx, MG_EINVAL, "rjmcmc_array (sharded): null argument");
+  if (rc == MG_OK) {
+    const int64_t C = cfg->nchains, base = C / R, rem = C % R;
+    const int64_t b = (int64_t)me * base + std::min<int64_t>(me, rem), cnt = base + (me < rem ? 1 : 0);
+    if (shard_begin) *shard_begin = b;
+    if (shard_count) *shard_count = cnt;
+    if (cnt > 0) {
+      mg_rjmcmc_cfg local = *cfg;
+      local.nchains = cnt; local.chain_offset = cfg->chain_offset + (uint64_t)b;
+      const int64_t acc0 = ctx->naccept;
+      rc = mg_rjmcmc_array(ctx, A, B, &local, a0, b0, out_model, out_samples, mine.data());
+      mine[2] = ctx->naccept - acc0; mine[3] = ctx->rj_cross[0]; mine[4] = ctx->rj_cross[1];
+    } else {
+      ctx->epoch++;                           // every rank consumes the same epoch of its context's key
+    }
+  }
+  if ((rc = comm_gather(c, rc, mine, all, "rjmcmc_array (sharded)"))) return rc;
+  int64_t tot[5] = {0, 0, 0, 0, 0};
+  for (int r = 0; r < R; ++r)
+    for (int k = 0; k < 5; ++k) tot[k] += all[5 * r + k];
+  out_counts[0] = tot[0]; out_counts[1] = tot[1];
+  ctx->rj_cross[0] = tot[3]; ctx->rj_cross[1] = tot[4];
+  return MG_OK;
 }
 
 extern "C" int mg_rjmcmc_jump_counters(const mg_ctx *ctx, int64_t *proposed, int64_t *accepted) {

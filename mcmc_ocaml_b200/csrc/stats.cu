@@ -9,7 +9,7 @@
 // exact than the reference's own sequential sum.  The tested error model is in
 // DESIGN.md section S (tests/test_stats_exact_gpu.py).
 // All kernels are HBM-bound: 8 bytes read per element per pass.
-#include "common.cuh"
+#include "comm.cuh"
 #include "models.cuh"
 #include "rng.cuh"
 #include "reduce.cuh"
@@ -358,6 +358,49 @@ extern "C" int mg_stats_multi_std(mg_ctx *ctx, const double *xs, int64_t n, int3
   if ((rc = table_cols(ctx, d_xs.get(), n, D, d_mu.get(), 2, (double)(n - 1), 1, d_out.get()))) return rc;
   MG_CUDA(ctx, cudaMemcpyAsync(out, d_out.get(), sizeof(double) * D, cudaMemcpyDeviceToHost, ctx->stream));
   MG_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+  return MG_OK;
+}
+
+// Stats.multi_mean / multi_std (stats.ml:58-87) of samples held by several ranks, from each rank's own
+// (count, mean[F], std[F]): a header exchange checks that F agrees, then the records are all-gathered and pooled in
+// rank order with the parallel-variance update (Chan et al.), std with n - 1 as the reference.  Every rank receives
+// the same values.
+extern "C" int mg_comm_pool_moments(mg_comm *c, int64_t n_local, const double *mean_local, const double *std_local,
+                                    int32_t F, int64_t *n_total, double *out_mean, double *out_std) {
+  if (!c) return MG_EINVAL;
+  mg_ctx *ctx = mg_comm_ctx(c);
+  int rc = MG_OK;
+  if (!(mean_local && std_local && F >= 1 && F <= 4096 && n_local >= 0)) rc = set_err(ctx, MG_EINVAL, "pool_moments: bad arguments");
+  std::vector<int32_t> hdr = {F}, hdrs;
+  if ((rc = comm_gather(c, rc, hdr, hdrs, "pool_moments"))) return rc;
+  for (int r = 0; r < mg_comm_size(c); ++r)
+    if (hdrs[r] != F) return set_err(ctx, MG_EINVAL, "pool_moments: rank %d has another F", r);
+  std::vector<double> mine((size_t)1 + 2 * F), all;
+  mine[0] = (double)n_local;
+  for (int i = 0; i < F; ++i) {
+    mine[1 + i] = mean_local[i];
+    mine[1 + F + i] = n_local > 1 ? std_local[i] * std_local[i] * ((double)n_local - 1.0) : 0.0;   // sum of squared deviations
+  }
+  if ((rc = comm_gather(c, MG_OK, mine, all, "pool_moments"))) return rc;
+  double n = 0.0;
+  std::vector<double> mean(F, 0.0), m2(F, 0.0);
+  for (int r = 0; r < mg_comm_size(c); ++r) {
+    const double *rec = all.data() + (size_t)r * mine.size();
+    const double cnt = rec[0];
+    if (cnt == 0.0) continue;
+    const double tot = n + cnt;
+    for (int i = 0; i < F; ++i) {
+      const double delta = rec[1 + i] - mean[i];
+      mean[i] = mean[i] + delta * (cnt / tot);
+      m2[i] = m2[i] + rec[1 + F + i] + delta * delta * (n * cnt / tot);
+    }
+    n = tot;
+  }
+  if (n_total) *n_total = (int64_t)n;
+  for (int i = 0; i < F; ++i) {
+    if (out_mean) out_mean[i] = mean[i];
+    if (out_std) out_std[i] = n > 1.0 ? sqrt(m2[i] / (n - 1.0)) : 0.0;
+  }
   return MG_OK;
 }
 
