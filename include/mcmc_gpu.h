@@ -125,7 +125,7 @@ int mg_memcpy_d2d(mg_ctx *ctx, void *dst_dev, const void *src_dev, int64_t nbyte
  * reference ships in bin/ and test/.  User kinds are added at run time with
  * mg_plugin_register_source (NVRTC, inlined into the sampler kernels) and are
  * accepted wherever a log_likelihood / log_prior is: mg_mcmc_array*,
- * mg_rjmcmc_array*, mg_nested_evidence, mg_logfn_eval. */
+ * mg_rjmcmc_array*, mg_nested_evidence, mg_evidence_tempered*, mg_logfn_eval. */
 
 enum {
   /* 0.0 */
@@ -605,6 +605,98 @@ int mg_stats_draw_dev(mg_ctx *ctx, int32_t kind, double a, double b,
                       int64_t n, double *d_out);
 
 /* ------------------------------------------------------------------ */
+/* Evidence by parallel tempering                                      */
+/* ------------------------------------------------------------------ */
+/* M ladders of T tempered chains ("rungs"): rung k samples
+ * pi_k ~ L^beta_k * prior, neighbouring rungs swap states, and log Z follows
+ * from thermodynamic integration (TI, log Z = int_0^1 E_beta[log L] dbeta) and
+ * from stepping stones (SS, Xie et al. 2011:
+ * log Z = sum_k log E_beta_k[L^(beta_k+1 - beta_k)]).
+ *
+ * Definition (the oracle, oracle/tempered_oracle.cpp, transcribes it):
+ * - Inputs: like, prior; props[T], one proposal per rung (pass the same one T
+ *   times for one proposal); betas[T] finite, strictly increasing,
+ *   betas[0] >= 0, betas[T-1] == 1; M ladders whose rungs all start at x0_m
+ *   (x0 [M][D], or [D] with x0_shared), evaluated as in mcmc.ml:59-61;
+ *   nbin >= 0, nsteps >= 1, swap_every >= 0, ladder_offset = global id of
+ *   ladder 0 (sharding).
+ * - Tempered step: rung k runs mcmc.ml:37-56 with the log posterior replaced
+ *   by tl(x) = (beta_k == 0 ? 0.0 : beta_k * ll(x)) + lp(x), in mh_step's
+ *   order: log_accept = tl(y) - tl(x), then + log_backward - log_forward for
+ *   asymmetric proposals; accepted iff log u < log_accept (strict, NaN rejects).
+ * - Draws: the uniforms of step t (t = 0 .. nbin + nsteps - 1) of rung k of
+ *   ladder m are those of (P_MH, g = (ladder_offset + m) * T + k, t).  With
+ *   swap_every = 0 the rung at beta = 1 is, draw for draw, chain g of
+ *   mg_mcmc_array on the same seed and epoch.
+ * - Swaps (even-odd): when swap_every > 0, a swap round follows every step t
+ *   with (t + 1) % swap_every == 0; its number is r = (t + 1) / swap_every - 1
+ *   and it tries the pairs (k, k+1) with k = r (mod 2).  The pair's uniform is
+ *   the first draw of (P_PT_SWAP, g = (ladder_offset + m) * 32 + k, r); the
+ *   swap is accepted iff log u < (beta_k+1 - beta_k) * (ll_k - ll_k+1) and
+ *   exchanges x, ll and lp.
+ * - Measurement: for t >= nbin, after the swap round that follows step t (if
+ *   any), rung k records its ll.  The pivot p is the first measured ll (0.0 if
+ *   that is not finite).  S1 = sum (ll - p) in step order, Neumaier-compensated
+ *   over the finite terms, the non-finite terms added apart (so a -inf gives
+ *   -inf and a NaN gives NaN).  For k < T-1, (a, s) accumulates
+ *   w = (beta_k+1 - beta_k) * ll as a log-sum-exp: a the running maximum,
+ *   s = sum exp(w - a), rescaled when a grows; w = -inf adds nothing.
+ *   Accepted MH steps per rung and accepted swaps per pair are counted over
+ *   the measured phase.
+ * - Per ladder: L_mk = p + S1 / nsteps;  TI_m = sum_k (beta_k+1 - beta_k) *
+ *   (L_mk + L_m,k+1) / 2 in k order;  SS_m = sum_k (a_mk + log(s_mk / nsteps)).
+ * - Pooled (every sum over ladders in ladder order; means and spreads by
+ *   Welford's / Chan's update over the finite values, non-finite values summed
+ *   apart and taking the result over): mean_ll[k] = mean over ladders of L_.k,
+ *   mean_ll_err[k] = sd / sqrt(M); log_z_ti = trapezoid over mean_ll,
+ *   log_z_ti_err = sd(TI_m) / sqrt(M); log_z_ss = sum_k [lse_m(a_mk + log s_mk)
+ *   - log(M * nsteps)], log_z_ss_err = sd(SS_m) / sqrt(M).  sd has M - 1 in
+ *   its denominator: M = 1, or a non-finite value, gives errors of NaN.
+ * - A rung at beta = 0 that measures ll = -inf (a prior draw outside the
+ *   likelihood's support) makes mean_ll[0] and log_z_ti -inf; SS is unaffected
+ *   (exp(-inf) = 0).  SS is the primary estimate; TI also carries the
+ *   trapezoid bias of its ladder (DESIGN 4d).
+ * - One call key (epoch); the context's accept / reject counters are left
+ *   unchanged.  MG_EINVAL: null pointers, M < 1, T outside [2, 32], betas that
+ *   break the rules above, nsteps < 1, nbin < 0, swap_every < 0, nbin + nsteps
+ *   >= 2^31, D outside 1..64, a plugin or proposal whose dim != D, ladder ids
+ *   that overflow the 48-bit chain id of the Philox counter. */
+#define MG_TEMPERED_MAX_T 32
+typedef struct {
+  int64_t nladders;       /* M (this rank's ladders in the sharded call) */
+  int32_t ntemps;         /* T, 2..32 */
+  int32_t dim;            /* D */
+  int64_t nbin;           /* steps before the measured phase */
+  int64_t nsteps;         /* measured steps */
+  int64_t swap_every;     /* a swap round every swap_every steps; 0 = none */
+  uint64_t ladder_offset; /* global id of ladder 0 */
+  int32_t x0_shared;      /* 1: x0 is one start point [D] */
+  int32_t reserved;
+} mg_tempered_cfg;
+
+/* Results.  The four log Z numbers are always written; every pointer may be
+ * NULL.  mean_ll, mean_ll_err, accept: [T]; swaps_accepted, swaps_tried:
+ * [T-1]; final: [M][T][D+2] (x, ll, lp of every replica at the end);
+ * ladder_mean_ll: [M][T] (L_mk).  final and ladder_mean_ll cover this rank's
+ * ladders in the sharded call, everything else all ladders. */
+typedef struct {
+  double log_z_ss, log_z_ss_err;
+  double log_z_ti, log_z_ti_err;
+  double *mean_ll, *mean_ll_err;
+  int64_t *accept, *swaps_accepted, *swaps_tried;
+  double *final;
+  double *ladder_mean_ll;
+} mg_tempered_out;
+
+/* The definition above on one GPU: one warp holds floor(32 / T) ladders, the
+ * swaps are warp shuffles, and every replica keeps its state and sums in
+ * registers for the whole run (DESIGN 4d).  Host arrays. */
+int mg_evidence_tempered(mg_ctx *ctx, const mg_logfn *like, const mg_logfn *prior,
+                         const mg_proposal *props, const double *betas,
+                         const mg_tempered_cfg *cfg, const double *x0,
+                         mg_tempered_out *out);
+
+/* ------------------------------------------------------------------ */
 /* Nested sampling                                                     */
 /* ------------------------------------------------------------------ */
 
@@ -662,7 +754,8 @@ double mg_nested_log_total_error(double log_ev, double log_dev, int32_t nlive);
  * Every entry point here is COLLECTIVE: all ranks of the communicator call it.
  * The rank-pooled calls (the sharded evidence estimators, the distributed
  * kd-tree build, mg_rjmcmc_array_sharded, mg_comm_pool_moments,
- * mg_comm_chain_diagnostics and mg_comm_quantiles) exchange every rank's status
+ * mg_comm_chain_diagnostics, mg_comm_quantiles and mg_evidence_tempered_sharded)
+ * exchange every rank's status
  * before they use another rank's data: an argument error or a failure on any
  * rank is returned on every rank, and the arguments that must be the same on
  * every rank are checked ("rank r has another ..." is MG_EINVAL).  A null comm
@@ -752,6 +845,17 @@ int mg_comm_chain_diagnostics(mg_comm *comm, const double *d_samples_local,
 int mg_comm_quantiles(mg_comm *comm, const double *d_samples_local, int64_t n,
                       int32_t D, int64_t C_local, const double *probs,
                       int32_t nq, double *out);
+/* mg_evidence_tempered (definition in the parallel-tempering section) with
+ * the ladders split over the ranks: each rank runs cfg->nladders ladders from
+ * global id cfg->ladder_offset (x0 covers its own ladders) and reduces them to
+ * a per-rank record, the records are pooled in rank order.  T, betas, nbin,
+ * nsteps, swap_every and dim must agree.  One rank: the single-GPU call's
+ * bits; several: per-ladder outputs and counts equal the single-GPU run on the
+ * union, pooled values agree to rounding. */
+int mg_evidence_tempered_sharded(mg_comm *comm, const mg_logfn *like,
+                                 const mg_logfn *prior, const mg_proposal *props,
+                                 const double *betas, const mg_tempered_cfg *cfg,
+                                 const double *x0, mg_tempered_out *out);
 
 /* ------------------------------------------------------------------ */
 /* Read_write: the text format of the reference's tools (host only)    */

@@ -71,6 +71,20 @@ class mg_diag_cfg(C.Structure):
                 ("split", C.c_int32), ("reserved", C.c_int32)]
 
 
+class mg_tempered_cfg(C.Structure):
+    _fields_ = [("nladders", C.c_int64), ("ntemps", C.c_int32), ("dim", C.c_int32), ("nbin", C.c_int64),
+                ("nsteps", C.c_int64), ("swap_every", C.c_int64), ("ladder_offset", C.c_uint64),
+                ("x0_shared", C.c_int32), ("reserved", C.c_int32)]
+
+
+class mg_tempered_out(C.Structure):
+    _fields_ = [("log_z_ss", C.c_double), ("log_z_ss_err", C.c_double), ("log_z_ti", C.c_double),
+                ("log_z_ti_err", C.c_double), ("mean_ll", c_double_p), ("mean_ll_err", c_double_p),
+                ("accept", c_int64_p), ("swaps_accepted", c_int64_p), ("swaps_tried", c_int64_p),
+                ("final", c_double_p), ("ladder_mean_ll", c_double_p)]
+
+
+TEMPERED_MAX_T = 32  # MG_TEMPERED_MAX_T
 DIAG_MAXLAG = 256   # MG_DIAG_MAXLAG
 QUANT_MAX = 64      # MG_QUANT_MAX
 
@@ -146,6 +160,11 @@ def load_library() -> C.CDLL:
         fn.restype = C.c_int
         items = c_int64_p if name == "mg_stats_order_statistics_dev" else c_double_p
         fn.argtypes = [C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_int64, items, C.c_int32, c_double_p]
+    for name, first in (("mg_evidence_tempered", C.c_void_p), ("mg_evidence_tempered_sharded", C.c_void_p)):
+        fn = getattr(lib, name)
+        fn.restype = C.c_int
+        fn.argtypes = [first, C.POINTER(mg_logfn), C.POINTER(mg_logfn), C.POINTER(mg_proposal), c_double_p,
+                       C.POINTER(mg_tempered_cfg), c_double_p, C.POINTER(mg_tempered_out)]
     _lib = lib
     return lib
 

@@ -190,3 +190,13 @@ class Comm:
         self.ctx.check(self.ctx.lib.mg_comm_quantiles(self.h, samples_ptr, n, D, nchains_local, _abi.ptr(p), p.size,
                                                       _abi.ptr(out)))
         return out
+
+    def evidence_tempered(self, log_likelihood, log_prior, jump_proposals, betas, start, *, nladders: int, nbin: int,
+                          nsteps: int, swap_every: int = 1, ladder_offset: int = 0):
+        """``evidence.evidence_tempered`` with the ladders split over the ranks: this rank runs ``nladders`` ladders
+        from global id ``ladder_offset`` (``start`` covers them); the pooled outputs cover every rank's ladders,
+        ``final`` and ``ladder_mean_ll`` this rank's."""
+        from .evidence import _evidence_tempered_call
+        return _evidence_tempered_call(self.ctx.lib.mg_evidence_tempered_sharded, self.h, log_likelihood, log_prior,
+                                       jump_proposals, betas, start, nladders, nbin, nsteps, swap_every, ladder_offset,
+                                       self.ctx.check)

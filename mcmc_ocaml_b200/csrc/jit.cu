@@ -21,6 +21,7 @@
 #include "mcmc_kernel.cuh"
 #include "nested_kernel_dev.cuh"
 #include "rj_kernel_dev.cuh"
+#include "tempered_kernel_dev.cuh"
 
 #include "build/embedded_headers.inc"
 
@@ -80,7 +81,7 @@ static Api &api() {
 
 struct JitKey { int device, dmax; size_t version; bool operator<(const JitKey &o) const {
   return device != o.device ? device < o.device : dmax != o.dmax ? dmax < o.dmax : version < o.version; } };
-struct JitMod { CUmodule_t mod = nullptr; CUfunction_t mh = nullptr, eval = nullptr, rj = nullptr, nest_init = nullptr, nest_replace = nullptr; };
+struct JitMod { CUmodule_t mod = nullptr; CUfunction_t mh = nullptr, eval = nullptr, rj = nullptr, nest_init = nullptr, nest_replace = nullptr, tempered = nullptr; };
 static std::map<JitKey, JitMod> g_mods;
 
 static const char *kPrelude =
@@ -111,7 +112,11 @@ static std::string make_source(const std::vector<UserFn> &fns, int dmax) {
        "extern \"C\" __global__ void mg_user_nest_init(mg::NestArgs a, double *x, double *ll, double *lp) {\n"
        "  mg::nest_init_body<" << dmax << ">(a, x, ll, lp);\n}\n"
        "extern \"C\" __global__ void mg_user_nest_replace(mg::NestArgs a, mg::NestProp p, int s0, int s1, int first, int last, double *cx, double *ccl) {\n"
-       "  mg::nest_replace_simple_body<" << dmax << ">(a, p, s0, s1, first, last, cx, ccl);\n}\n";
+       "  mg::nest_replace_simple_body<" << dmax << ">(a, p, s0, s1, first, last, cx, ccl);\n}\n"
+       // the parallel-tempering evidence kernel (tempered.cu) with the user functions as log_likelihood / log_prior
+       "#include \"tempered_kernel_dev.cuh\"\n"
+       "extern \"C\" __global__ void __maxnreg__(255) mg_user_tempered(const __grid_constant__ mg::TpArgs a) {\n"
+       "  mg::tempered_body<" << dmax << ">(a);\n}\n";
   return s.str();
 }
 
@@ -146,7 +151,8 @@ static int get_module(mg_ctx *ctx, int dmax, JitMod *out) {
   if (a.cuModuleLoadData(&m.mod, cubin.data())) return set_err(ctx, MG_ECUDA, "cuda: cuModuleLoadData failed for the plugin module");
   if (a.cuModuleGetFunction(&m.mh, m.mod, "mg_user_mh") || a.cuModuleGetFunction(&m.eval, m.mod, "mg_user_eval") ||
       a.cuModuleGetFunction(&m.rj, m.mod, "mg_user_rj") || a.cuModuleGetFunction(&m.nest_init, m.mod, "mg_user_nest_init") ||
-      a.cuModuleGetFunction(&m.nest_replace, m.mod, "mg_user_nest_replace"))
+      a.cuModuleGetFunction(&m.nest_replace, m.mod, "mg_user_nest_replace") ||
+      a.cuModuleGetFunction(&m.tempered, m.mod, "mg_user_tempered"))
     return set_err(ctx, MG_ECUDA, "cuda: plugin module lacks its entry points");
   g_mods[key] = m;
   *out = m;
@@ -221,6 +227,18 @@ int jit_launch_nest_replace(mg_ctx *ctx, int D, const NestArgs &a, const NestPro
   void *params[] = {&aa, &pp, &s0, &s1, &first, &last, &chain_x, &chain_cl};
   if (api().cuLaunchKernel(m.nest_replace, (unsigned)((a.K + 63) / 64), 1, 1, 64, 1, 1, 0, ctx->stream, params, nullptr))
     return set_err(ctx, MG_ECUDA, "cuda: launch of the plugin nested-replacement kernel failed");
+  return MG_OK;
+}
+
+// mg_evidence_tempered with user-registered log-densities (called from tempered.cu)
+int jit_launch_tempered(mg_ctx *ctx, const TpArgs &a, int D, unsigned grid, unsigned block) {
+  JitMod m;
+  int rc = get_module(ctx, dmax_for(D), &m);
+  if (rc) return rc;
+  TpArgs aa = a;
+  void *params[] = {&aa};
+  if (api().cuLaunchKernel(m.tempered, grid, 1, 1, block, 1, 1, 0, ctx->stream, params, nullptr))
+    return set_err(ctx, MG_ECUDA, "cuda: launch of the plugin parallel-tempering kernel failed");
   return MG_OK;
 }
 

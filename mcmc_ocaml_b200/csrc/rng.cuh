@@ -16,7 +16,7 @@ namespace mg {
 
 enum Purpose : uint32_t {
   P_MH = 1, P_RJ = 2, P_RJ_INIT = 3, P_DRAW = 4, P_NEST_INIT = 5,
-  P_NEST_MCMC = 6, P_NEST_START = 7, P_POST = 8, P_BOOT = 9
+  P_NEST_MCMC = 6, P_NEST_START = 7, P_POST = 8, P_BOOT = 9, P_PT_SWAP = 10
 };
 
 #define MG_PHILOX_M0 0xD2511F53u

@@ -55,6 +55,10 @@ external quantiles_raw :
 external quantiles_dev_raw :
   ctx -> int64 -> int -> int -> int -> (float, float64_elt, c_layout) Array1.t -> (float, float64_elt, c_layout) Array2.t ->
   unit = "mcmcgpu_quantiles_dev_bytecode" "mcmcgpu_quantiles_dev_native"
+external evidence_tempered_raw :
+  ctx -> logfn -> logfn -> proposal array -> (float, float64_elt, c_layout) Array1.t -> int array ->
+  (float, float64_elt, c_layout) Array2.t -> (float, float64_elt, c_layout) Array1.t ->
+  (int64, int64_elt, c_layout) Array1.t -> unit = "mcmcgpu_evidence_tempered_bytecode" "mcmcgpu_evidence_tempered_native"
 (* the record the stub reads field by field (rj_of_value in mcmc_gpu_stubs.c) *)
 type rj_model_raw = {
   r_like : logfn; r_prior : logfn; r_prop : proposal; r_into : tree option;
@@ -230,6 +234,23 @@ let quantiles_dev ctx ~probs ~n ~dim ~nchains (block : int64) =
   let out = Array2.create float64 c_layout f (Array.length probs) in
   quantiles_dev_raw ctx block n dim nchains (Array1.of_array float64 c_layout probs) out;
   quantiles_result f probs out
+
+(* Evidence by parallel tempering (mg_evidence_tempered; the definition is in include/mcmc_gpu.h) *)
+type tempered = {
+  log_z_ss : float; log_z_ss_err : float; log_z_ti : float; log_z_ti_err : float;
+  mean_ll : float array; mean_ll_err : float array;
+  accept : int array; swaps_accepted : int array; swaps_tried : int array;
+}
+let evidence_tempered ctx ?(swap_every = 1) ~nladders ~nbin ~nsteps like prior props betas (start : float array array) =
+  let t = Array.length betas in
+  let x0 = Array2.of_array float64 c_layout start in
+  let out = Array1.create float64 c_layout (4 + 2 * t) and cnt = Array1.create int64 c_layout (3 * t) in
+  evidence_tempered_raw ctx like prior props (Array1.of_array float64 c_layout betas)
+    [| nladders; nbin; nsteps; swap_every |] x0 out cnt;
+  let ints o n = Array.init n (fun i -> Int64.to_int cnt.{o + i}) in
+  { log_z_ss = out.{0}; log_z_ss_err = out.{1}; log_z_ti = out.{2}; log_z_ti_err = out.{3};
+    mean_ll = Array.init t (fun k -> out.{4 + k}); mean_ll_err = Array.init t (fun k -> out.{4 + t + k});
+    accept = ints 0 t; swaps_accepted = ints t (t - 1); swaps_tried = ints (2 * t) (t - 1) }
 
 (* Nested.nested_evidence ?epsrel ?nmcmc ?nlive ?mode_hopping_frac (nested.ml:122-146; nested.mli:50-61) with draw_prior
    uniform on [prior_low, prior_high]; ?batch live points are replaced per iteration (1 = the reference's schedule).

@@ -117,6 +117,19 @@ val quantiles :
 val quantiles_dev : ctx -> probs:float array -> n:int -> dim:int -> nchains:int -> int64 -> float array array
 (** The same on a device block (its address), which is not modified. *)
 
+type tempered = {
+  log_z_ss : float; log_z_ss_err : float; log_z_ti : float; log_z_ti_err : float;
+  mean_ll : float array; mean_ll_err : float array;
+  accept : int array; swaps_accepted : int array; swaps_tried : int array;
+}
+val evidence_tempered :
+  ctx -> ?swap_every:int -> nladders:int -> nbin:int -> nsteps:int -> logfn -> logfn -> proposal array -> float array ->
+  float array array -> tempered
+(** log Z by parallel tempering: [nladders] ladders of [Array.length betas] tempered chains (one proposal per rung,
+    betas strictly increasing from >= 0 to 1), all rungs of a ladder starting at its row of [start] (one row: shared).
+    [log_z_ss] (stepping stones) is the primary estimate; [log_z_ti] also carries the trapezoid bias of the ladder.
+    Definitions in mcmc_gpu.h.  [Invalid_argument] for fewer than 2 or more than 32 rungs, bad betas, nsteps < 1. *)
+
 (** {2 Nested (nested.mli:50-69)} *)
 val nested_evidence :
   ctx -> ?epsrel:float -> ?nmcmc:int -> ?nlive:int -> ?mode_hopping_frac:float -> ?batch:int -> ?max_points:int ->

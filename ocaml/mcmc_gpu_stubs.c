@@ -370,6 +370,46 @@ CAMLprim value mcmcgpu_quantiles_dev_bytecode(value *a, int argn) {
   return mcmcgpu_quantiles_dev_native(a[0], a[1], a[2], a[3], a[4], a[5], a[6]);
 }
 
+/* ---- evidence by parallel tempering (mg_evidence_tempered) ----------------------------------------------------
+ * external evidence_tempered : ctx -> logfn -> logfn -> proposal array -> Array1.t (* betas [T] *) ->
+ *   int array (* nladders, nbin, nsteps, swap_every *) -> Array2.t (* start [M][D] or [1][D] *) ->
+ *   Array1.t (* out: 4 log Z numbers, mean_ll [T], mean_ll_err [T] *) ->
+ *   (int64) Array1.t (* accept [T], swaps_accepted [T], swaps_tried [T]; the last of each pair block unused *) -> unit */
+CAMLprim value mcmcgpu_evidence_tempered_native(value ctx, value like, value prior, value props, value betas, value cfgv,
+                                                value start, value out, value cnt) {
+  CAMLparam5(ctx, like, prior, props, betas);
+  CAMLxparam4(cfgv, start, out, cnt);
+  mg_ctx *c = Ctx_val(ctx);
+  const int T = (int)Wosize_val(props);
+  if (T < 2 || T > MG_TEMPERED_MAX_T || (int)Caml_ba_array_val(betas)->dim[0] != T)
+    caml_invalid_argument("evidence_tempered: 2..32 rungs, one proposal per beta");
+  mg_proposal ps[MG_TEMPERED_MAX_T];
+  for (int k = 0; k < T; ++k) ps[k] = proposal_of_value(Field(props, k));
+  const mg_logfn l = logfn_of_value(like), p = logfn_of_value(prior);
+  struct caml_ba_array *st = Caml_ba_array_val(start);
+  mg_tempered_cfg cfg;
+  memset(&cfg, 0, sizeof cfg);
+  cfg.nladders = Long_val(Field(cfgv, 0)); cfg.ntemps = T; cfg.dim = l.dim;
+  cfg.nbin = Long_val(Field(cfgv, 1)); cfg.nsteps = Long_val(Field(cfgv, 2)); cfg.swap_every = Long_val(Field(cfgv, 3));
+  cfg.x0_shared = st->dim[0] == 1 ? 1 : 0;
+  if (st->dim[1] != l.dim || (!cfg.x0_shared && st->dim[0] != cfg.nladders))
+    caml_invalid_argument("evidence_tempered: start must be [nladders][D] or [1][D]");
+  double *o = (double *)Caml_ba_data_val(out);
+  int64_t *n = (int64_t *)Caml_ba_data_val(cnt);
+  mg_tempered_out r;
+  memset(&r, 0, sizeof r);
+  r.mean_ll = o + 4; r.mean_ll_err = o + 4 + T;
+  r.accept = n; r.swaps_accepted = n + T; r.swaps_tried = n + 2 * T;
+  check(c, mg_evidence_tempered(c, &l, &p, ps, (const double *)Caml_ba_data_val(betas), &cfg,
+                                (const double *)Caml_ba_data_val(start), &r));
+  o[0] = r.log_z_ss; o[1] = r.log_z_ss_err; o[2] = r.log_z_ti; o[3] = r.log_z_ti_err;
+  CAMLreturn(Val_unit);
+}
+CAMLprim value mcmcgpu_evidence_tempered_bytecode(value *a, int argn) {
+  (void)argn;
+  return mcmcgpu_evidence_tempered_native(a[0], a[1], a[2], a[3], a[4], a[5], a[6], a[7], a[8]);
+}
+
 /* ---- Stats.draw_uniform / draw_gaussian / draw_cauchy (stats.ml:89-91,113-128), n draws per call ----------
  * external stats_draw : ctx -> int -> float -> float -> (float, float64_elt, c_layout) Array1.t -> unit
  * kind: 0 uniform a b | 1 gaussian mu sigma | 2 cauchy x0 gamma (MG_DRAW_*) */

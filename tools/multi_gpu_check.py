@@ -17,6 +17,8 @@ NCCL id and allocates the test data):
      identical rows), so that the level table of that rank comes from the first builder.
   9. exact quantiles of a seeded block whose chains are shared unevenly over the ranks (mg_comm_quantiles): the same
      bytes on every rank, equal to the single-GPU call on the whole block.
+ 10. parallel-tempering evidence with ladders shared unevenly over the ranks (mg_evidence_tempered_sharded): every
+     rank's ladders and the counts equal to the single-GPU call over all ladders, pooled values within 1e-12.
 Prints one JSON line on rank 0."""
 from __future__ import annotations
 
@@ -179,6 +181,30 @@ def main():
         one = stats.quantiles(xq, probs, ctx=ctx)
         out["quantiles_identical_on_all_ranks"] = bool(all(np.array_equal(allq[r_], allq[0]) for r_ in range(world)))
         out["quantiles_bit_identical_to_single_gpu"] = bool(np.array_equal(qv.view(np.int64), one.view(np.int64)))
+    # ---- 10. parallel tempering with ladders shared unevenly (mg_evidence_tempered_sharded) ------------------------
+    Dt, Tt, Mt = 6, 12, 301
+    like_t = P.gauss_diag(np.full(Dt, 0.5), np.full(Dt, 0.1)); prior_t = P.box(np.zeros(Dt), np.ones(Dt), 0.0)
+    betas_t = (np.arange(Tt) / (Tt - 1.0)) ** 3
+    props_t = [P.box_proposal(np.full(Dt, 0.5 if b == 0 else min(0.5, 2.4 * 0.1 / np.sqrt(b * Dt)))) for b in betas_t]
+    x0_t = np.random.default_rng(77).uniform(0.2, 0.8, (Mt, Dt))
+    te = [Mt * r_ * (r_ + 1) // (world * (world + 1)) for r_ in range(world + 1)]
+    tb, tn = te[rank], te[rank + 1] - te[rank]
+    kw_t = dict(nbin=200, nsteps=2000, swap_every=1)
+    ctx.set_seed(99)
+    sh = comm.evidence_tempered(like_t, prior_t, props_t, betas_t, x0_t[tb:tb + tn], nladders=tn, ladder_offset=tb, **kw_t)
+    ctx.set_seed(99)
+    one_t = evidence.evidence_tempered(like_t, prior_t, props_t, betas_t, x0_t, nladders=Mt, ctx=ctx, **kw_t)
+    pooled = np.array([sh.log_z_ss, sh.log_z_ss_err, sh.log_z_ti, sh.log_z_ti_err, *sh.mean_ll, *sh.mean_ll_err])
+    pooled1 = np.array([one_t.log_z_ss, one_t.log_z_ss_err, one_t.log_z_ti, one_t.log_z_ti_err, *one_t.mean_ll,
+                        *one_t.mean_ll_err])
+    ok_t = (np.array_equal(sh.final, one_t.final[tb:tb + tn]) and np.array_equal(sh.ladder_mean_ll, one_t.ladder_mean_ll[tb:tb + tn])
+            and all(np.array_equal(getattr(sh, k_), getattr(one_t, k_)) for k_ in ("accept", "swaps_accepted", "swaps_tried"))
+            and np.allclose(pooled, pooled1, rtol=1e-12, atol=1e-12))
+    flags_t = np.asarray(comm.allgather(np.array([1.0 if ok_t else 0.0, *pooled])))
+    if rank == 0:
+        out["tempered_ladders_and_counts_equal_single_gpu_on_every_rank"] = bool(flags_t[:, 0].min() == 1.0)
+        out["tempered_pooled_identical_on_all_ranks"] = bool(all(np.array_equal(flags_t[r_, 1:], flags_t[0, 1:]) for r_ in range(world)))
+        out["tempered_log_z_ss"] = [float(sh.log_z_ss), float(sh.log_z_ss_err)]
     # ---- 5. sharded RJMCMC over the broadcast tree(s) ----------------------------
     d2 = Dm
     likeA = P.gauss_diag(np.full(d2, 0.5), np.full(d2, 0.08)); priorA = P.box(np.zeros(d2), np.ones(d2), 0.0)
@@ -247,6 +273,8 @@ def main():
                          and out["evidence_bit_identical_to_single_gpu"] and out["rj_counts_equal"]
                          and out["diagnostics_identical_on_all_ranks"] and out["diagnostics_within_1e12_of_single_gpu"]
                          and out["quantiles_identical_on_all_ranks"] and out["quantiles_bit_identical_to_single_gpu"]
+                         and out["tempered_ladders_and_counts_equal_single_gpu_on_every_rank"]
+                         and out["tempered_pooled_identical_on_all_ranks"]
                          and all(out[f"dist_build_ms{ms}"]["identical_to_single_gpu_on_every_rank"] for ms in (2, 64))
                          and out["dist_build_first_builder"]["identical_to_single_gpu_on_every_rank"])
         s_ = json.dumps(out)
